@@ -21,11 +21,11 @@ step through formgpu_batch_submit - calls of the same kind share ONE launch per 
             vs the measured HBM peak (+ every other group under roofline.kernel_groups)
   single_sequence   the latency mode: ONE sequence per GPU (value / e2e / kernel times)
   cpu_baseline      the same multi-sequence job on the CPU oracle (kind "port"): one
-            single-threaded replay per host core, bounded sample; plus the reference's own
+            single-threaded replay per host core, --cpu-sample scans each; plus the reference's own
             threading (one sequence, parallel_for over keypoints) for comparison
 
-`--impl reference` times the CPU oracle on the same job.  The reference cannot be built as
-shipped here (no Eigen / GTSAM / TBB); its C++ sources do compile, unmodified, over API stand-ins
+`--impl reference` times the CPU oracle on the same job, --steps scans per sequence.  The
+reference cannot be built as shipped here (no Eigen / GTSAM / TBB); its C++ sources do compile, unmodified, over API stand-ins
 into oracle/_ref, but that library is a checker (restated Eigen arithmetic, serial TBB, restated
 GTSAM optimiser), not a representative build: it is timed only as labelled extra rows
 (reference_code_stage1, reference_code_pipeline), where it is the SLOWER of the two CPU codes.
@@ -208,6 +208,47 @@ def sequence_id(rank: int, m: int) -> int:
     return rank * 1000 + m
 
 
+DUMP_BUDGET = 64 << 20  # bytes of .npy data that --dump-outputs may write
+
+
+def dump_sequences(M: int) -> list:
+    """The sequences (slots of rank 0) whose outputs --dump-outputs writes: 8 drawn with a fixed
+    seed from the first 32, which every automatic --sequences-per-gpu has, so that runs on hosts
+    with different free memory still dump the same sequences."""
+    pool = min(M, 32)
+    return sorted(int(m) for m in np.random.default_rng(0).choice(pool, size=min(pool, 8), replace=False))
+
+
+def write_outputs(out_dir: str, dumped: dict):
+    """DIR/<leg>_<name>.npy, float64, one row per record; column 0 is the sequence.  `leg` is
+    `value` (device-resident scans) or `e2e` (host scans, so the keypoints come back too); every
+    record of the last timed scan of each dumped sequence, in call order.  Over DUMP_BUDGET, rows
+    are thinned by a fixed seed."""
+    def columns(a):
+        if a.dtype.names is None:
+            return a.reshape(a.shape[0], int(np.prod(a.shape[1:]))).astype(np.float64)
+        return np.stack([a[f].astype(np.float64) for f in a.dtype.names], axis=1)
+
+    names = {"counts": "pair_counts", "blocks": "blocks", "errors": "errors", "keypoint_counts": "keypoint_counts",
+             "planar": "planar_keypoints", "point": "point_keypoints"}
+    arrays = {}
+    for leg, per_seq in dumped.items():
+        for name, file_name in names.items():
+            out = np.concatenate([np.column_stack([np.full(len(c[name]), float(m)), columns(c[name])])
+                                  for m, c in sorted(per_seq.items())])
+            if len(out):  # value leg: no keypoints come back; fused LM schedule: no error calls
+                arrays[f"{leg}_{file_name}"] = out
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BUDGET:
+        rng = np.random.default_rng(0)
+        for k, a in arrays.items():
+            keep = int(len(a) * DUMP_BUDGET / total * 0.99)
+            arrays[k] = a[np.sort(rng.choice(len(a), size=keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def run_ours(args, rank, world, local_rank):
     import torch
 
@@ -293,8 +334,9 @@ def run_ours(args, rank, world, local_rank):
         torch.cuda.synchronize()
 
     groups = [list(range(g, M, G)) for g in range(G)]
+    dumped = {}  # leg -> {sequence: what the calls of its last timed scan returned}
 
-    def timed_batched(ptr_table, on_device):
+    def timed_batched(ptr_table, on_device, leg):
         """G concurrent batches replay scans W..S of their sequences; device time by CUDA
         events on the current stream around a full-device synchronize on both sides."""
         reps = [BatchReplay([traces[i] for i in grp], p) for grp in groups]
@@ -302,6 +344,9 @@ def run_ours(args, rank, world, local_rank):
         run_batches(reps, 0, W0, gptrs, on_device, T)  # pre-roll + warm-up: fills every fixed-lag window
         for r_ in reps:
             r_.reset_stats()
+        if args.dump_outputs:  # only the dumped sequences copy their records inside the timed region
+            for m in dump_sequences(M):
+                reps[m % G].capture_last_scan(m // G)
         launches0 = sum(r_.launch_count() for r_ in reps)
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
@@ -313,6 +358,8 @@ def run_ours(args, rank, world, local_rank):
         t_dev = a.elapsed_time(b) / 1e3
         st = sum_stats([r_.stats() for r_ in reps])
         launches = sum(r_.launch_count() for r_ in reps) - launches0
+        if args.dump_outputs:
+            dumped[leg] = {m: reps[m % G].captured(m // G) for m in dump_sequences(M)}
         for r_ in reps:
             r_.close()
         return t_dev, t_host, st, launches
@@ -334,18 +381,20 @@ def run_ours(args, rank, world, local_rank):
         rp.close()
         return {g: round(1e3 * v["ms"] / (M * K), 2) for g, v in sorted(prof.items()) if v["launches"]} if rank == 0 else None
     if args.only_e2e:  # development aid: only the host-buffer leg
-        t_e2e, _, _, _ = timed_batched(host_ptrs, False)
+        t_e2e, _, _, _ = timed_batched(host_ptrs, False, "e2e")
         sampler.stop()
         return {"sequences_per_gpu": M, "batches_per_gpu": G, "e2e": round(M * K / t_e2e, 2)} if rank == 0 else None
-    t_value, t_value_host, stats_d, gpu_launches = timed_batched(dev_ptrs, True)
+    t_value, t_value_host, stats_d, gpu_launches = timed_batched(dev_ptrs, True, "value")
     if args.only_value:  # development aid (configuration sweeps): not a bench line
         sampler.stop()
         return {"sequences_per_gpu": M, "batches_per_gpu": G, "value": round(M * K / t_value, 2),
                 "setup_s": round(t_gen + t_record, 1)} if rank == 0 else None
     # ---- e2e: pinned host scans in, f64 keypoints + blocks out, through the same C-ABI ----
-    t_e2e, _, stats_h, _ = timed_batched(host_ptrs, False)
+    t_e2e, _, stats_h, _ = timed_batched(host_ptrs, False, "e2e")
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, dumped)
 
     # ---- per-kernel-group CUDA-event timing of the same region: ONE batch with all M
     # sequences, events around every launch (this inflates short launches by a few us) ----
@@ -1025,9 +1074,7 @@ def run_reference(args, rank, world):
     S = W + K
     cores = host_cores()
     workers = cores if args.sequences_per_gpu <= 0 else min(cores, args.sequences_per_gpu)
-    # bounded sample: the CPU needs ~0.2 s per scan and core
-    last = min(S, W + max(1, min(K, args.cpu_sample)))
-    n = last - W
+    last, n = S, K
 
     def scans_of(w):
         return [synth.scan(args.sensor, sequence_id(0, w), k, 1) for k in range(last)]
@@ -1070,7 +1117,9 @@ def main():
                     help="sequences: independent sequences per GPU (the headline, weak scaling); sharded: "
                          "configs[4], ONE dense 128x2048 sequence point-sharded over the ranks (strong scaling)")
     ap.add_argument("--sensor", default="os0-128", choices=sorted(SENSOR_OF_WORKLOAD))
-    ap.add_argument("--cpu-sample", type=int, default=20, help="scans per sequence timed on the CPU")
+    ap.add_argument("--cpu-sample", type=int, default=20,
+                    help="scans per sequence of the cpu_baseline row that --impl ours reports beside the GPU "
+                         "value (--impl reference times --steps scans)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--sequences-per-gpu", type=int, default=0,
                     help="independent sequences sharing one GPU (0 = 128 if host memory allows, else 64)")
@@ -1091,7 +1140,18 @@ def main():
                     help="the sequences of a GPU are split over this many concurrent batches (measured, 128 "
                          "sequences: 8 batches 3.6-8.7 k scans/s - one batch per host thread leaves a stream idle "
                          "whenever its thread is descheduled -, 12: 9.4-9.5 k, 16: 8.6-8.9 k, 32: 7.2 k)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the calls of the last timed scan returned (pair "
+                         "counts, normal-equation blocks, error values, keypoints) for a fixed sample of "
+                         "sequences as DIR/<name>.npy (float64, at most 64 MB), to compare two builds")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "sequences"):
+        ap.error("--dump-outputs needs --impl ours --mode sequences")
+    if args.dump_outputs and (args.only_value or args.only_e2e or args.only_profile):
+        ap.error("--dump-outputs needs both timed legs: it cannot be combined with --only-value, --only-e2e "
+                 "or --only-profile")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     rank = int(os.environ.get("RANK", "0"))

@@ -257,6 +257,8 @@ FORMHOST_SYMBOLS = {
     "formhost_batch_replay_run_pipelined": (_d, [_vp, _sz, _sz, _sz, _sz, _vp, _i]),
     "formhost_batch_replay_stats": (None, [_vp, _i, _vp, C.POINTER(_d)]),
     "formhost_batch_replay_reset_stats": (None, [_vp]),
+    "formhost_batch_replay_capture": (None, [_vp, _sz, _i]),
+    "formhost_batch_replay_captured": (_sz, [_vp, _sz, _i, _vp, _sz]),
     **estimator_symbols("formhost_"),
 }
 

@@ -16,6 +16,16 @@ namespace form {
 
 class BatchReplay {
 public:
+  /// What the calls of one scan of one sequence handed back, in call order.
+  struct Captured {
+    std::vector<PairCount> counts;  // every ASSOCIATE / ASSOC_LIN
+    std::vector<double> blocks;     // 91 per pair, every ASSOC_LIN / LINEARIZE
+    std::vector<double> errors;     // one per pair, every ERROR
+    std::vector<uint64_t> keypoint_counts; // EXTRACT: planar, point; COMMIT: novel planar, point
+    std::vector<PlanarFeat> planar; // host-scan replays only
+    std::vector<PointFeat> point;
+  };
+
   /// traces[s] drives sequence s.  `stream` = cudaStream_t of the batch (nullptr: private).
   BatchReplay(const std::vector<const Trace *> &traces, const HotPathParams &hp, int device,
               void *stream, int max_window_scans)
@@ -40,6 +50,9 @@ public:
   formgpu_batch *batch() const { return m_batch; }
   size_t size() const { return m_traces.size(); }
   ReplayStats &stats(size_t s) { return m_stats[s]; }
+  /// on: every later run keeps what the calls of its last scan return for sequence s
+  void capture_last_scan(size_t s, bool on) { m_seq[s].capture = on; }
+  const Captured &captured(size_t s) const { return m_seq[s].last; }
 
   /// Replays scans [first, last) of every sequence.  scans[s][k] = scan k of sequence s
   /// (device pointers when on_device, host pointers otherwise; host scans come back as
@@ -65,6 +78,8 @@ public:
       m_seq[s].op = lo < hi ? t.scan_begin[lo] : 0;
       m_seq[s].end = lo < hi ? t.op_end(hi - 1) : 0;
       m_seq[s].scan_hi = hi;
+      m_seq[s].last_begin = lo < hi ? t.scan_begin[hi - 1] : 0;
+      if (m_seq[s].capture) m_seq[s].last = Captured();
     }
     m_on_device = on_device;
     m_rounds = 0;
@@ -97,6 +112,7 @@ public:
       const size_t s = m_owner[r];
       const TraceOp &op = (*m_traces[s]).ops[m_seq[s].op];
       account(s, op, m_reqs[r]);
+      if (m_seq[s].capture && m_seq[s].op >= m_seq[s].last_begin) capture(s, op, m_reqs[r]);
       m_seq[s].op += 1;
       // a log is being reprocessed: the next scan of the sequence is known, so its upload starts
       // as soon as the extraction of this one has completed (the scan buffers alternate)
@@ -141,13 +157,45 @@ private:
   struct Seq {
     size_t op = 0, end = 0;
     size_t scan_hi = 0; // scans [.., scan_hi) belong to the run in progress
+    size_t last_begin = 0; // first op of scan scan_hi - 1
     uint64_t cur_scan = 0;
     size_t cur_np = 0, cur_nq = 0;
     std::vector<PairCount> counts;
     std::vector<double> out;
     PlanarFeat *planar = nullptr; // page-locked (host-scan replays only)
     PointFeat *point = nullptr;
+    bool capture = false;
+    Captured last;
   };
+
+  void capture(size_t s, const TraceOp &op, const formgpu_request &r) {
+    Seq &q = m_seq[s];
+    Captured &c = q.last;
+    switch (op.kind) {
+    case TraceOp::EXTRACT:
+    case TraceOp::COMMIT:
+      c.keypoint_counts.push_back(r.n_planar);
+      c.keypoint_counts.push_back(r.n_point);
+      if (op.kind == TraceOp::EXTRACT && r.planar_out) {
+        c.planar.assign(q.planar, q.planar + r.n_planar);
+        c.point.assign(q.point, q.point + r.n_point);
+      }
+      break;
+    case TraceOp::ASSOCIATE:
+    case TraceOp::ASSOC_LIN:
+      c.counts.insert(c.counts.end(), q.counts.begin(), q.counts.begin() + r.n_counts);
+      if (op.kind == TraceOp::ASSOC_LIN) c.blocks.insert(c.blocks.end(), q.out.begin(), q.out.begin() + 91 * r.n_counts);
+      break;
+    case TraceOp::LINEARIZE:
+      c.blocks.insert(c.blocks.end(), q.out.begin(), q.out.begin() + 91 * op.pairs.size());
+      break;
+    case TraceOp::ERROR:
+      c.errors.insert(c.errors.end(), q.out.begin(), q.out.begin() + op.pairs.size());
+      break;
+    default:
+      break;
+    }
+  }
 
   void ensure_host_buffers() {
     if (m_host_ready) return;

@@ -359,6 +359,36 @@ void formhost_batch_replay_stats(void *r, int seq, uint64_t out[20], double *che
   }
   if (checksum) *checksum = cs;
 }
+/// on != 0: every later run keeps what the calls of its last scan returned for sequence `seq`.
+void formhost_batch_replay_capture(void *r, size_t seq, int on) {
+  auto *b = static_cast<BatchReplay *>(r);
+  if (seq < b->size()) b->capture_last_scan(seq, on != 0);
+}
+
+/// What the calls of the last scan of sequence `seq` returned in the latest run with capture on.
+/// what: 0 pair counts (16 B records), 1 blocks (91 doubles per pair), 2 errors (doubles),
+/// 3 planar / 4 point keypoints (72 / 40 B records, host-scan runs only), 5 keypoint counts
+/// (uint64: extracted planar, point, then committed novel planar, point).  Copies at most `cap`
+/// elements to `out` (may be null) and returns how many there are.
+size_t formhost_batch_replay_captured(void *r, size_t seq, int what, void *out, size_t cap) {
+  auto *b = static_cast<BatchReplay *>(r);
+  if (seq >= b->size()) return 0;
+  const BatchReplay::Captured &c = b->captured(seq);
+  auto copy = [&](const auto &v) {
+    if (out) std::memcpy(out, v.data(), std::min(cap, v.size()) * sizeof(v[0]));
+    return v.size();
+  };
+  switch (what) {
+  case 0: return copy(c.counts);
+  case 1: return copy(c.blocks);
+  case 2: return copy(c.errors);
+  case 3: return copy(c.planar);
+  case 4: return copy(c.point);
+  case 5: return copy(c.keypoint_counts);
+  default: return 0;
+  }
+}
+
 void formhost_batch_replay_reset_stats(void *r) {
   auto *b = static_cast<BatchReplay *>(r);
   for (size_t s = 0; s < b->size(); ++s) {

@@ -250,6 +250,26 @@ class BatchReplay:
     def reset_stats(self):
         self._lib.formhost_batch_replay_reset_stats(self._h)
 
+    def capture_last_scan(self, seq: int, on=True):
+        """on: every later run keeps what the calls of its last scan return for sequence `seq`
+        (see captured)."""
+        self._lib.formhost_batch_replay_capture(self._h, seq, int(on))
+
+    def captured(self, seq: int) -> dict:
+        """What the calls of the last scan of sequence `seq` returned in the latest run with
+        capture on, in call order: pair counts of every association, 91-double blocks of every
+        linearisation, error values, keypoint counts (extracted, then committed) and - for host
+        scans - the keypoints."""
+        out = {}
+        for what, (name, dtype, width) in enumerate((
+                ("counts", _capi.PAIR_COUNT, 1), ("blocks", np.float64, 91), ("errors", np.float64, 1),
+                ("planar", _capi.PLANAR_FEAT, 1), ("point", _capi.POINT_FEAT, 1), ("keypoint_counts", np.uint64, 1))):
+            n = self._lib.formhost_batch_replay_captured(self._h, seq, what, None, 0)
+            a = np.zeros(n, dtype=dtype)
+            self._lib.formhost_batch_replay_captured(self._h, seq, what, _capi.ptr(a), n)
+            out[name] = a.reshape(-1, width) if width > 1 else a
+        return out
+
     def profile_enable(self, on=True):
         _capi.gpu_lib().formgpu_batch_profile_enable(self.batch(), int(on))
 

@@ -83,6 +83,60 @@ def test_batched_replay_is_bit_identical_to_single_contexts():
         assert b2.stats(s) == br.stats(s)
 
 
+def test_captured_last_scan_is_what_its_calls_returned():
+    """capture_last_scan (bench.py --dump-outputs): over a run of several scans, the records kept are
+    those of its LAST scan only - keypoints as the live estimator got them, counts and blocks that
+    add up to the work counters and checksum of a separate run of that one scan - and only for the
+    sequences asked for."""
+    import torch
+
+    from form_b200.pipeline import BatchReplay, Estimator
+
+    n = 8
+    rows, cols = synth.shape("vlp-16")
+    p = _capi.default_est_params(rows, cols, record_trace=1, gtsam_lm_schedule=1)
+    runs = []
+    for seq in (1, 4, 6):
+        scans = [synth.scan("vlp-16", seq, k) for k in range(n)]
+        est = Estimator(p)
+        kp = [est.register_scan(s) for s in scans]
+        runs.append((est, scans, kp[-1]))
+    traces = [est.trace() for est, _, _ in runs]
+    dev = [[torch.from_numpy(s.view(np.uint8)).cuda() for s in scans] for _, scans, _ in runs]
+    torch.cuda.synchronize()
+    got = {}
+    for on_device, ptrs in ((True, [[d.data_ptr() for d in seq] for seq in dev]),
+                            (False, [[s.ctypes.data for s in scans] for _, scans, _ in runs])):
+        # the last scan alone, for its work counters
+        one = BatchReplay(traces, p)
+        one.run(0, n - 1, ptrs, on_device)
+        one.reset_stats()
+        one.run(n - 1, n, ptrs, on_device)
+        # the same scan as the last of a three-scan run with capture on for sequences 0 and 1
+        br = BatchReplay(traces, p)
+        br.run(0, n - 3, ptrs, on_device)
+        br.capture_last_scan(0)
+        br.capture_last_scan(1)
+        br.run(n - 3, n, ptrs, on_device)
+        assert all(len(v) == 0 for v in br.captured(2).values())
+        for s in range(2):
+            c, st = br.captured(s), one.stats(s)
+            kc = [int(v) for v in c["keypoint_counts"]]  # extract, then every commit
+            assert kc[:2] == [st["planar_kp"], st["point_kp"]] and sum(kc[2::2]) == st["novel_planar"]
+            assert int(c["counts"]["n_planar"].sum()) == st["assoc_planar"] > 0
+            assert len(c["blocks"]) == st["lin_pairs"] > 0 and len(c["errors"]) == st["err_pairs"]
+            cs = c["blocks"][:, 90].sum() + c["errors"].sum()
+            assert abs(cs - st["checksum"]) <= 1e-12 * abs(st["checksum"])
+            got[on_device, s] = c
+        br.close()
+        one.close()
+    for s, (_, _, (pl, pt)) in enumerate(runs[:2]):
+        assert len(got[True, s]["planar"]) == 0  # device-resident scans: keypoints stay on the GPU
+        assert got[False, s]["planar"].tobytes() == pl.tobytes() and got[False, s]["point"].tobytes() == pt.tobytes()
+        assert np.array_equal(got[False, s]["counts"], got[True, s]["counts"])
+        assert np.allclose(got[False, s]["blocks"], got[True, s]["blocks"], rtol=1e-12, atol=0)
+
+
 def test_batch_submit_extract_matches_oracle_and_reports_errors():
     import oracle_lib
 

@@ -61,7 +61,8 @@ def ref():
 
             subprocess.call(["make", "-s", "-C", os.path.join(ROOT, "oracle", "ref")])
         if not os.path.exists(REF_LIB):
-            pytest.skip("oracle/_ref/libformref.so is not built (needs /root/reference)")
+            pytest.skip("oracle/_ref/libformref.so is not built: it needs FORM's own sources (oracle/ref/Makefile, "
+                        "REFERENCE=<FORM checkout>)")
         _ref = C.CDLL(REF_LIB)
         for name, (res, args) in _SYMS.items():
             fn = getattr(_ref, name)
