@@ -181,6 +181,7 @@ FORMGPU_SYMBOLS = {
     "formgpu_linearize_device": (_i, [_vp, _vp, _sz, _vp, _sz, _vp]),
     "formgpu_error_device": (_i, [_vp, _vp, _sz, _vp, _sz, _vp]),
     "formgpu_batch_create": (_i, [C.POINTER(Params), _i, _vp, _sz, C.POINTER(_vp)]),
+    "formgpu_batch_create_mixed": (_i, [C.POINTER(Params), _i, _vp, _sz, C.POINTER(_vp)]),
     "formgpu_batch_destroy": (None, [_vp]),
     "formgpu_batch_size": (_sz, [_vp]),
     "formgpu_batch_ctx": (_vp, [_vp, _sz]),
@@ -246,10 +247,12 @@ FORMHOST_SYMBOLS = {
     "formhost_replay_run_device": (_d, [_vp, _sz, _sz, _vp]),
     "formhost_replay_run_device_multi": (_d, [_vp, _sz, _sz, _sz, _vp]),
     "formhost_pool_create": (_vp, [_pest, _sz, _i]),
+    "formhost_pool_create_mixed": (_vp, [_pest, _sz, _i]),
     "formhost_pool_destroy": (None, [_vp]),
     "formhost_pool_stats": (None, [_vp, _vp]),
     "formhost_pool_est_create": (_vp, [_vp, _pest, _sz]),
     "formhost_batch_replay_create": (_vp, [_vp, _sz, _pest, _vp]),
+    "formhost_batch_replay_create_mixed": (_vp, [_vp, _sz, _pest, _vp]),
     "formhost_batch_replay_destroy": (None, [_vp]),
     "formhost_batch_replay_batch": (_vp, [_vp]),
     "formhost_batch_replay_run": (_d, [_vp, _sz, _sz, _vp, _i, _psz]),

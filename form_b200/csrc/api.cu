@@ -88,6 +88,31 @@ void poll_relax(unsigned spins) {
 
 } // namespace formgpu
 
+namespace formgpu {
+
+int validate_params(const formgpu_params &P, std::string &msg) {
+  auto bad = [&](int code, const char *m) {
+    msg = m;
+    return code;
+  };
+  if (P.neighbor_points < 1 || P.neighbor_points > 16)
+    return bad(FORMGPU_ERR_UNSUPPORTED, "neighbor_points must be in [1, 16]");
+  if (P.num_sectors < 1 || P.num_rows < 1 || P.num_columns < 2 * P.neighbor_points + 1 ||
+      P.num_columns > 4096 || P.num_columns / P.num_sectors < 1)
+    return bad(FORMGPU_ERR_UNSUPPORTED,
+               "need 2*neighbor_points < num_columns <= 4096, num_rows >= 1, "
+               "1 <= num_sectors <= num_columns");
+  if (P.planar_feats_per_sector < 0 || P.point_feats_per_sector < 0 || P.min_points < 0)
+    return bad(FORMGPU_ERR_INVALID_ARG, "negative feature counts");
+  if (P.max_window_scans < 2 || P.max_window_scans > kMaxWindow)
+    return bad(FORMGPU_ERR_UNSUPPORTED, "max_window_scans must be in [2, 128]");
+  if (!(P.max_dist_matching > 0) || !(P.sigma > 0))
+    return bad(FORMGPU_ERR_INVALID_ARG, "max_dist_matching and sigma must be positive");
+  return FORMGPU_OK;
+}
+
+} // namespace formgpu
+
 extern "C" {
 
 int formgpu_abi_version(void) { return FORMGPU_ABI_VERSION; }
@@ -119,19 +144,11 @@ const char *formgpu_last_error(const formgpu_ctx *ctx) {
 
 static int create_impl(formgpu_ctx *ctx) {
   const formgpu_params &P = ctx->P;
-  if (P.neighbor_points < 1 || P.neighbor_points > 16)
-    return fail(ctx, FORMGPU_ERR_UNSUPPORTED, "neighbor_points must be in [1, 16]");
-  if (P.num_sectors < 1 || P.num_rows < 1 || P.num_columns < 2 * P.neighbor_points + 1 ||
-      P.num_columns > 4096 || P.num_columns / P.num_sectors < 1)
-    return fail(ctx, FORMGPU_ERR_UNSUPPORTED,
-                "need 2*neighbor_points < num_columns <= 4096, num_rows >= 1, "
-                "1 <= num_sectors <= num_columns");
-  if (P.planar_feats_per_sector < 0 || P.point_feats_per_sector < 0 || P.min_points < 0)
-    return fail(ctx, FORMGPU_ERR_INVALID_ARG, "negative feature counts");
-  if (P.max_window_scans < 2 || P.max_window_scans > kMaxWindow)
-    return fail(ctx, FORMGPU_ERR_UNSUPPORTED, "max_window_scans must be in [2, 128]");
-  if (!(P.max_dist_matching > 0) || !(P.sigma > 0))
-    return fail(ctx, FORMGPU_ERR_INVALID_ARG, "max_dist_matching and sigma must be positive");
+  {
+    std::string msg;
+    const int rc = validate_params(P, msg);
+    if (rc != FORMGPU_OK) return fail(ctx, rc, msg);
+  }
 
   ctx->rows = P.num_rows;
   ctx->cols = P.num_columns;

@@ -20,6 +20,7 @@
 #include <cstdlib>
 #include <functional>
 #include <new>
+#include <tuple>
 
 using namespace formgpu;
 
@@ -329,7 +330,26 @@ int formgpu_batch_create(const formgpu_params *p, int device, void *stream, size
     g_batch_error = "formgpu_batch_create: bad argument";
     return FORMGPU_ERR_INVALID_ARG;
   }
+  const std::vector<formgpu_params> params(n_sequences, *p);
+  return formgpu_batch_create_mixed(params.data(), device, stream, n_sequences, out);
+}
+
+int formgpu_batch_create_mixed(const formgpu_params *params, int device, void *stream, size_t n_sequences,
+                               formgpu_batch **out) {
+  if (!params || !out || n_sequences == 0 || n_sequences > 4096) {
+    g_batch_error = "formgpu_batch_create_mixed: bad argument";
+    return FORMGPU_ERR_INVALID_ARG;
+  }
   *out = nullptr;
+  // every entry is checked before the first CUDA call, so a bad one fails on any machine
+  for (size_t i = 0; i < n_sequences; ++i) {
+    std::string msg;
+    const int rc = validate_params(params[i], msg);
+    if (rc != FORMGPU_OK) {
+      g_batch_error = "formgpu_batch_create: params of sequence " + std::to_string(i) + ": " + msg;
+      return rc;
+    }
+  }
   formgpu_batch *b = new (std::nothrow) formgpu_batch();
   if (!b) return FORMGPU_ERR_CAPACITY;
   b->device = device;
@@ -365,11 +385,14 @@ int formgpu_batch_create(const formgpu_params *p, int device, void *stream, size
   }
   for (size_t i = 0; i < n_sequences; ++i) {
     formgpu_ctx *c = nullptr;
-    const int rc = formgpu_create(p, device, b->stream, &c); // every context shares the batch stream
-    if (rc != FORMGPU_OK) return bail(rc, std::string("formgpu_create: ") + formgpu_last_error(nullptr));
+    const int rc = formgpu_create(&params[i], device, b->stream, &c); // every context shares the batch stream
+    if (rc != FORMGPU_OK)
+      return bail(rc, "formgpu_create (sequence " + std::to_string(i) + "): " + formgpu_last_error(nullptr));
     c->moment_unit = kMomentUnit; // throughput-sized units (kernels.hpp)
     b->ctx.push_back(c);
   }
+  // switches read from the environment when a context is created are the same for every context
+  // of the batch; the batch takes them from its first
   b->moment_cache = b->ctx[0]->moment_cache;
   b->block_dma = b->block_dma && b->moment_cache; // the evaluation kernels write plain blocks
   b->assoc_block_off.assign(n_sequences, kNoBlocks);
@@ -518,7 +541,8 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
 
   // ---- stage 1 ----
   std::function<int()> extract_launcher; // queued after every other group: extraction is the long pole
-  std::vector<std::pair<float4 *, const void *>> scan_uploads; // host scans of this submission
+  // host scans of this submission: device buffer, source, bytes (each sequence's own point count)
+  std::vector<std::tuple<float4 *, const void *, size_t>> scan_uploads;
   {
     std::vector<ExtractArgs> items;
     for (size_t r : by_op[FORMGPU_OP_EXTRACT]) {
@@ -544,7 +568,7 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
           // uploaded ahead of this request (formgpu_batch_prefetch_scan, same stream): adopt the buffer
           std::swap(ctx->d_scan, ctx->d_scan_next);
         } else {
-          scan_uploads.push_back({ctx->d_scan, q.scan});
+          scan_uploads.emplace_back(ctx->d_scan, q.scan, ctx->n_points * sizeof(float4));
         }
         ctx->prefetched_host = nullptr;
         scan_dev = ctx->d_scan;
@@ -568,17 +592,20 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
       live_extract.push_back(r);
     }
     if (!items.empty()) {
+      // ONE launch per kernel whatever the mix of scan shapes (DESIGN.md 6): the grid covers the
+      // largest rows, shared memory is the largest need; a homogeneous submission gets exactly the
+      // grid and shared memory of a single-shape launch
       size_t off = 0;
       const int rc = stage_args(b, items.data(), items.size(), &off);
       if (rc) return rc;
-      const ExtractArgs shape = items[0];
+      const ExtractLaunchShape shape = extract_launch_shape(items.data(), (int)items.size());
       const int n_items = (int)items.size();
-      const size_t scan_bytes = b->ctx[0]->n_points * sizeof(float4);
       extract_launcher = [=]() -> int {
         // on the batch's own stream, right before the kernels that read them (every other group of
         // the submission is already queued ahead): no side stream, no event pair per submission
         for (const auto &u : scan_uploads)
-          BATCH_CUDA(b, cudaMemcpyAsync(u.first, u.second, scan_bytes, cudaMemcpyHostToDevice, b->stream));
+          BATCH_CUDA(b, cudaMemcpyAsync(std::get<0>(u), std::get<1>(u), std::get<2>(u), cudaMemcpyHostToDevice,
+                                        b->stream));
         extract_batch_launch(shape, staged<ExtractArgs>(b, off), n_items, b->many_rows_min, b->stream, b->prof);
         BATCH_CUDA(b, cudaGetLastError());
         return FORMGPU_OK;

@@ -50,6 +50,8 @@ int wait_flag(formgpu_ctx *ctx, int which, unsigned long long seq);
 /// sched_yield() every 64 polls, so that a thread which is only waiting hands its core to one
 /// that has a submit to build.  Without the variable the loop never enters the kernel.
 void poll_relax(unsigned spins);
+/// The parameter checks of formgpu_create that need no GPU: FORMGPU_OK, or an error code and `msg`.
+int validate_params(const formgpu_params &P, std::string &msg);
 
 /// Stage 3 building blocks (api_stage3.cu), also used by the fused association call.
 void relative_pose(const formgpu_pose &Ti, const formgpu_pose &Tj, double rel[12]);

@@ -475,6 +475,7 @@ __global__ void __launch_bounds__(512) extract_select_kernel(ExtractArgs a) {
 __global__ void __launch_bounds__(512) extract_select_batch_kernel(const ExtractArgs *items) {
   __shared__ ExtractArgs s_a;
   load_item_args(s_a, items + blockIdx.y);
+  if ((int)blockIdx.x >= s_a.rows) return; // the grid covers the launch's largest scan
   extract_select_body(s_a, blockIdx.x, 0);
 }
 
@@ -1015,12 +1016,14 @@ __device__ __forceinline__ void extract_normals_thread_body(const ExtractArgs &a
 __global__ void __launch_bounds__(256) extract_normals_batch_kernel(const ExtractArgs *items) {
   __shared__ ExtractArgs s_a;
   load_item_args(s_a, items + blockIdx.y);
+  if ((int)blockIdx.x >= s_a.rows * kNormalSplit) return;
   extract_normals_body(s_a, blockIdx.x, 0);
 }
 
 __global__ void __launch_bounds__(256) extract_normals_rows_kernel(const ExtractArgs *items) {
   __shared__ ExtractArgs s_a;
   load_item_args(s_a, items + blockIdx.y);
+  if ((int)blockIdx.x >= s_a.rows) return;
   extract_normals_thread_body(s_a, blockIdx.x, 0);
 }
 
@@ -1165,6 +1168,7 @@ __global__ void __launch_bounds__(128) extract_pack_kernel(ExtractArgs a) {
 __global__ void __launch_bounds__(128) extract_pack_batch_kernel(const ExtractArgs *items) {
   __shared__ ExtractArgs s_a;
   load_item_args(s_a, items + blockIdx.y);
+  if ((int)blockIdx.x >= s_a.rows) return; // before the item's buffers and its done_counter
   extract_pack_body(s_a, blockIdx.x, 0);
 }
 
@@ -1184,38 +1188,50 @@ size_t extract_normals_smem(int cols, int words, int pr_cap) {
 }
 
 cudaError_t extract_configure(const ExtractArgs &shape) {
-  const int cols = shape.cols, words = shape.words, pr_cap = shape.pr_cap;
-  // the attribute belongs to the function, not to a context: it only ever grows, so that contexts
-  // of different scan shapes can live in one process
+  // the attributes belong to the functions, not to a context: they only ever grow, so that contexts
+  // of different scan shapes can live in one process (a 16x1800 context needs more normals shared
+  // memory than a 64x1024 one created after it)
   static std::mutex mu;
-  static size_t select_hi = 0;
+  static size_t select_hi = 0, normals_hi = 0;
   std::lock_guard<std::mutex> lock(mu);
   select_hi = std::max(select_hi, extract_select_smem(shape));
+  normals_hi = std::max(normals_hi, extract_normals_smem(shape.cols, shape.words, shape.pr_cap));
   cudaError_t e = cudaFuncSetAttribute(extract_select_kernel,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)select_hi);
   if (e != cudaSuccess) return e;
   e = cudaFuncSetAttribute(extract_select_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)select_hi);
   if (e != cudaSuccess) return e;
-  e = cudaFuncSetAttribute(extract_normals_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                           (int)extract_normals_smem(cols, words, pr_cap));
+  e = cudaFuncSetAttribute(extract_normals_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)normals_hi);
   if (e != cudaSuccess) return e;
-  e = cudaFuncSetAttribute(extract_normals_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                           (int)extract_normals_smem(cols, words, pr_cap));
+  e = cudaFuncSetAttribute(extract_normals_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)normals_hi);
   if (e != cudaSuccess) return e;
-  return cudaFuncSetAttribute(extract_normals_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                              (int)extract_normals_smem(cols, words, pr_cap));
+  return cudaFuncSetAttribute(extract_normals_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)normals_hi);
 }
 
-void extract_batch_launch(const ExtractArgs &shape, const ExtractArgs *items_dev, int n_items,
+ExtractLaunchShape extract_launch_shape(const ExtractArgs *items, int n_items) {
+  ExtractLaunchShape sh;
+  for (int i = 0; i < n_items; ++i) {
+    const ExtractArgs &a = items[i];
+    sh.max_rows = std::max(sh.max_rows, a.rows);
+    sh.sum_rows += a.rows;
+    sh.select_smem = std::max(sh.select_smem, extract_select_smem(a));
+    sh.normals_smem = std::max(sh.normals_smem, extract_normals_smem(a.cols, a.words, a.pr_cap));
+    sh.pack_smem = std::max(sh.pack_smem, (size_t)a.pr_cap * sizeof(uint16_t));
+  }
+  return sh;
+}
+
+void extract_batch_launch(const ExtractLaunchShape &sh, const ExtractArgs *items_dev, int n_items,
                           int many_rows_min, cudaStream_t stream, Profiler &prof) {
-  const ExtractArgs &a = shape; // geometry (rows, cols, caps) is common to the batch
-  const dim3 grid(a.rows, n_items);
+  // the items may differ in geometry (rows, cols, sectors, caps): the grid covers the largest rows
+  // (CTAs past their own item's rows leave at once) and shared memory is the largest need
+  const dim3 grid(sh.max_rows, n_items);
   prof.begin(FORMGPU_KG_EXTRACT_SELECT);
   // One warp of every CTA ends up walking the row's greedy selections alone, so what bounds a
   // many-row launch is how many rows are RESIDENT (registers: 2 CTAs of 512 threads per SM, 10
   // of 128).  Launches with more rows than fit at 512 threads use 128-thread CTAs: the parallel
   // part of a row takes four times longer, but five times as many serial walks overlap it.
-  const bool many_rows = a.rows * n_items >= many_rows_min;
+  const bool many_rows = sh.sum_rows >= many_rows_min;
   // many rows: one warp per sector for the speculative walks (six sectors by default) and as many
   // rows resident as the registers allow; FORMGPU_SELECT_THREADS overrides it for tuning
   static const int select_many = [] {
@@ -1231,19 +1247,19 @@ void extract_batch_launch(const ExtractArgs &shape, const ExtractArgs *items_dev
     return e ? std::atoi(e) : 0;
   }();
   for (int r = 0; r <= repeat; ++r)
-    extract_select_batch_kernel<<<grid, select_threads, extract_select_smem(a), stream>>>(items_dev);
+    extract_select_batch_kernel<<<grid, select_threads, sh.select_smem, stream>>>(items_dev);
   prof.end(FORMGPU_KG_EXTRACT_SELECT, 1);
   prof.begin(FORMGPU_KG_EXTRACT_NORMALS);
   // many rows: one thread per pick (one CTA per row); few rows: one warp per pick, four CTAs
   // per row, which spreads a small launch over the whole GPU
   if (many_rows)
-    extract_normals_rows_kernel<<<grid, 256, extract_normals_smem(a.cols, a.words, a.pr_cap), stream>>>(items_dev);
+    extract_normals_rows_kernel<<<grid, 256, sh.normals_smem, stream>>>(items_dev);
   else
-    extract_normals_batch_kernel<<<dim3(a.rows * kNormalSplit, n_items), 256,
-                                   extract_normals_smem(a.cols, a.words, a.pr_cap), stream>>>(items_dev);
+    extract_normals_batch_kernel<<<dim3(sh.max_rows * kNormalSplit, n_items), 256, sh.normals_smem, stream>>>(
+        items_dev);
   prof.end(FORMGPU_KG_EXTRACT_NORMALS, 1);
   prof.begin(FORMGPU_KG_EXTRACT_PACK);
-  extract_pack_batch_kernel<<<grid, 128, (size_t)a.pr_cap * sizeof(uint16_t), stream>>>(items_dev);
+  extract_pack_batch_kernel<<<grid, 128, sh.pack_smem, stream>>>(items_dev);
   prof.end(FORMGPU_KG_EXTRACT_PACK, 1);
 }
 

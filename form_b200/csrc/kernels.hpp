@@ -60,12 +60,22 @@ inline size_t extract_select_smem(const ExtractArgs &a) {
 size_t extract_normals_smem(int cols, int words, int pr_cap);
 /// Launches the three stage-1 kernels.
 void extract_launch(const ExtractArgs &a, int n_scans, cudaStream_t stream, Profiler &prof);
+/// What a batched extraction launch needs of its items' geometry, which may differ from item to
+/// item: the grid covers the largest `rows`, dynamic shared memory is the largest need of each
+/// kernel, and the many-row choice counts the true sum of rows.
+struct ExtractLaunchShape {
+  int max_rows = 0;
+  long long sum_rows = 0;
+  size_t select_smem = 0, normals_smem = 0, pack_smem = 0;
+};
+ExtractLaunchShape extract_launch_shape(const ExtractArgs *items, int n_items);
 /// Same three kernels for n_items scans of DIFFERENT contexts (one ExtractArgs each, in
-/// device memory); `shape` supplies the common geometry.
-/// Launches with at least `many_rows_min` rows (rows x items) use the many-row variants: 128-thread
-/// select CTAs and the thread-per-pick normals kernel, which trade per-row latency for rows in flight.
+/// device memory); `shape` comes from extract_launch_shape over the same items.
+/// Launches with at least `many_rows_min` rows (summed over the items) use the many-row variants:
+/// 128-thread select CTAs and the thread-per-pick normals kernel, which trade per-row latency for
+/// rows in flight.
 constexpr int kManyRowsMin = 1; // measured: +5 % batched throughput over switching at 2 x 148 rows
-void extract_batch_launch(const ExtractArgs &shape, const ExtractArgs *items_dev, int n_items,
+void extract_batch_launch(const ExtractLaunchShape &shape, const ExtractArgs *items_dev, int n_items,
                           int many_rows_min, cudaStream_t stream, Profiler &prof);
 
 // ---- stage 2 (map_assoc.cu, compiled with -fmad=false) ----

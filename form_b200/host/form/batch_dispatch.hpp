@@ -27,12 +27,17 @@ namespace form {
 
 class BatchDispatcher {
 public:
+  /// n_sequences sequences with the same hot-path parameters.
   BatchDispatcher(const HotPathParams &hp, int device, size_t n_sequences, int max_window_scans = 64,
                   std::chrono::microseconds linger = std::chrono::microseconds(200))
-      : m_linger(linger), m_slots(n_sequences) {
-    formgpu_params g = to_formgpu_params(hp);
-    g.max_window_scans = max_window_scans;
-    const int rc = formgpu_batch_create(&g, device, nullptr, n_sequences, &m_batch);
+      : BatchDispatcher(std::vector<formgpu_params>(n_sequences, to_formgpu_params(hp, max_window_scans)), device,
+                        linger) {}
+  /// One sequence per entry of `params` (hot-path parameters and window of its context): sensors of
+  /// different shapes and parameter variants in one batch (formgpu_batch_create_mixed).
+  BatchDispatcher(const std::vector<formgpu_params> &params, int device,
+                  std::chrono::microseconds linger = std::chrono::microseconds(200))
+      : m_linger(linger), m_slots(params.size()), m_params(params) {
+    const int rc = formgpu_batch_create_mixed(params.data(), device, nullptr, params.size(), &m_batch);
     if (rc != FORMGPU_OK)
       throw HotPathError(std::string("formgpu_batch_create: ") + formgpu_batch_last_error(nullptr));
     m_thread = std::thread([this] { run(); });
@@ -52,6 +57,8 @@ public:
   size_t size() const { return m_slots.size(); }
   formgpu_batch *batch() const { return m_batch; }
   formgpu_ctx *ctx(size_t i) const { return formgpu_batch_ctx(m_batch, i); }
+  /// The parameters sequence i's context was created with.
+  const formgpu_params &params(size_t i) const { return m_params[i]; }
   uint64_t submits() const { return m_submits; }
   uint64_t requests() const { return m_requests; }
 
@@ -142,6 +149,7 @@ private:
   std::mutex m_mu;
   std::condition_variable m_cv_work, m_cv_done;
   std::vector<Slot> m_slots;
+  std::vector<formgpu_params> m_params;
   size_t m_pending = 0, m_busy = 0;
   std::chrono::steady_clock::time_point m_first_post;
   bool m_stop = false;

@@ -29,13 +29,19 @@ public:
   /// traces[s] drives sequence s.  `stream` = cudaStream_t of the batch (nullptr: private).
   BatchReplay(const std::vector<const Trace *> &traces, const HotPathParams &hp, int device,
               void *stream, int max_window_scans)
+      : BatchReplay(traces, std::vector<formgpu_params>(traces.size(), to_formgpu_params(hp, max_window_scans)),
+                    device, stream) {}
+  /// traces[s] drives sequence s, whose context is configured by params[s] (sensor shape and
+  /// hot-path parameters may differ between sequences: formgpu_batch_create_mixed).
+  BatchReplay(const std::vector<const Trace *> &traces, const std::vector<formgpu_params> &params, int device,
+              void *stream)
       : m_traces(traces), m_stats(traces.size()), m_seq(traces.size()) {
-    formgpu_params g = to_formgpu_params(hp);
-    g.max_window_scans = max_window_scans;
-    m_points = (size_t)g.num_rows * (size_t)g.num_columns;
+    if (params.size() != traces.size()) throw HotPathError("BatchReplay: one params entry per trace");
+    for (size_t s = 0; s < params.size(); ++s)
+      m_seq[s].points = (size_t)params[s].num_rows * (size_t)params[s].num_columns;
     if (const char *env = std::getenv("FORM_REPLAY_SKIP_KEYPOINTS")) m_skip_keypoints = env[0] == '1'; // probe only
     if (const char *env = std::getenv("FORM_REPLAY_PREFETCH")) m_prefetch = env[0] != '0';
-    const int rc = formgpu_batch_create(&g, device, stream, traces.size(), &m_batch);
+    const int rc = formgpu_batch_create_mixed(params.data(), device, stream, traces.size(), &m_batch);
     if (rc != FORMGPU_OK)
       throw HotPathError(std::string("formgpu_batch_create: ") + formgpu_batch_last_error(nullptr));
     for (auto &s : m_seq) {
@@ -117,7 +123,7 @@ public:
       // a log is being reprocessed: the next scan of the sequence is known, so its upload starts
       // as soon as the extraction of this one has completed (the scan buffers alternate)
       if (m_prefetch && !m_on_device && op.kind == TraceOp::EXTRACT && m_scans && op.scan + 1 < m_seq[s].scan_hi)
-        formgpu_batch_prefetch_scan(m_batch, s, m_scans[s][op.scan + 1], m_points);
+        formgpu_batch_prefetch_scan(m_batch, s, m_scans[s][op.scan + 1], m_seq[s].points);
     }
     ++m_rounds;
   }
@@ -156,6 +162,7 @@ public:
 private:
   struct Seq {
     size_t op = 0, end = 0;
+    size_t points = 0;  // rows x cols of the sequence's sensor
     size_t scan_hi = 0; // scans [.., scan_hi) belong to the run in progress
     size_t last_begin = 0; // first op of scan scan_hi - 1
     uint64_t cur_scan = 0;
@@ -164,6 +171,7 @@ private:
     std::vector<double> out;
     PlanarFeat *planar = nullptr; // page-locked (host-scan replays only)
     PointFeat *point = nullptr;
+    size_t planar_cap = 0, point_cap = 0;
     bool capture = false;
     Captured last;
   };
@@ -199,12 +207,13 @@ private:
 
   void ensure_host_buffers() {
     if (m_host_ready) return;
-    formgpu_ctx *c0 = formgpu_batch_ctx(m_batch, 0);
-    m_planar_cap = formgpu_max_planar(c0);
-    m_point_cap = formgpu_max_point(c0);
-    for (auto &s : m_seq) {
-      s.planar = static_cast<PlanarFeat *>(formgpu_alloc_pinned(m_planar_cap * sizeof(PlanarFeat)));
-      s.point = static_cast<PointFeat *>(formgpu_alloc_pinned(m_point_cap * sizeof(PointFeat)));
+    for (size_t i = 0; i < m_seq.size(); ++i) {
+      Seq &s = m_seq[i];
+      formgpu_ctx *c = formgpu_batch_ctx(m_batch, i);
+      s.planar_cap = formgpu_max_planar(c);
+      s.point_cap = formgpu_max_point(c);
+      s.planar = static_cast<PlanarFeat *>(formgpu_alloc_pinned(s.planar_cap * sizeof(PlanarFeat)));
+      s.point = static_cast<PointFeat *>(formgpu_alloc_pinned(s.point_cap * sizeof(PointFeat)));
       if (!s.planar || !s.point) throw HotPathError("formgpu_alloc_pinned failed");
       m_pinned.emplace_back(s.planar, formgpu_free_pinned);
       m_pinned.emplace_back(s.point, formgpu_free_pinned);
@@ -222,13 +231,13 @@ private:
       r.op = FORMGPU_OP_EXTRACT;
       r.flags = on_device ? FORMGPU_REQ_SCAN_ON_DEVICE : 0u;
       r.scan = scans[op.scan];
-      r.n_points = m_points;
+      r.n_points = q.points;
       r.scan_idx = op.scan;
       if (!on_device && !m_skip_keypoints) {
         r.planar_out = reinterpret_cast<formgpu_planar_feat *>(q.planar);
-        r.planar_cap = m_planar_cap;
+        r.planar_cap = q.planar_cap;
         r.point_out = reinterpret_cast<formgpu_point_feat *>(q.point);
-        r.point_cap = m_point_cap;
+        r.point_cap = q.point_cap;
       }
       break;
     case TraceOp::MAP_REBUILD:
@@ -301,7 +310,7 @@ private:
       q.cur_np = r.n_planar;
       q.cur_nq = r.n_point;
       st.scans += 1;
-      st.points += m_points;
+      st.points += q.points;
       st.planar_kp += r.n_planar;
       st.point_kp += r.n_point;
       break;
@@ -366,8 +375,6 @@ private:
   std::vector<ReplayStats> m_stats;
   std::vector<Seq> m_seq;
   formgpu_batch *m_batch = nullptr;
-  size_t m_points = 0;
-  size_t m_planar_cap = 0, m_point_cap = 0;
   bool m_host_ready = false;
   bool m_on_device = false;
   bool m_skip_keypoints = false; // development probe: host scans in, only the counts back

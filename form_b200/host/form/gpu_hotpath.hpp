@@ -17,7 +17,7 @@ static_assert(sizeof(PlanarFeat) == sizeof(formgpu_planar_feat), "PlanarFeat lay
 static_assert(sizeof(PointFeat) == sizeof(formgpu_point_feat), "PointFeat layout");
 static_assert(sizeof(PointXYZf) == sizeof(formgpu_point4f), "PointXYZf layout");
 
-inline formgpu_params to_formgpu_params(const HotPathParams &p) {
+inline formgpu_params to_formgpu_params(const HotPathParams &p, int max_window_scans = 64) {
   formgpu_params g;
   formgpu_default_params(&g);
   g.neighbor_points = (int32_t)p.neighbor_points;
@@ -34,7 +34,20 @@ inline formgpu_params to_formgpu_params(const HotPathParams &p) {
   g.max_dist_matching = p.max_dist_matching;
   g.min_dist_map = p.min_dist_map;
   g.sigma = p.sigma;
+  g.max_window_scans = max_window_scans;
   return g;
+}
+
+/// Field-wise equality of two context configurations (every field a context reads).
+inline bool same_formgpu_params(const formgpu_params &a, const formgpu_params &b) {
+  return a.neighbor_points == b.neighbor_points && a.num_sectors == b.num_sectors &&
+         a.planar_feats_per_sector == b.planar_feats_per_sector &&
+         a.point_feats_per_sector == b.point_feats_per_sector && a.min_points == b.min_points &&
+         a.num_columns == b.num_columns && a.num_rows == b.num_rows && a.max_window_scans == b.max_window_scans &&
+         a.planar_threshold == b.planar_threshold && a.radius == b.radius &&
+         a.min_norm_squared == b.min_norm_squared && a.max_norm_squared == b.max_norm_squared &&
+         a.max_dist_matching == b.max_dist_matching && a.min_dist_map == b.min_dist_map && a.sigma == b.sigma &&
+         a.max_batch_scans == b.max_batch_scans;
 }
 
 class GpuHotPath : public HotPath {

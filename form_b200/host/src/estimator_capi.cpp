@@ -4,6 +4,7 @@
 #include "form/capi_impl.hpp"
 
 #include <atomic>
+#include <stdexcept>
 #include <thread>
 
 using namespace form;
@@ -11,9 +12,26 @@ using namespace form::capi;
 
 namespace {
 std::string g_error;
+int window_of(const formhost_est_params &p) { return p.hot.max_window_scans > 0 ? p.hot.max_window_scans : 64; }
 std::shared_ptr<HotPath> make_gpu(const HotPathParams &hp, const formhost_est_params &p) {
-  const int window = p.hot.max_window_scans > 0 ? p.hot.max_window_scans : 64;
-  return std::make_shared<GpuHotPath>(hp, p.device, nullptr, window);
+  return std::make_shared<GpuHotPath>(hp, p.device, nullptr, window_of(p));
+}
+/// What the context of an estimator with params p is created with (hot-path part and window).
+formgpu_params context_params(const formhost_est_params &p) {
+  return to_formgpu_params(Estimator::hotpath_params(to_estimator_params(p)), window_of(p));
+}
+/// One context configuration per entry; every entry must name the same device.
+std::vector<formgpu_params> context_params(const formhost_est_params *p, size_t n, const char *who) {
+  if (!p || n == 0) throw std::invalid_argument(std::string(who) + ": no params");
+  std::vector<formgpu_params> out;
+  for (size_t i = 0; i < n; ++i) {
+    if (p[i].device != p[0].device)
+      throw std::invalid_argument(std::string(who) + ": params of sequence " + std::to_string(i) + " name device " +
+                                  std::to_string(p[i].device) + ", sequence 0 device " +
+                                  std::to_string(p[0].device) + " (a batch runs on one GPU)");
+    out.push_back(context_params(p[i]));
+  }
+  return out;
 }
 } // namespace
 
@@ -186,6 +204,21 @@ void *formhost_pool_create(const formhost_est_params *p, size_t n_sequences, int
     return nullptr;
   }
 }
+/// As formhost_pool_create, with sequence i configured by p[i] (n entries): sensor shape and hot-path
+/// parameters may differ, and so may the host-side fields (smoother, key scans, disable_smoothing,
+/// gtsam_lm_schedule), which formhost_pool_est_create takes from its own argument.  Every entry
+/// must name the same device.
+void *formhost_pool_create_mixed(const formhost_est_params *p, size_t n, int linger_us) {
+  try {
+    auto *pool = new std::shared_ptr<BatchDispatcher>(std::make_shared<BatchDispatcher>(
+        context_params(p, n, "formhost_pool_create_mixed"), p[0].device,
+        std::chrono::microseconds(linger_us > 0 ? linger_us : 200)));
+    return pool;
+  } catch (const std::exception &e) {
+    g_error = e.what();
+    return nullptr;
+  }
+}
 void formhost_pool_destroy(void *pool) { delete static_cast<std::shared_ptr<BatchDispatcher> *>(pool); }
 void formhost_pool_stats(void *pool, uint64_t out[2]) {
   auto &d = *static_cast<std::shared_ptr<BatchDispatcher> *>(pool);
@@ -196,6 +229,13 @@ void *formhost_pool_est_create(void *pool, const formhost_est_params *p, size_t 
   auto &d = *static_cast<std::shared_ptr<BatchDispatcher> *>(pool);
   if (seq >= d->size()) {
     g_error = "formhost_pool_est_create: sequence index outside the pool";
+    return nullptr;
+  }
+  // the context of sequence seq already exists: an estimator whose hot-path parameters differ from
+  // it would silently run with the context's
+  if (!p || !same_formgpu_params(context_params(*p), d->params(seq))) {
+    g_error = "formhost_pool_est_create: the hot-path parameters differ from those sequence " + std::to_string(seq) +
+              " of the pool was created with";
     return nullptr;
   }
   auto make = [&](const HotPathParams &, const formhost_est_params &) -> std::shared_ptr<HotPath> {
@@ -215,6 +255,20 @@ void *formhost_batch_replay_create(const void *const *traces, size_t n, const fo
     const Estimator::Params ep = to_estimator_params(*p);
     const int window = p->hot.max_window_scans > 0 ? p->hot.max_window_scans : 64;
     return new BatchReplay(tr, Estimator::hotpath_params(ep), p->device, stream, window);
+  } catch (const std::exception &e) {
+    g_error = e.what();
+    return nullptr;
+  }
+}
+/// As formhost_batch_replay_create, with sequence s configured by p[s] (n entries; sensor shape and
+/// hot-path parameters may differ).  Every entry must name the same device.
+void *formhost_batch_replay_create_mixed(const void *const *traces, size_t n, const formhost_est_params *p,
+                                         void *stream) {
+  try {
+    if (!traces) throw std::invalid_argument("formhost_batch_replay_create_mixed: no traces");
+    std::vector<const Trace *> tr;
+    for (size_t i = 0; i < n; ++i) tr.push_back(static_cast<const Trace *>(traces[i]));
+    return new BatchReplay(tr, context_params(p, n, "formhost_batch_replay_create_mixed"), p[0].device, stream);
   } catch (const std::exception &e) {
     g_error = e.what();
     return nullptr;

@@ -197,15 +197,32 @@ def run_device_multi(replays, first: int, last: int, dev_ptrs_per_replay) -> flo
     return t
 
 
+def _params_list(params, n, what: str):
+    """`params` as a ctypes array of n EstParams: one EstParams for every sequence, or a list
+    with one entry per sequence."""
+    if isinstance(params, _capi.EstParams):
+        return None
+    params = list(params)
+    if len(params) != n:
+        raise ValueError(f"{what}: {len(params)} params for {n} sequences")
+    return (_capi.EstParams * n)(*params)
+
+
 class BatchReplay:
     """Lock-step replay of the recorded traces of several sequences through
-    formgpu_batch_submit: calls of the same kind share one launch per kernel."""
+    formgpu_batch_submit: calls of the same kind share one launch per kernel.  `params` is one
+    EstParams for every sequence, or a list with one per trace (sensor shapes and hot-path
+    parameters may then differ from sequence to sequence)."""
 
-    def __init__(self, traces, params: _capi.EstParams, stream: int | None = None):
+    def __init__(self, traces, params, stream: int | None = None):
         self._lib = _capi.host_lib()
         self.n = len(traces)
         arr = (C.c_void_p * self.n)(*traces)
-        self._h = self._lib.formhost_batch_replay_create(arr, self.n, C.byref(params), C.c_void_p(stream or 0))
+        mixed = _params_list(params, self.n, "BatchReplay")
+        if mixed is None:
+            self._h = self._lib.formhost_batch_replay_create(arr, self.n, C.byref(params), C.c_void_p(stream or 0))
+        else:
+            self._h = self._lib.formhost_batch_replay_create_mixed(arr, self.n, mixed, C.c_void_p(stream or 0))
         if not self._h:
             raise RuntimeError("formhost_batch_replay_create failed: " +
                                (self._lib.formhost_last_error() or b"").decode())
@@ -304,16 +321,32 @@ class EstimatorPool:
     """Many live form::Estimators on one GPU behind a batching dispatcher
     (form/batch_dispatch.hpp): the hot-path calls of the pool's sequences are funnelled
     through formgpu_batch_submit, so calls of the same kind share one launch per kernel.
-    Drive each estimator from its own thread (ctypes releases the GIL inside a call)."""
+    Drive each estimator from its own thread (ctypes releases the GIL inside a call).
 
-    def __init__(self, params: _capi.EstParams, n_sequences: int, linger_us: int = 200):
+    `params` is one EstParams for all `n_sequences` estimators, or a list with one entry per
+    estimator (then `n_sequences` may be omitted): sensors of different shapes and parameter
+    variants, host-side fields included, in one pool."""
+
+    def __init__(self, params, n_sequences: int | None = None, linger_us: int = 200):
         self._lib = _capi.host_lib()
-        self.params = params
-        self.n = n_sequences
-        self._h = self._lib.formhost_pool_create(C.byref(params), n_sequences, linger_us)
+        if isinstance(params, _capi.EstParams):
+            if n_sequences is None:
+                raise TypeError("EstimatorPool: n_sequences is required with a single EstParams")
+            self.params = params
+            self.n = n_sequences
+            self._seq_params = [params] * n_sequences
+            self._h = self._lib.formhost_pool_create(C.byref(params), n_sequences, linger_us)
+        else:
+            self._seq_params = list(params)
+            if n_sequences is not None and n_sequences != len(self._seq_params):
+                raise ValueError(f"EstimatorPool: {len(self._seq_params)} params for {n_sequences} sequences")
+            self.params = self._seq_params
+            self.n = len(self._seq_params)
+            arr = _params_list(self._seq_params, self.n, "EstimatorPool")
+            self._h = self._lib.formhost_pool_create_mixed(arr, self.n, linger_us)
         if not self._h:
             raise RuntimeError("formhost_pool_create failed: " + (self._lib.formhost_last_error() or b"").decode())
-        self.estimators = [PooledEstimator(self, i) for i in range(n_sequences)]
+        self.estimators = [PooledEstimator(self, i) for i in range(self.n)]
 
     def stats(self) -> dict:
         out = np.zeros(2, np.uint64)
@@ -345,9 +378,9 @@ class PooledEstimator(EstimatorBase):
     """form::Estimator of one sequence of an EstimatorPool (same calls as Estimator)."""
 
     def __init__(self, pool: EstimatorPool, seq: int):
-        self.params = pool.params
-        self.rows, self.cols = pool.params.hot.num_rows, pool.params.hot.num_columns
-        self._h = pool._lib.formhost_pool_est_create(pool._h, C.byref(pool.params), seq)
+        self.params = pool._seq_params[seq]
+        self.rows, self.cols = self.params.hot.num_rows, self.params.hot.num_columns
+        self._h = pool._lib.formhost_pool_est_create(pool._h, C.byref(self.params), seq)
         if not self._h:
             raise RuntimeError("formhost_pool_est_create failed: " + self._last_error())
         cap = self.rows * self.cols

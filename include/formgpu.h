@@ -352,9 +352,19 @@ typedef struct formgpu_request {
 
 typedef struct formgpu_batch formgpu_batch;
 
-/* `stream`: cudaStream_t shared by all sequences of the batch, or NULL for a private one. */
+/* `stream`: cudaStream_t shared by all sequences of the batch, or NULL for a private one.
+ * Every sequence is configured by `p`: formgpu_batch_create_mixed with p repeated. */
 int formgpu_batch_create(const formgpu_params *p, int device, void *stream, size_t n_sequences,
                          formgpu_batch **out);
+/* A batch whose sequence i is configured by params[i] (n_sequences entries): sensors of different
+ * shapes and parameter variants share one launch per kernel.  Every field of formgpu_params may
+ * differ from sequence to sequence.  Shared by the whole batch: `device`, `stream`, and the switches
+ * read from the environment when a context is created (FORMGPU_CELL_BUCKETS,
+ * FORMGPU_STREAM_LINEARIZE), which the batch takes from its first context.  Every entry goes
+ * through formgpu_create's parameter checks before any CUDA call; when one fails,
+ * formgpu_batch_last_error(NULL) names the index of its sequence. */
+int formgpu_batch_create_mixed(const formgpu_params *params, int device, void *stream, size_t n_sequences,
+                               formgpu_batch **out);
 void formgpu_batch_destroy(formgpu_batch *b);
 size_t formgpu_batch_size(const formgpu_batch *b);
 /* The context of sequence i, for the calls that are not batched (formgpu_get_matches,
