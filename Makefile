@@ -15,7 +15,7 @@ CXXFLAGS  := -O3 -std=c++17 -fPIC -pthread -ffp-contract=off -Wall -Iinclude -If
 LIBDIR    := form_b200/lib
 OBJDIR    := build/obj
 
-GPU_OBJS  := $(OBJDIR)/extract.o $(OBJDIR)/map_assoc.o $(OBJDIR)/linearize.o $(OBJDIR)/moments.o $(OBJDIR)/api.o $(OBJDIR)/api_stage2.o $(OBJDIR)/api_stage3.o $(OBJDIR)/api_batch.o $(OBJDIR)/comm.o
+GPU_OBJS  := $(OBJDIR)/extract.o $(OBJDIR)/map_assoc.o $(OBJDIR)/linearize.o $(OBJDIR)/moments.o $(OBJDIR)/api.o $(OBJDIR)/api_stage2.o $(OBJDIR)/api_stage3.o $(OBJDIR)/api_batch.o $(OBJDIR)/comm.o $(OBJDIR)/organize.o $(OBJDIR)/api_cloud.o
 HOST_SRCS := $(wildcard form_b200/host/src/*.cpp)
 HOST_OBJS := $(HOST_SRCS:form_b200/host/src/%.cpp=$(OBJDIR)/host_%.o)
 CSRC_HDRS := $(wildcard form_b200/csrc/*.hpp) $(wildcard form_b200/csrc/*.cuh) include/formgpu.h
@@ -36,6 +36,10 @@ $(OBJDIR)/extract.o: form_b200/csrc/extract.cu $(CSRC_HDRS)
 	$(NVCC) $(NVFLAGS) $(EXACT) -Xptxas -v -c $< -o $@
 
 $(OBJDIR)/map_assoc.o: form_b200/csrc/map_assoc.cu $(CSRC_HDRS)
+	@mkdir -p $(OBJDIR)
+	$(NVCC) $(NVFLAGS) $(EXACT) -Xptxas -v -c $< -o $@
+
+$(OBJDIR)/organize.o: form_b200/csrc/organize.cu $(CSRC_HDRS)
 	@mkdir -p $(OBJDIR)
 	$(NVCC) $(NVFLAGS) $(EXACT) -Xptxas -v -c $< -o $@
 

@@ -100,6 +100,127 @@ class Request(C.Structure):
 (OP_EXTRACT, OP_MAP_REBUILD, OP_ASSOCIATE, OP_ASSOC_LIN, OP_LINEARIZE, OP_ERROR, OP_COMMIT,
  OP_REMOVE) = range(8)
 REQ_SCAN_ON_DEVICE = 1
+REQ_CLOUD = 2
+
+# ---- raw sensor clouds (formgpu_cloud_format, rule R8) ---------------------------
+CLOUD_ABSENT = -1
+FIELD_F32, FIELD_F64, FIELD_U8, FIELD_U16, FIELD_U32, FIELD_U32_NS = range(6)
+ROW_FROM_FIELD, ROW_FROM_ELEVATION = range(2)
+COL_FROM_FIELD, COL_FROM_TIME, COL_FROM_AZIMUTH = range(3)
+CLOUD_STATS = np.dtype([(k, "<u8") for k in (
+    "records", "placed", "pixels", "dropped_nonfinite", "dropped_zero", "dropped_time", "dropped_row",
+    "dropped_col")])
+
+
+class CloudFormat(C.Structure):
+    """formgpu_cloud_format: record layout of a raw cloud and how it is organised."""
+
+    _fields_ = [
+        ("stride", C.c_uint32), ("off_x", C.c_int32), ("off_y", C.c_int32), ("off_z", C.c_int32),
+        ("xyz_type", C.c_int32), ("off_row", C.c_int32), ("row_type", C.c_int32), ("off_col", C.c_int32),
+        ("col_type", C.c_int32), ("off_time", C.c_int32), ("time_type", C.c_int32), ("row_source", C.c_int32),
+        ("col_source", C.c_int32), ("azimuth_dir", C.c_int32), ("scan_period", C.c_double),
+        ("azimuth_origin", C.c_double), ("beam_elevations", C.POINTER(C.c_double)), ("max_records", C.c_uint64),
+    ]
+
+    def beams(self):
+        """The beam-elevation table as a numpy array (None without one)."""
+        b = getattr(self, "_beams", None)
+        return None if b is None else np.array(b)
+
+
+assert C.sizeof(CloudFormat) == 88
+
+_ROW_FROM = {"field": ROW_FROM_FIELD, "ring": ROW_FROM_FIELD, "row": ROW_FROM_FIELD, "elevation": ROW_FROM_ELEVATION}
+_COL_FROM = {"field": COL_FROM_FIELD, "col": COL_FROM_FIELD, "time": COL_FROM_TIME, "azimuth": COL_FROM_AZIMUTH}
+_INDEX_TYPES = {np.dtype("u1"): FIELD_U8, np.dtype("<u2"): FIELD_U16, np.dtype("<u4"): FIELD_U32}
+
+
+def cloud_format(dtype, *, row_from: str | None = None, col_from: str | None = None, scan_period: float = 0.1,
+                 azimuth_origin: float = 0.0, azimuth_dir: int = 1, beams=None,
+                 max_records: int = 1 << 20) -> CloudFormat:
+    """formgpu_cloud_format of the records of a numpy structured dtype.  Fields by name: x, y, z
+    (f4 or f8, all three alike), ring or row (u1/u2/u4), col (u1/u2/u4), t or time (f4/f8 seconds
+    since the scan started, or u4 nanoseconds).  Row source: the ring / row field when there is one,
+    else the beam-elevation table `beams` (radians, one per row, strictly monotonic).  Column source:
+    the col field, else the time field, else the azimuth (column c centred at
+    azimuth_origin + azimuth_dir * 2 pi c / cols).  `row_from` ("ring" | "elevation") and `col_from`
+    ("col" | "time" | "azimuth") override the choice."""
+    dt = np.dtype(dtype)
+    names = dt.names or ()
+
+    def field(*cands):
+        for n in cands:
+            if n in names:
+                sub, off = dt.fields[n][0], dt.fields[n][1]
+                if sub.shape:
+                    raise ValueError(f"cloud field {n!r} must be a scalar")
+                return n, sub, off
+        return None, None, CLOUD_ABSENT
+
+    xyz = [field(a) for a in "xyz"]
+    if any(f[0] is None for f in xyz):
+        raise ValueError(f"cloud records need fields x, y, z; got {names}")
+    kinds = {f[1].newbyteorder("<") if f[1].byteorder == ">" else f[1] for f in xyz}
+    if kinds == {np.dtype("<f4")}:
+        xyz_type = FIELD_F32
+    elif kinds == {np.dtype("<f8")}:
+        xyz_type = FIELD_F64
+    else:
+        raise ValueError(f"x, y, z must all be float32 or all float64; got {sorted(map(str, kinds))}")
+    if any(f[1].byteorder == ">" for f in xyz):
+        raise ValueError("big-endian coordinates are not supported")
+    rname, rtype, roff = field("ring", "row")
+    cname, ctype, coff = field("col")
+    tname, ttype, toff = field("t", "time")
+
+    def index_type(name, sub):
+        if sub is None:
+            return 0
+        if sub not in _INDEX_TYPES:
+            raise ValueError(f"cloud field {name!r}: {sub} is not u1, u2 or u4")
+        return _INDEX_TYPES[sub]
+
+    if ttype is None:
+        time_type = 0
+    elif ttype == np.dtype("<f4"):
+        time_type = FIELD_F32
+    elif ttype == np.dtype("<f8"):
+        time_type = FIELD_F64
+    elif ttype == np.dtype("<u4"):
+        time_type = FIELD_U32_NS
+    else:
+        raise ValueError(f"cloud field {tname!r}: {ttype} is not f4, f8 or u4 (nanoseconds)")
+    if row_from is None:
+        row_from = "ring" if rname else "elevation"
+    if col_from is None:
+        col_from = "col" if cname else ("time" if tname else "azimuth")
+    if row_from not in _ROW_FROM:
+        raise ValueError(f"row_from must be one of {sorted(_ROW_FROM)}, not {row_from!r}")
+    if col_from not in _COL_FROM:
+        raise ValueError(f"col_from must be one of {sorted(_COL_FROM)}, not {col_from!r}")
+    f = CloudFormat(stride=dt.itemsize, off_x=xyz[0][2], off_y=xyz[1][2], off_z=xyz[2][2], xyz_type=xyz_type,
+                    off_row=roff, row_type=index_type(rname, rtype), off_col=coff, col_type=index_type(cname, ctype),
+                    off_time=toff, time_type=time_type, row_source=_ROW_FROM[row_from],
+                    col_source=_COL_FROM[col_from], azimuth_dir=int(azimuth_dir), scan_period=float(scan_period),
+                    azimuth_origin=float(azimuth_origin), max_records=int(max_records))
+    if beams is not None:
+        set_beams(f, beams)
+    return f
+
+
+def set_beams(fmt: CloudFormat, beams) -> None:
+    """Point fmt.beam_elevations at a copy of `beams` (radians) that lives as long as fmt."""
+    arr = (C.c_double * len(beams))(*[float(b) for b in beams])
+    fmt._beams = arr
+    fmt.beam_elevations = C.cast(arr, C.POINTER(C.c_double))
+
+
+def check_cloud_format(fmt: CloudFormat, rows: int, cols: int) -> tuple[int, str]:
+    """formgpu_cloud_format_check: (status, message); needs no GPU."""
+    buf = C.create_string_buffer(512)
+    rc = gpu_lib().formgpu_cloud_format_check(C.byref(fmt), rows, cols, buf, len(buf))
+    return rc, buf.value.decode()
 
 
 def default_est_params(rows: int = 64, cols: int = 1024, **overrides) -> EstParams:
@@ -191,6 +312,12 @@ FORMGPU_SYMBOLS = {
     "formgpu_batch_done": (_i, [_vp]),
     "formgpu_batch_prefetch_scan": (_i, [_vp, _sz, _vp, _sz]),
     "formgpu_batch_last_error": (C.c_char_p, [_vp]),
+    "formgpu_cloud_format_check": (_i, [_vp, _i, _i, _vp, _sz]),
+    "formgpu_set_cloud_format": (_i, [_vp, _vp]),
+    "formgpu_organize": (_i, [_vp, _vp, _sz, _vp, _vp]),
+    "formgpu_extract_cloud": (_i, [_vp, _vp, _sz, _u64, _vp, _sz, _psz, _vp, _sz, _psz]),
+    "formgpu_cloud_stats_last": (_i, [_vp, _vp]),
+    "formgpu_batch_prefetch_cloud": (_i, [_vp, _sz, _vp, _sz]),
     "formgpu_batch_profile_enable": (_i, [_vp, _i]),
     "formgpu_batch_profile_read": (_i, [_vp, _vp, _vp]),
     "formgpu_batch_launch_count": (_u64, [_vp]),
@@ -262,6 +389,9 @@ FORMHOST_SYMBOLS = {
     "formhost_batch_replay_reset_stats": (None, [_vp]),
     "formhost_batch_replay_capture": (None, [_vp, _sz, _i]),
     "formhost_batch_replay_captured": (_sz, [_vp, _sz, _i, _vp, _sz]),
+    "formhost_est_set_cloud_format": (_i, [_vp, _vp]),
+    "formhost_est_register_cloud": (_i, [_vp, _vp, _sz, _vp, _sz, _psz, _vp, _sz, _psz]),
+    "formhost_est_cloud_stats": (_i, [_vp, _vp]),
     **estimator_symbols("formhost_"),
 }
 

@@ -68,6 +68,37 @@ class Context:
             _capi.ptr(self._point_buf), self.max_point, C.byref(npt)))
         return self._planar_buf[: npl.value].copy(), self._point_buf[: npt.value].copy()
 
+    # -- raw clouds (rule R8) ----------------------------------------------------------
+    def set_cloud_format(self, fmt: _capi.CloudFormat):
+        """formgpu_set_cloud_format: the record layout of the clouds organize / extract_cloud take."""
+        self._check(self._lib.formgpu_set_cloud_format(self._h, C.byref(fmt)))
+        self.cloud_format = fmt
+
+    def organize(self, records: np.ndarray):
+        """formgpu_organize: -> (scan (rows*cols,) POINT4F, stats CLOUD_STATS record)."""
+        records = np.ascontiguousarray(records)
+        scan = np.zeros(self.rows * self.cols, dtype=_capi.POINT4F)
+        stats = np.zeros(1, dtype=_capi.CLOUD_STATS)
+        self._check(self._lib.formgpu_organize(self._h, _capi.ptr(records), len(records), _capi.ptr(scan),
+                                               _capi.ptr(stats)))
+        return scan, stats[0]
+
+    def extract_cloud(self, records: np.ndarray, scan_idx: int):
+        """formgpu_extract_cloud: extract() of a raw cloud; returns (planar, point) records."""
+        records = np.ascontiguousarray(records)
+        npl, npt = C.c_size_t(), C.c_size_t()
+        self._check(self._lib.formgpu_extract_cloud(
+            self._h, _capi.ptr(records), len(records), scan_idx,
+            _capi.ptr(self._planar_buf), self.max_planar, C.byref(npl),
+            _capi.ptr(self._point_buf), self.max_point, C.byref(npt)))
+        return self._planar_buf[: npl.value].copy(), self._point_buf[: npt.value].copy()
+
+    def cloud_stats(self):
+        """formgpu_cloud_stats_last as a CLOUD_STATS record."""
+        stats = np.zeros(1, dtype=_capi.CLOUD_STATS)
+        self._check(self._lib.formgpu_cloud_stats_last(self._h, _capi.ptr(stats)))
+        return stats[0]
+
     def extract_device(self, scan_dev_ptr: int, n: int, scan_idx: int):
         npl, npt = C.c_size_t(), C.c_size_t()
         self._check(self._lib.formgpu_extract_device(self._h, C.c_void_p(scan_dev_ptr), n, scan_idx,

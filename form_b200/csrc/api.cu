@@ -350,6 +350,7 @@ void formgpu_destroy(formgpu_ctx *ctx) {
   comm_release(ctx);
   F(ctx->d_stage_planar); F(ctx->d_stage_point);
   F(ctx->d_scan_next);
+  F(ctx->d_records); F(ctx->d_pixel_keys); F(ctx->d_cloud_tab); F(ctx->d_cloud_stats); H(ctx->h_cloud_stats);
   if (ctx->ev_prefetch) cudaEventDestroy(ctx->ev_prefetch);
   if (ctx->h_flags) cudaFreeHost(const_cast<unsigned long long *>(ctx->h_flags));
   H(ctx->h_counts); H(ctx->h_planar); H(ctx->h_point); H(ctx->h_upload);
@@ -531,6 +532,11 @@ static int extract_run(formgpu_ctx *ctx, const float4 *scan_dev, uint64_t scan_i
   extract_launch(a, 1, ctx->stream, ctx->prof);
   FORMGPU_CUDA(ctx, cudaGetLastError());
   return extract_finish(ctx, a, scan_idx);
+}
+
+int formgpu::extract_run_scan(formgpu_ctx *ctx, const float4 *scan_dev, uint64_t scan_idx, bool host_records,
+                              formgpu_planar_feat *direct_planar, formgpu_point_feat *direct_point) {
+  return extract_run(ctx, scan_dev, scan_idx, host_records, direct_planar, direct_point);
 }
 
 extern "C" {

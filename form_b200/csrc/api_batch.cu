@@ -542,17 +542,30 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
   // ---- stage 1 ----
   std::function<int()> extract_launcher; // queued after every other group: extraction is the long pole
   // host scans of this submission: device buffer, source, bytes (each sequence's own point count)
-  std::vector<std::tuple<float4 *, const void *, size_t>> scan_uploads;
+  std::vector<std::tuple<void *, const void *, size_t>> scan_uploads;
   {
     std::vector<ExtractArgs> items;
+    // raw clouds of this submission (FORMGPU_REQ_CLOUD): organised into their sequences' scan buffers
+    // by one launch per kernel, queued right before the extraction
+    std::vector<OrganizeArgs> cloud_items;
+    std::vector<formgpu_ctx *> cloud_ctx;
+    size_t max_records = 0, max_pixels = 0;
     for (size_t r : by_op[FORMGPU_OP_EXTRACT]) {
       formgpu_request &q = reqs[r];
       formgpu_ctx *ctx = b->ctx[q.sequence];
+      const bool cloud = (q.flags & FORMGPU_REQ_CLOUD) != 0;
+      if (cloud) {
+        const int rc = cloud_check_request(ctx, q.scan, q.n_points, "extract (cloud)");
+        if (rc) {
+          set_status(q, rc);
+          continue;
+        }
+      }
       if (!q.scan) {
         set_status(q, fail(ctx, FORMGPU_ERR_INVALID_ARG, "extract: null scan"));
         continue;
       }
-      if (q.n_points != ctx->n_points) {
+      if (!cloud && q.n_points != ctx->n_points) {
         set_status(q, fail(ctx, FORMGPU_ERR_BAD_SCAN_SIZE,
                            "Provided scan does not match the expected size " +
                                std::to_string(ctx->n_points) + " != " + std::to_string(q.n_points)));
@@ -563,8 +576,26 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
       formgpu_planar_feat *dp = nullptr;
       formgpu_point_feat *dq = nullptr;
       bool host_records = false;
+      if (cloud) {
+        const unsigned char *rec = reinterpret_cast<const unsigned char *>(q.scan);
+        if (!on_device) {
+          if (!(ctx->prefetched_cloud == q.scan && ctx->prefetched_cloud_n == q.n_points) && q.n_points)
+            scan_uploads.emplace_back(ctx->d_records, q.scan, q.n_points * ctx->cloud.stride);
+          rec = ctx->d_records;
+        }
+        ctx->prefetched_cloud = nullptr;
+        ctx->prefetched_host = nullptr; // a prefetched organised scan is discarded, as for another pointer
+        cloud_items.push_back(cloud_args(ctx, rec, q.n_points));
+        cloud_ctx.push_back(ctx);
+        ctx->cloud_last_n = q.n_points;
+        max_records = std::max(max_records, q.n_points);
+        max_pixels = std::max(max_pixels, ctx->n_points);
+        scan_dev = ctx->d_scan;
+      }
       if (!on_device) {
-        if (ctx->d_scan_next && ctx->prefetched_host == q.scan) {
+        if (cloud) {
+          // organised on the device into d_scan (above)
+        } else if (ctx->d_scan_next && ctx->prefetched_host == q.scan) {
           // uploaded ahead of this request (formgpu_batch_prefetch_scan, same stream): adopt the buffer
           std::swap(ctx->d_scan, ctx->d_scan_next);
         } else {
@@ -600,12 +631,26 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
       if (rc) return rc;
       const ExtractLaunchShape shape = extract_launch_shape(items.data(), (int)items.size());
       const int n_items = (int)items.size();
+      size_t off_cloud = 0;
+      if (!cloud_items.empty()) {
+        const int rc2 = stage_args(b, cloud_items.data(), cloud_items.size(), &off_cloud);
+        if (rc2) return rc2;
+      }
+      const int n_cloud = (int)cloud_items.size();
       extract_launcher = [=]() -> int {
         // on the batch's own stream, right before the kernels that read them (every other group of
         // the submission is already queued ahead): no side stream, no event pair per submission
         for (const auto &u : scan_uploads)
           BATCH_CUDA(b, cudaMemcpyAsync(std::get<0>(u), std::get<1>(u), std::get<2>(u), cudaMemcpyHostToDevice,
                                         b->stream));
+        if (n_cloud) {
+          organize_batch_launch(staged<OrganizeArgs>(b, off_cloud), n_cloud, max_records, max_pixels, b->stream,
+                                b->prof);
+          BATCH_CUDA(b, cudaGetLastError());
+          for (formgpu_ctx *c : cloud_ctx)
+            BATCH_CUDA(b, cudaMemcpyAsync(c->h_cloud_stats, c->d_cloud_stats, kOrgStats * sizeof(unsigned),
+                                          cudaMemcpyDeviceToHost, b->stream));
+        }
         extract_batch_launch(shape, staged<ExtractArgs>(b, off), n_items, b->many_rows_min, b->stream, b->prof);
         BATCH_CUDA(b, cudaGetLastError());
         return FORMGPU_OK;
@@ -1055,6 +1100,22 @@ int formgpu_batch_prefetch_scan(formgpu_batch *b, size_t sequence, const formgpu
   BATCH_CUDA(b, cudaMemcpyAsync(ctx->d_scan_next, scan, n_points * sizeof(float4), cudaMemcpyHostToDevice,
                                 b->stream));
   ctx->prefetched_host = scan;
+  return FORMGPU_OK;
+}
+
+int formgpu_batch_prefetch_cloud(formgpu_batch *b, size_t sequence, const void *records, size_t n) {
+  if (!b || sequence >= b->ctx.size() || !records)
+    return bfail(b, FORMGPU_ERR_INVALID_ARG, "formgpu_batch_prefetch_cloud: bad argument");
+  formgpu_ctx *ctx = b->ctx[sequence];
+  const int rc = cloud_check_request(ctx, records, n, "formgpu_batch_prefetch_cloud");
+  if (rc) return bfail(b, rc, formgpu_last_error(ctx));
+  BATCH_CUDA(b, cudaSetDevice(b->device));
+  // d_records is free: the submission that last read it has been waited for; same stream as the
+  // organisation that will read it, so no event is needed
+  if (n)
+    BATCH_CUDA(b, cudaMemcpyAsync(ctx->d_records, records, n * ctx->cloud.stride, cudaMemcpyHostToDevice, b->stream));
+  ctx->prefetched_cloud = records;
+  ctx->prefetched_cloud_n = n;
   return FORMGPU_OK;
 }
 

@@ -83,6 +83,18 @@ void extract_direct_targets(formgpu_ctx *ctx, formgpu_planar_feat *planar_out, s
 int extract_widen(formgpu_ctx *ctx, uint64_t scan_idx, formgpu_planar_feat *planar_out, size_t planar_cap,
                   formgpu_point_feat *point_out, size_t point_cap);
 
+/// The whole of stage 1 on a scan already in device memory (formgpu_extract after its upload).
+int extract_run_scan(formgpu_ctx *ctx, const float4 *scan_dev, uint64_t scan_idx, bool host_records,
+                     formgpu_planar_feat *direct_planar, formgpu_point_feat *direct_point);
+
+/// Raw clouds (api_cloud.cu): the checks of formgpu_set_cloud_format; the boundary tables of rule R8
+/// ([cols + 1] azimuth | [rows - 1] ascending beam midpoints; desc = beam table given top-down); the
+/// argument block of one organisation into the context's scan buffer; the checks of one cloud request.
+int check_cloud_format(const formgpu_cloud_format &f, int rows, int cols, std::string &msg);
+void cloud_tables(const formgpu_cloud_format &f, int rows, int cols, std::vector<double2> &tab, int &desc);
+OrganizeArgs cloud_args(formgpu_ctx *ctx, const unsigned char *records_dev, size_t n);
+int cloud_check_request(formgpu_ctx *ctx, const void *records, size_t n, const char *who);
+
 /// Reparative rebuild: uploads the request of this context on `stream` and fills the two
 /// MapArgs and the region (cursor + hash tables) that must be zero before the build.
 /// upload = false: the request is left in ctx->h_map_req (ctx->map_req_bytes) for the caller to

@@ -183,6 +183,19 @@ struct formgpu_ctx {
   void *direct_probe[2] = {nullptr, nullptr};
   void *direct_alias[2] = {nullptr, nullptr};
 
+  // ---- raw clouds (formgpu_set_cloud_format; organize.cu writes the organised scan to d_scan) ----
+  bool have_cloud = false;
+  formgpu_cloud_format cloud{};          // beam_elevations is not kept (the tables below are)
+  int cloud_el_desc = 0;
+  unsigned char *d_records = nullptr;    // record staging, cloud.max_records * cloud.stride bytes
+  unsigned long long *d_pixel_keys = nullptr; // [rows * cols]
+  double2 *d_cloud_tab = nullptr;        // [cols + 1] azimuth boundaries | [rows - 1] beam midpoints
+  unsigned *d_cloud_stats = nullptr;     // [8] outcome counters of the last organisation
+  unsigned *h_cloud_stats = nullptr;     // pinned copy, queued behind the gather kernel
+  size_t cloud_last_n = 0;
+  const void *prefetched_cloud = nullptr; // formgpu_batch_prefetch_cloud: records already in d_records
+  size_t prefetched_cloud_n = 0;
+
   // ---- current scan ----
   bool have_current = false;
   uint64_t cur_scan = 0;

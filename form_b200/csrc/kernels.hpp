@@ -78,6 +78,32 @@ constexpr int kManyRowsMin = 1; // measured: +5 % batched throughput over switch
 void extract_batch_launch(const ExtractLaunchShape &shape, const ExtractArgs *items_dev, int n_items,
                           int many_rows_min, cudaStream_t stream, Profiler &prof);
 
+// ---- raw clouds -> organised scans (organize.cu, compiled with -fmad=false; rule R8) ----
+// outcome counters of one organisation (formgpu_cloud_stats order; slot 0 is filled by the host)
+constexpr int kOrgStatPlaced = 1, kOrgStatPixels = 2, kOrgStatNonfinite = 3, kOrgStatZero = 4,
+              kOrgStatTime = 5, kOrgStatRow = 6, kOrgStatCol = 7, kOrgStats = 8;
+struct OrganizeArgs {
+  const unsigned char *records; // n records of `stride` bytes (device)
+  unsigned n, stride;
+  int off_x, off_y, off_z, off_row, off_col, off_time; // byte offsets, -1 = absent
+  int xyz_type, row_type, col_type, time_type;         // FORMGPU_FIELD_*
+  int row_source, col_source;                          // FORMGPU_ROW_FROM_* / FORMGPU_COL_FROM_*
+  int rows, cols;
+  int az_dir, el_desc; // column direction (+1 / -1); beam table given top-down
+  double scan_period;
+  const double2 *az_tab;    // [cols + 1] (cos, sin) of the column boundaries
+  const double2 *el_tab;    // [rows - 1] (cos, sin) of the beam midpoints, ascending
+  unsigned long long *keys; // [rows * cols] winner key per pixel
+  float4 *scan;             // [rows * cols] organised output (the context's scan buffer)
+  unsigned *stats;          // [kOrgStats]
+};
+/// clear + scatter + gather of one cloud on `stream`.
+void organize_launch(const OrganizeArgs &a, cudaStream_t stream, Profiler &prof);
+/// The same three kernels for n_items clouds of different contexts in one launch each; the grids
+/// cover the largest record count and the largest pixel count of the items.
+void organize_batch_launch(const OrganizeArgs *items_dev, int n_items, size_t max_records, size_t max_pixels,
+                           cudaStream_t stream, Profiler &prof);
+
 // ---- stage 2 (map_assoc.cu, compiled with -fmad=false) ----
 struct MapArgs {
   int type;            // 0 planar, 1 point

@@ -198,6 +198,36 @@ public:
     point.assign(m_point, m_point + r.n_point);
   }
 
+  /// Not batched: straight on the sequence's context.  Only call while no request of this sequence
+  /// is in flight (before its first scan, or between scans).
+  void set_cloud_format(const formgpu_cloud_format &fmt) override {
+    const int rc = formgpu_set_cloud_format(m_pool->ctx(m_seq), &fmt);
+    if (rc != FORMGPU_OK) fail(rc);
+  }
+
+  /// A FORMGPU_REQ_CLOUD extraction: the pool's clouds are organised by one launch per kernel.
+  void extract_cloud(const void *records, size_t n, uint64_t scan_idx, std::vector<PlanarFeat> &planar,
+                     std::vector<PointFeat> &point) override {
+    formgpu_request r{};
+    r.op = FORMGPU_OP_EXTRACT;
+    r.flags = FORMGPU_REQ_CLOUD;
+    r.scan = static_cast<const formgpu_point4f *>(records);
+    r.n_points = n;
+    r.scan_idx = scan_idx;
+    r.planar_out = reinterpret_cast<formgpu_planar_feat *>(m_planar);
+    r.planar_cap = m_planar_cap;
+    r.point_out = reinterpret_cast<formgpu_point_feat *>(m_point);
+    r.point_cap = m_point_cap;
+    run(r);
+    planar.assign(m_planar, m_planar + r.n_planar);
+    point.assign(m_point, m_point + r.n_point);
+  }
+
+  void cloud_stats(formgpu_cloud_stats &s) override {
+    const int rc = formgpu_cloud_stats_last(m_pool->ctx(m_seq), &s);
+    if (rc != FORMGPU_OK) fail(rc);
+  }
+
   void map_rebuild(const ScanPose *poses, size_t n_poses) override {
     formgpu_request r{};
     r.op = FORMGPU_OP_MAP_REBUILD;
@@ -295,7 +325,7 @@ private:
     std::string msg = formgpu_last_error(m_pool->ctx(m_seq));
     const std::string batch = m_pool->batch_error();
     if (!batch.empty()) msg += (msg.empty() ? "" : "; ") + std::string("batch: ") + batch;
-    throw HotPathError(std::string("formgpu error ") + std::to_string(rc) + ": " + msg);
+    throw HotPathError(std::string("formgpu error ") + std::to_string(rc) + ": " + msg, rc);
   }
 
   std::shared_ptr<BatchDispatcher> m_pool;

@@ -203,6 +203,31 @@ struct Estimator {
 
   std::tuple<std::vector<PlanarFeat>, std::vector<PointFeat>>
   register_scan(const PointXYZf *scan, size_t n) noexcept {
+    return register_impl([&](size_t scan_idx, std::vector<PlanarFeat> &planar, std::vector<PointFeat> &point) {
+      m_hotpath->extract(scan, n, scan_idx, planar, point);
+    });
+  }
+
+  /// register_scan on a raw sensor cloud: n records in the layout given to set_cloud_format (a
+  /// driver's unordered points, missing returns absent).  They are organised into the scan on the
+  /// device (rule R8, DESIGN.md §4); every later stage is register_scan's.  Errors (no format, more
+  /// records than the format's max_records, ...) are reported through last_error().
+  std::tuple<std::vector<PlanarFeat>, std::vector<PointFeat>> register_cloud(const void *records,
+                                                                              size_t n) noexcept {
+    return register_impl([&](size_t scan_idx, std::vector<PlanarFeat> &planar, std::vector<PointFeat> &point) {
+      m_hotpath->extract_cloud(records, n, scan_idx, planar, point);
+    });
+  }
+
+  /// Record layout and organisation rule of the clouds register_cloud receives (throws HotPathError).
+  void set_cloud_format(const formgpu_cloud_format &fmt) { m_hotpath->set_cloud_format(fmt); }
+
+  size_t icp_iterations() const { return m_icp_iterations; }
+
+private:
+  /// form.cpp:40-114; `extract` is the feature extraction step (form.cpp:53-55) of the input at hand
+  template <typename Extract>
+  std::tuple<std::vector<PlanarFeat>, std::vector<PointFeat>> register_impl(Extract &&extract) noexcept {
     std::tuple<std::vector<PlanarFeat>, std::vector<PointFeat>> keypoints;
     struct ScanBracket { // tells a pooled hot path that this sequence is inside register_scan
       HotPath &hp;
@@ -215,7 +240,7 @@ struct Estimator {
       const size_t scan_idx = m_constraints.step(prediction);
 
       // ---- feature extraction (form.cpp:53-55) ----
-      m_hotpath->extract(scan, n, scan_idx, std::get<0>(keypoints), std::get<1>(keypoints));
+      extract(scan_idx, std::get<0>(keypoints), std::get<1>(keypoints));
       const size_t num_keypoints = std::get<0>(keypoints).size() + std::get<1>(keypoints).size();
 
       // ---- world map at the latest smoothed poses (form.cpp:61-65) ----
@@ -268,9 +293,6 @@ struct Estimator {
     return keypoints;
   }
 
-  size_t icp_iterations() const { return m_icp_iterations; }
-
-private:
   std::string m_last_error;
   size_t m_icp_iterations = 0;
   std::vector<double> m_first_blocks;

@@ -102,6 +102,19 @@ public:
   const PlanarFeat *planar_buffer() const { return m_planar; }
   const PointFeat *point_buffer() const { return m_point; }
 
+  void set_cloud_format(const formgpu_cloud_format &fmt) override { check(formgpu_set_cloud_format(m_ctx, &fmt)); }
+
+  void extract_cloud(const void *records, size_t n, uint64_t scan_idx, std::vector<PlanarFeat> &planar,
+                     std::vector<PointFeat> &point) override {
+    size_t np = 0, nq = 0;
+    check(formgpu_extract_cloud(m_ctx, records, n, scan_idx, reinterpret_cast<formgpu_planar_feat *>(m_planar),
+                                m_planar_cap, &np, reinterpret_cast<formgpu_point_feat *>(m_point), m_point_cap, &nq));
+    planar.assign(m_planar, m_planar + np);
+    point.assign(m_point, m_point + nq);
+  }
+
+  void cloud_stats(formgpu_cloud_stats &s) override { check(formgpu_cloud_stats_last(m_ctx, &s)); }
+
   /// Scan already resident in device memory; nothing is copied back.
   void extract_device(const void *scan_dev, size_t n, uint64_t scan_idx, size_t &n_planar,
                       size_t &n_point) {
@@ -172,7 +185,8 @@ private:
   void check(int rc) const {
     if (rc != FORMGPU_OK)
       throw HotPathError(std::string("formgpu error ") + std::to_string(rc) + ": " +
-                         formgpu_last_error(m_ctx));
+                             formgpu_last_error(m_ctx),
+                         rc);
   }
   formgpu_ctx *m_ctx = nullptr;
   PlanarFeat *m_planar = nullptr; // page-locked, formgpu_max_planar entries

@@ -12,6 +12,7 @@
 
 #include "form/pose3.hpp"
 #include "form/types.hpp"
+#include "formgpu.h"
 
 #include <cstdint>
 #include <stdexcept>
@@ -63,6 +64,8 @@ struct ScanPose {
 class HotPathError : public std::runtime_error {
 public:
   using std::runtime_error::runtime_error;
+  HotPathError(const std::string &msg, int code_) : std::runtime_error(msg), code(code_) {}
+  int code = 0; // FORMGPU_* status of the failing call, 0 when not from the C-ABI
 };
 
 class HotPath {
@@ -79,6 +82,20 @@ public:
   /// "current scan" whose keypoints later calls match and commit.
   virtual void extract(const PointXYZf *scan, size_t n, uint64_t scan_idx,
                        std::vector<PlanarFeat> &planar, std::vector<PointFeat> &point) = 0;
+
+  /// Raw sensor clouds (formgpu_set_cloud_format / formgpu_extract_cloud): the record layout of the
+  /// clouds extract_cloud() receives, then extract() of the organised cloud (rule R8).  Hot paths that
+  /// do not organise clouds (the CPU oracle, trace recording) keep these defaults.
+  virtual void set_cloud_format(const formgpu_cloud_format &) {
+    throw HotPathError("this hot path does not organise raw clouds", FORMGPU_ERR_UNSUPPORTED);
+  }
+  virtual void extract_cloud(const void *, size_t, uint64_t, std::vector<PlanarFeat> &, std::vector<PointFeat> &) {
+    throw HotPathError("this hot path does not organise raw clouds", FORMGPU_ERR_UNSUPPORTED);
+  }
+  /// Counters of the last organisation (formgpu_cloud_stats_last).
+  virtual void cloud_stats(formgpu_cloud_stats &) {
+    throw HotPathError("this hot path does not organise raw clouds", FORMGPU_ERR_UNSUPPORTED);
+  }
 
   /// KeypointMap::to_voxel_map for both keypoint types (map.hpp:137,
   /// form.cpp:61-65): re-transform every stored keypoint with the given poses

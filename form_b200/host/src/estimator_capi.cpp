@@ -64,6 +64,58 @@ int formhost_est_register_scan(void *h, const formgpu_point4f *scan, size_t n,
   return est_register_scan(static_cast<EstimatorHandle *>(h), scan, n, planar, planar_cap, n_planar,
                            point, point_cap, n_point);
 }
+/// Raw sensor clouds, for stand-alone and pooled estimators alike (in a pool every sequence has
+/// its own format).  Set the format before the first formhost_est_register_cloud of the estimator,
+/// or between its scans.
+int formhost_est_set_cloud_format(void *h, const formgpu_cloud_format *fmt) {
+  auto *e = static_cast<EstimatorHandle *>(h);
+  if (!fmt) {
+    e->error = "formhost_est_set_cloud_format: null format";
+    return FORMGPU_ERR_INVALID_ARG;
+  }
+  try {
+    e->est->set_cloud_format(*fmt);
+  } catch (const HotPathError &x) {
+    e->error = x.what();
+    return x.code ? x.code : FORMGPU_ERR_STATE;
+  } catch (const std::exception &x) {
+    e->error = x.what();
+    return FORMGPU_ERR_STATE;
+  }
+  return FORMGPU_OK;
+}
+/// Estimator::register_cloud: as formhost_est_register_scan, with n records of the estimator's cloud
+/// format as input.
+int formhost_est_register_cloud(void *h, const void *records, size_t n, formgpu_planar_feat *planar,
+                                size_t planar_cap, size_t *n_planar, formgpu_point_feat *point, size_t point_cap,
+                                size_t *n_point) {
+  auto *e = static_cast<EstimatorHandle *>(h);
+  auto kp = e->est->register_cloud(records, n);
+  if (!e->est->last_error().empty() && std::get<0>(kp).empty() && std::get<1>(kp).empty() &&
+      e->est->last_error() != e->error) {
+    e->error = e->est->last_error();
+    return FORMGPU_ERR_STATE;
+  }
+  const auto &pl = std::get<0>(kp);
+  const auto &pt = std::get<1>(kp);
+  if (n_planar) *n_planar = pl.size();
+  if (n_point) *n_point = pt.size();
+  if (pl.size() > planar_cap || pt.size() > point_cap) return FORMGPU_ERR_CAPACITY;
+  if (planar && !pl.empty()) std::memcpy(planar, pl.data(), pl.size() * sizeof(PlanarFeat));
+  if (point && !pt.empty()) std::memcpy(point, pt.data(), pt.size() * sizeof(PointFeat));
+  return FORMGPU_OK;
+}
+/// Counters of the estimator's last organised cloud.
+int formhost_est_cloud_stats(void *h, formgpu_cloud_stats *out) {
+  auto *e = static_cast<EstimatorHandle *>(h);
+  try {
+    e->backend->cloud_stats(*out);
+  } catch (const HotPathError &x) {
+    e->error = x.what();
+    return x.code ? x.code : FORMGPU_ERR_STATE;
+  }
+  return FORMGPU_OK;
+}
 void formhost_est_pose(void *h, formgpu_pose *out) { est_pose(static_cast<EstimatorHandle *>(h), out); }
 int formhost_est_window(void *h, formgpu_scan_pose *out, size_t cap, size_t *n) {
   return est_window(static_cast<EstimatorHandle *>(h), out, cap, n);

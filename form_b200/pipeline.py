@@ -61,6 +61,35 @@ class EstimatorBase:
             raise RuntimeError(f"register_scan failed (rc={rc})")
         return self._planar[: a.value].copy(), self._point[: b.value].copy()
 
+    def set_cloud_format(self, fmt: _capi.CloudFormat):
+        """formhost_est_set_cloud_format: record layout of the clouds register_cloud takes."""
+        rc = self._lib().formhost_est_set_cloud_format(self._h, C.byref(fmt))
+        if rc != 0:
+            raise RuntimeError(f"set_cloud_format failed (rc={rc}): "
+                               + (self._lib().formhost_est_error(self._h) or b"").decode())
+        self.cloud_format = fmt
+
+    def register_cloud(self, records: np.ndarray):
+        """Estimator::register_cloud: register_scan of a raw sensor cloud (records of the format given
+        to set_cloud_format), organised on the device.  Returns (planar, point) keypoints."""
+        records = np.ascontiguousarray(records)
+        a, b = C.c_size_t(), C.c_size_t()
+        rc = self._lib().formhost_est_register_cloud(self._h, _capi.ptr(records), len(records),
+                                                     _capi.ptr(self._planar), self._planar.shape[0], C.byref(a),
+                                                     _capi.ptr(self._point), self._point.shape[0], C.byref(b))
+        if rc != 0:
+            raise RuntimeError(f"register_cloud failed (rc={rc}): "
+                               + (self._lib().formhost_est_error(self._h) or b"").decode())
+        return self._planar[: a.value].copy(), self._point[: b.value].copy()
+
+    def cloud_stats(self):
+        """Counters of the last organised cloud as a CLOUD_STATS record."""
+        out = np.zeros(1, dtype=_capi.CLOUD_STATS)
+        rc = self._lib().formhost_est_cloud_stats(self._h, _capi.ptr(out))
+        if rc != 0:
+            raise RuntimeError(f"cloud_stats failed (rc={rc}): " + (self._lib().formhost_est_error(self._h) or b"").decode())
+        return out[0]
+
     def pose(self) -> np.ndarray:
         """Estimator::current_lidar_estimate as a POSE record."""
         out = np.zeros(1, dtype=_capi.POSE)
@@ -325,9 +354,13 @@ class EstimatorPool:
 
     `params` is one EstParams for all `n_sequences` estimators, or a list with one entry per
     estimator (then `n_sequences` may be omitted): sensors of different shapes and parameter
-    variants, host-side fields included, in one pool."""
+    variants, host-side fields included, in one pool.
 
-    def __init__(self, params, n_sequences: int | None = None, linger_us: int = 200):
+    `cloud_formats`: one CloudFormat (or None) per sequence; the estimators of sequences with a format
+    take raw clouds through register_cloud - formats may differ from sequence to sequence, and cloud
+    and organised-scan sequences share the pool's launches."""
+
+    def __init__(self, params, n_sequences: int | None = None, linger_us: int = 200, cloud_formats=None):
         self._lib = _capi.host_lib()
         if isinstance(params, _capi.EstParams):
             if n_sequences is None:
@@ -347,6 +380,18 @@ class EstimatorPool:
         if not self._h:
             raise RuntimeError("formhost_pool_create failed: " + (self._lib.formhost_last_error() or b"").decode())
         self.estimators = [PooledEstimator(self, i) for i in range(self.n)]
+        if cloud_formats is not None:
+            cloud_formats = list(cloud_formats)
+            if len(cloud_formats) != self.n:
+                self.close()
+                raise ValueError(f"EstimatorPool: {len(cloud_formats)} cloud formats for {self.n} sequences")
+            try:
+                for est, fmt in zip(self.estimators, cloud_formats):
+                    if fmt is not None:
+                        est.set_cloud_format(fmt)
+            except Exception:
+                self.close()
+                raise
 
     def stats(self) -> dict:
         out = np.zeros(2, np.uint64)

@@ -13,6 +13,14 @@ PooledEstimator on its own thread; all of them share one pool (one formgpu batch
 --pool-size caps the estimators per pool.  Output, in evalio's CSV layout:
 OUT/synthetic/<sensor>/<seq>/<variant>.csv per run, gt.csv once per sequence, and OUT/summary.csv
 (variant, sequence, scans, hz, ATE rmse against ground truth).
+
+Recorded logs join the same pool: `--log NAME=DIR` (repeatable) names a directory of raw clouds
+(form_b200/clouds.py: .npy structured arrays or KITTI .bin), organised on the GPU through
+register_cloud.  Their shape and record format come from --rows/--cols and the cloud flags of
+run_sequence (--row-from, --col-from, --scan-period, --beams).  Every scan of the log is run; its
+runs land in OUT/log/NAME/<variant>.csv, and a log has no ground truth, so its ate_rmse stays empty.
+
+    python -m form_b200.sweep --log mylog=DIR --rows 16 --cols 1800 --sensor vlp-16 --out sweeps
 """
 from __future__ import annotations
 
@@ -24,7 +32,7 @@ import time
 
 import numpy as np
 
-from . import _capi, synth, trajectory
+from . import _capi, clouds, synth, trajectory
 from .pipeline import EstimatorPool
 from .run_sequence import relative_gt
 
@@ -112,50 +120,82 @@ def est_params(rows: int, cols: int, overrides: dict) -> _capi.EstParams:
     return p
 
 
+def parse_log(spec: str) -> tuple[str, str]:
+    """`NAME=DIR` -> (name, dir)."""
+    name, eq, path = spec.partition("=")
+    name = name.strip()
+    if not eq or not name or not path or "/" in name or name in (".", ".."):
+        raise ValueError(f"--log {spec!r}: expected NAME=DIR with a NAME usable as a file name")
+    return name, path
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description=__doc__.split("\n\n")[0])
     ap.add_argument("--sensor", action="append", choices=sorted(synth.SENSORS),
-                    help="sensor (repeatable; default os1-64)")
+                    help="sensor (repeatable; default os1-64 when no --log is given)")
     ap.add_argument("--sequences", default="0", help="comma-separated sequence ids")
     ap.add_argument("--scans", type=int, default=100)
     ap.add_argument("--rate-hz", type=float, default=10.0)
     ap.add_argument("--variant", action="append",
                     help="NAME or NAME:key=value,... (repeatable; default: one variant 'form')")
+    ap.add_argument("--log", action="append", default=[], help="NAME=DIR: a recorded log of raw clouds (repeatable)")
     ap.add_argument("--pool-size", type=int, default=0,
                     help="estimators per pool (default 0: every run in one pool)")
     ap.add_argument("--linger-us", type=int, default=200)
     ap.add_argument("--out", default="sweeps")
+    clouds.add_format_args(ap)
     args = ap.parse_args(argv)
 
-    sensors = args.sensor or ["os1-64"]
+    sensors = args.sensor or ([] if args.log else ["os1-64"])
     sequences = [int(s) for s in args.sequences.split(",") if s.strip()]
     try:
         variants = parse_variants(args.variant or ["form"])
+        logs = [parse_log(spec) for spec in args.log]
     except ValueError as e:
         ap.error(str(e))
-    if args.scans < 1 or not sequences:
+    if len({name for name, _ in logs}) != len(logs):
+        ap.error("duplicate --log name")
+    if logs and not (args.rows and args.cols):
+        ap.error("--log needs the scan shape of the recorded sensor: --rows and --cols")
+    if args.scans < 1 or (sensors and not sequences):
         ap.error("need at least one scan and one sequence")
 
-    runs = [(sensor, seq, name, overrides) for sensor in sensors for seq in sequences for name, overrides in variants]
-    scans = {}
+    # a source is ("synthetic", sensor, seq) or ("log", name); a run is (source, variant, overrides)
+    sources = [("synthetic", sensor, seq) for sensor in sensors for seq in sequences] + [("log", n) for n, _ in logs]
+    scans, formats, shapes = {}, {}, {}
     for sensor in sensors:
         for seq in sequences:
-            scans[sensor, seq] = [synth.scan(sensor, seq, k) for k in range(args.scans)]
-    params = [est_params(*synth.shape(sensor), overrides) for sensor, _, _, overrides in runs]
+            scans["synthetic", sensor, seq] = [synth.scan(sensor, seq, k) for k in range(args.scans)]
+            shapes["synthetic", sensor, seq] = synth.shape(sensor)
+    for name, path in logs:
+        recs = clouds.read_dir(path)
+        max_records = args.max_records if args.max_records > 0 else max(len(c) for c in recs)
+        fmt_args = argparse.Namespace(**{**vars(args), "max_records": max_records})
+        try:
+            formats["log", name] = clouds.format_from_args(recs[0].dtype, fmt_args, args.rows)
+        except ValueError as e:
+            ap.error(f"--log {name}: {e}")
+        scans["log", name] = recs
+        shapes["log", name] = (args.rows, args.cols)
+    runs = [(src, name, overrides) for src in sources for name, overrides in variants]
+    params = [est_params(*shapes[src], overrides) for src, _, overrides in runs]
+    cloud_formats = [formats.get(src) for src, _, _ in runs]
 
     size = args.pool_size if args.pool_size > 0 else len(runs)
-    pools = [EstimatorPool(params[i:i + size], linger_us=args.linger_us) for i in range(0, len(runs), size)]
+    pools = [EstimatorPool(params[i:i + size], linger_us=args.linger_us, cloud_formats=cloud_formats[i:i + size])
+             for i in range(0, len(runs), size)]
     estimators = [est for pool in pools for est in pool.estimators]
     poses = [[] for _ in runs]
     steps = [[] for _ in runs]
     errors = [None] * len(runs)
 
     def drive(i):
-        sensor, seq = runs[i][0], runs[i][1]
+        src = runs[i][0]
+        register = estimators[i].register_cloud if src[0] == "log" else estimators[i].register_scan
         try:
-            for scan in scans[sensor, seq]:
+            for scan in scans[src]:
                 t0 = time.perf_counter()
-                estimators[i].register_scan(scan)
+                register(scan)
                 steps[i].append(time.perf_counter() - t0)
                 poses[i].append(estimators[i].pose().copy())
         except Exception as e:  # reported after every thread has finished
@@ -172,31 +212,33 @@ def main(argv=None):
             pool.close()
     for i, e in enumerate(errors):
         if e is not None:
-            raise RuntimeError(f"run {runs[i][:3]} failed: {e}") from e
+            raise RuntimeError(f"run {runs[i][0][1:]} {runs[i][1]!r} failed: {e}") from e
 
-    stamps = [k / args.rate_hz for k in range(args.scans)]
     summary = []
-    for sensor in sensors:
-        for seq in sequences:
-            seq_name = f"synthetic/{sensor}/{seq}"
-            d = os.path.join(args.out, seq_name)
-            os.makedirs(d, exist_ok=True)
-            gt = [relative_gt(seq, k) for k in range(args.scans)]
+    for src in sources:
+        n = len(scans[src])
+        stamps = [k / args.rate_hz for k in range(n)]
+        seq_name = f"synthetic/{src[1]}/{src[2]}" if src[0] == "synthetic" else f"log/{src[1]}"
+        d = os.path.join(args.out, seq_name)
+        os.makedirs(d, exist_ok=True)
+        gt = None
+        if src[0] == "synthetic":
+            gt = [relative_gt(src[2], k) for k in range(n)]
             trajectory.write_evalio_csv(os.path.join(d, "gt.csv"), stamps, gt, name="gt", pipeline="gt",
                                         sequence=seq_name)
-            for i, (s_, q_, name, overrides) in enumerate(runs):
-                if (s_, q_) != (sensor, seq):
-                    continue
-                trajectory.write_evalio_csv(os.path.join(d, f"{name}.csv"), stamps, poses[i], name=name,
-                                            params=overrides, total_elapsed=sum(steps[i]),
-                                            max_step_elapsed=max(steps[i]), sequence=seq_name)
+        for i, (s_, name, overrides) in enumerate(runs):
+            if s_ != src:
+                continue
+            trajectory.write_evalio_csv(os.path.join(d, f"{name}.csv"), stamps, poses[i], name=name,
+                                        params=overrides, total_elapsed=sum(steps[i]),
+                                        max_step_elapsed=max(steps[i]), sequence=seq_name)
+            row = dict(variant=name, sequence=seq_name, scans=n, hz=round(n / sum(steps[i]), 3), ate_rmse="")
+            if gt is not None:
                 err = [float(np.linalg.norm(a["t"] - b["t"])) for a, b in zip(poses[i], gt)]
-                row = dict(variant=name, sequence=seq_name, scans=args.scans,
-                           hz=round(args.scans / sum(steps[i]), 3),
-                           ate_rmse=round(float(np.sqrt(np.mean(np.square(err)))), 6))
-                summary.append(row)
-                print(f"{seq_name} [{name}]: {args.scans} scans, hz = {row['hz']:.1f}, "
-                      f"ATE rmse vs ground truth = {row['ate_rmse']:.4f} m")
+                row["ate_rmse"] = round(float(np.sqrt(np.mean(np.square(err)))), 6)
+            summary.append(row)
+            ate = f"ATE rmse vs ground truth = {row['ate_rmse']:.4f} m" if gt is not None else "no ground truth"
+            print(f"{seq_name} [{name}]: {n} scans, hz = {row['hz']:.1f}, {ate}")
     os.makedirs(args.out, exist_ok=True)
     with open(os.path.join(args.out, "summary.csv"), "w", newline="") as f:
         w = csv.DictWriter(f, fieldnames=["variant", "sequence", "scans", "hz", "ate_rmse"])

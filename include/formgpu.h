@@ -174,6 +174,94 @@ int formgpu_extract_debug(formgpu_ctx *ctx, uint8_t *valid_mask, uint8_t *point_
                           int32_t *closest_prev, int32_t *closest_next, size_t *n_planar_picks,
                           uint32_t *point_indices, size_t *n_point_picks);
 
+/* ---- raw sensor clouds: organisation on the device ---------------------- */
+
+/* A driver's point cloud (unordered records, missing returns absent) is turned into the
+ * organised row-major scan the extraction reads, on the device (rule R8, DESIGN.md §4):
+ *   - records that are dropped, counted by reason: a non-finite coordinate, the exact zero point,
+ *     time outside [0, scan_period), row or column out of range;
+ *   - row: the record's ring / row field, or the nearest beam of an elevation table (sign tests
+ *     z cos(mu) - rho sin(mu) against the midpoints mu of adjacent beams);
+ *   - column: the record's col field, floor(t * cols / scan_period) in f64 (clamped to cols - 1),
+ *     or the nearest column centre origin + dir * 2 pi c / cols (half-plane sign tests
+ *     y cos(phi) - x sin(phi) against a boundary table built once, no atan2);
+ *   - collisions: the nearest point wins, key (f32 bits of |p|^2) << 32 | record index, ties to
+ *     the lower index; pixels nobody claimed are (0, 0, 0, 0).
+ * x, y, z in f64 are converted with (float)v. */
+#define FORMGPU_CLOUD_ABSENT (-1)
+#define FORMGPU_FIELD_F32 0
+#define FORMGPU_FIELD_F64 1
+#define FORMGPU_FIELD_U8 2
+#define FORMGPU_FIELD_U16 3
+#define FORMGPU_FIELD_U32 4
+#define FORMGPU_FIELD_U32_NS 5 /* time: u32 nanoseconds since scan start */
+
+#define FORMGPU_ROW_FROM_FIELD 0
+#define FORMGPU_ROW_FROM_ELEVATION 1
+#define FORMGPU_COL_FROM_FIELD 0
+#define FORMGPU_COL_FROM_TIME 1
+#define FORMGPU_COL_FROM_AZIMUTH 2
+
+typedef struct formgpu_cloud_format {
+  uint32_t stride;     /* bytes per record                                         */
+  int32_t off_x, off_y, off_z; /* byte offsets inside a record                      */
+  int32_t xyz_type;    /* FORMGPU_FIELD_F32 or _F64                                 */
+  int32_t off_row;     /* ring / row field, FORMGPU_CLOUD_ABSENT if none            */
+  int32_t row_type;    /* _U8, _U16 or _U32                                         */
+  int32_t off_col;     /* column field, or FORMGPU_CLOUD_ABSENT                     */
+  int32_t col_type;    /* _U16 or _U32                                              */
+  int32_t off_time;    /* time since scan start, or FORMGPU_CLOUD_ABSENT            */
+  int32_t time_type;   /* _F32 / _F64 seconds or _U32_NS                            */
+  int32_t row_source;  /* FORMGPU_ROW_FROM_*                                        */
+  int32_t col_source;  /* FORMGPU_COL_FROM_*                                        */
+  int32_t azimuth_dir; /* +1: columns advance counter-clockwise, -1: clockwise      */
+  double scan_period;  /* seconds, > 0                                              */
+  double azimuth_origin; /* radians: centre of column 0                            */
+  const double *beam_elevations; /* [num_rows] radians, strictly monotonic, |e| < pi/2
+                                    (ROW_FROM_ELEVATION; copied by set_cloud_format) */
+  uint64_t max_records; /* capacity: records of the largest cloud, < 2^32            */
+} formgpu_cloud_format;
+
+/* Outcome of the last organisation of a context: every record lands in exactly one of
+ * placed / dropped_*; pixels = pixels that received a point (placed - pixels lost a collision). */
+typedef struct formgpu_cloud_stats {
+  uint64_t records;
+  uint64_t placed;
+  uint64_t pixels;
+  uint64_t dropped_nonfinite;
+  uint64_t dropped_zero;
+  uint64_t dropped_time;
+  uint64_t dropped_row;
+  uint64_t dropped_col;
+} formgpu_cloud_stats;
+
+/* The checks of formgpu_set_cloud_format for a rows x cols scan, without a context or GPU.
+ * Returns FORMGPU_OK or the error code, with a message in msg (may be NULL). */
+int formgpu_cloud_format_check(const formgpu_cloud_format *fmt, int rows, int cols, char *msg, size_t msg_cap);
+
+/* Give the context a cloud format (checked before any CUDA call).  Allocates, once, the record
+ * staging buffer (max_records * stride bytes), the per-pixel keys and the boundary tables, so
+ * nothing is allocated per scan.  Also valid on formgpu_batch_ctx(b, i).  A later call replaces
+ * the format. */
+int formgpu_set_cloud_format(formgpu_ctx *ctx, const formgpu_cloud_format *fmt);
+
+/* Organise n records (HOST memory) into the context's scan buffer and, when out is not NULL,
+ * copy the rows*cols scan to it; stats may be NULL.  FORMGPU_ERR_STATE without a format,
+ * FORMGPU_ERR_CAPACITY when n > max_records.  The context's current scan (its keypoints and
+ * matches) is unchanged; formgpu_extract_debug needs a new formgpu_extract afterwards. */
+int formgpu_organize(formgpu_ctx *ctx, const void *records, size_t n, formgpu_point4f *out,
+                     formgpu_cloud_stats *stats);
+
+/* formgpu_extract with a raw cloud as input: organise, then extract the organised scan.  Same
+ * outputs and "current scan" semantics. */
+int formgpu_extract_cloud(formgpu_ctx *ctx, const void *records, size_t n, uint64_t scan_idx,
+                          formgpu_planar_feat *planar_out, size_t planar_cap, size_t *n_planar,
+                          formgpu_point_feat *point_out, size_t point_cap, size_t *n_point);
+
+/* Counters of the context's last organisation (formgpu_organize, formgpu_extract_cloud or a
+ * FORMGPU_REQ_CLOUD request of a batch). */
+int formgpu_cloud_stats_last(const formgpu_ctx *ctx, formgpu_cloud_stats *stats);
+
 /* ---- stage 2: reparative map + association ------------------------------ */
 
 /* KeypointMap::to_voxel_map for both keypoint types (form/mapping/map.hpp:137,
@@ -320,6 +408,10 @@ int formgpu_comm_destroy(formgpu_ctx *ctx);
 #define FORMGPU_OP_COUNT 8
 
 #define FORMGPU_REQ_SCAN_ON_DEVICE 1u /* `scan` is a device pointer; no keypoints copied back */
+/* FORMGPU_OP_EXTRACT on a raw cloud (formgpu_extract_cloud): `scan` points at n_points records of
+ * the sequence's cloud format.  The clouds of a submission are organised by one launch per kernel
+ * ahead of the extraction.  With FORMGPU_REQ_SCAN_ON_DEVICE the records are in device memory. */
+#define FORMGPU_REQ_CLOUD 2u
 
 typedef struct formgpu_request {
   uint32_t sequence; /* index of the sequence inside the batch */
@@ -395,6 +487,9 @@ int formgpu_batch_done(formgpu_batch *b);
  * a different pointer in the request simply discards the prefetched copy.  Call it between
  * formgpu_batch_wait and the next submission of the batch. */
 int formgpu_batch_prefetch_scan(formgpu_batch *b, size_t sequence, const formgpu_point4f *scan, size_t n_points);
+/* The same for a raw cloud: the n records go ahead into the sequence's record staging buffer, and
+ * the FORMGPU_REQ_CLOUD request that names the same pointer and count does not upload them again. */
+int formgpu_batch_prefetch_cloud(formgpu_batch *b, size_t sequence, const void *records, size_t n);
 const char *formgpu_batch_last_error(const formgpu_batch *b);
 /* As formgpu_profile_enable / _read / formgpu_launch_count, for the batched launches. */
 int formgpu_batch_profile_enable(formgpu_batch *b, int on);
