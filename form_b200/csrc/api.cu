@@ -251,7 +251,7 @@ static int create_impl(formgpu_ctx *ctx) {
   FORMGPU_CUDA(ctx, dev_alloc(&ctx->d_mapmem,
                               256 + (ctx->hash_cap[0] + ctx->hash_cap[1]) * sizeof(HashSlot)));
   ctx->map_req_bytes = W * 12 * sizeof(double) + W * sizeof(uint64_t) +
-                       (2 * (W + 1) + W) * sizeof(int);
+                       (2 * (W + 1) + 2 * W) * sizeof(int);
   ctx->map_req_bytes = (ctx->map_req_bytes + 7) / 8 * 8; // moved in 8-byte words by batched rebuilds
   FORMGPU_CUDA(ctx, dev_alloc(&ctx->d_map_req, ctx->map_req_bytes));
   FORMGPU_CUDA(ctx, cudaHostAlloc(reinterpret_cast<void **>(&ctx->h_map_req), ctx->map_req_bytes,

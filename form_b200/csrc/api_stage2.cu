@@ -22,6 +22,16 @@ void clear_pairs_of_slot(formgpu_ctx *ctx, int slot) {
   }
 }
 
+/// The window's used slots in ascending scan id (rule R4): the order of map points, pair counts and
+/// exported keypoints.
+std::vector<int> slots_by_scan(const formgpu_ctx *ctx) {
+  std::vector<int> order;
+  for (int s = 0; s < ctx->W; ++s)
+    if (ctx->slot_used[s]) order.push_back(s);
+  std::sort(order.begin(), order.end(), [&](int a, int b) { return ctx->slot_scan[a] < ctx->slot_scan[b]; });
+  return order;
+}
+
 /// scan id -> window slot, allocating one on first touch (KeypointMap::get,
 /// map.tpp:98-110; ConstraintManager::get_constraints, constraints.cpp:39-64).
 int ensure_slot(formgpu_ctx *ctx, uint64_t scan) {
@@ -46,6 +56,7 @@ struct MapReq {
   uint64_t *scan;
   int *off;   // [2][W+1]
   int *order; // [W]
+  int *rank;  // [W] position of each slot in ascending scan-id order (rule R4, map rebuilds)
 };
 MapReq map_req_view(unsigned char *base, int W) {
   MapReq r;
@@ -53,6 +64,7 @@ MapReq map_req_view(unsigned char *base, int W) {
   r.scan = reinterpret_cast<uint64_t *>(base + (size_t)W * 12 * sizeof(double));
   r.off = reinterpret_cast<int *>(base + (size_t)W * 12 * sizeof(double) + (size_t)W * sizeof(uint64_t));
   r.order = r.off + 2 * (W + 1);
+  r.rank = r.order + W;
   return r;
 }
 
@@ -109,6 +121,13 @@ int map_rebuild_prepare(formgpu_ctx *ctx, const formgpu_scan_pose *poses, size_t
     ctx->map_n[t] = (size_t)run;
   }
   for (int s = 0; s < W; ++s) h.scan[s] = ctx->slot_scan[s];
+  // the tie-break id of a map point is (rank of its scan, k): the scan id itself would need all 64
+  // bits, and ranks (< W) order the scans exactly as their ids do
+  {
+    const std::vector<int> order = slots_by_scan(ctx);
+    for (int s = 0; s < W; ++s) h.rank[s] = 0;
+    for (size_t o = 0; o < order.size(); ++o) h.rank[order[o]] = (int)o;
+  }
   if (upload) {
     FORMGPU_CUDA(ctx, cudaMemcpyAsync(ctx->d_map_req, ctx->h_map_req, ctx->map_req_bytes,
                                       cudaMemcpyHostToDevice, stream));
@@ -137,7 +156,7 @@ int map_rebuild_prepare(formgpu_ctx *ctx, const formgpu_scan_pose *poses, size_t
     a[t].store = t == 0 ? (const void *)ctx->d_store_planar : (const void *)ctx->d_store_point;
     a[t].slot_off = d.off + t * (W + 1);
     a[t].slot_pose = d.pose;
-    a[t].slot_scan = d.scan;
+    a[t].slot_rank = d.rank;
     a[t].n_total = (int)ctx->map_n[t];
     a[t].voxel_width = ctx->P.max_dist_matching; // form.cpp:61-65
     a[t].inv_voxel_width = 1.0 / ctx->P.max_dist_matching;
@@ -187,10 +206,8 @@ int assoc_prepare(formgpu_ctx *ctx, const formgpu_pose *pose_k, const formgpu_sc
     }
     if (pk < 0) return fail(ctx, FORMGPU_ERR_INVALID_ARG, "associate_linearize: no pose for the current scan");
     std::vector<int> order;
-    for (int i = 0; i < W; ++i)
-      if (ctx->slot_used[i] && i != slot_k && pose_idx[i] >= 0) order.push_back(i);
-    std::sort(order.begin(), order.end(),
-              [&](int a, int b) { return ctx->slot_scan[a] < ctx->slot_scan[b]; });
+    for (const int i : slots_by_scan(ctx))
+      if (i != slot_k && pose_idx[i] >= 0) order.push_back(i);
     const int rc = ensure_out(ctx, order.size() + 1);
     if (rc) return rc;
     for (size_t n = 0; n < order.size(); ++n) {
@@ -593,11 +610,7 @@ int formgpu_world_keypoints(formgpu_ctx *ctx, const formgpu_scan_pose *poses, si
     has_pose[s] = 1;
   }
   // slots in ascending scan id (rule R4)
-  std::vector<int> order;
-  for (int s = 0; s < W; ++s)
-    if (ctx->slot_used[s]) order.push_back(s);
-  std::sort(order.begin(), order.end(),
-            [&](int a, int b) { return ctx->slot_scan[a] < ctx->slot_scan[b]; });
+  const std::vector<int> order = slots_by_scan(ctx);
   size_t total[2];
   for (int t = 0; t < 2; ++t) {
     int run = 0;

@@ -112,7 +112,7 @@ struct MapArgs {
   const void *store;   // PlanarRec* or PointRec*
   const int *slot_off; // [W+1] exclusive prefix of store counts (device)
   const double *slot_pose;   // [W][12]
-  const uint64_t *slot_scan; // [W]
+  const int *slot_rank;      // [W] rank of the slot's scan id among the window's (tie-break, rule R4)
   int n_total;
   double voxel_width;
   double inv_voxel_width; // 1 / voxel_width (host, IEEE): fast path of voxel_coord

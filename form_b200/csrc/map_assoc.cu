@@ -181,7 +181,7 @@ __device__ __forceinline__ void map_insert_body(const MapArgs &a) {
   a.world_slot[g] = h;
   WorldPoint wp;
   wp.x = wx; wp.y = wy; wp.z = wz;
-  wp.tie = (a.slot_scan[slot] << 24) | (unsigned long long)k; // rule R4 id
+  wp.tie = ((unsigned long long)a.slot_rank[slot] << 24) | (unsigned long long)k; // rule R4 id
   a.world_tmp[g] = wp;
 }
 } // namespace
