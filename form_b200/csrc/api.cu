@@ -182,8 +182,8 @@ static int create_impl(formgpu_ctx *ctx) {
   }
   ctx->prof.stream = ctx->stream;
   FORMGPU_CUDA(ctx, cudaHostAlloc(reinterpret_cast<void **>(const_cast<unsigned long long **>(&ctx->h_flags)),
-                                  24 * sizeof(unsigned long long), cudaHostAllocMapped));
-  for (int i = 0; i < 24; ++i) ctx->h_flags[i] = 0;
+                                  8 * sizeof(unsigned long long), cudaHostAllocMapped));
+  for (int i = 0; i < 8; ++i) ctx->h_flags[i] = 0;
 
   const size_t B = ctx->B, R = ctx->rows, W = ctx->W;
   // stage 1
@@ -225,8 +225,6 @@ static int create_impl(formgpu_ctx *ctx) {
       return fail(ctx, FORMGPU_ERR_INVALID_ARG, "num_sectors exceeds " + std::to_string(kExtractMaxSectors));
     FORMGPU_CUDA(ctx, extract_configure(shape));
   }
-  FORMGPU_CUDA(ctx, linearize_configure());
-  if (const char *env = std::getenv("FORMGPU_CELL_BUCKETS")) ctx->cell_buckets = env[0] != '0';
   if (const char *env = std::getenv("FORMGPU_SINGLE_CELL_SEARCH")) ctx->cell_search_single = env[0] == '1';
 
   // window / keypoint store
@@ -243,9 +241,9 @@ static int create_impl(formgpu_ctx *ctx) {
     ctx->map_cap[t] = cap[t];
     ctx->hash_cap[t] = next_pow2(2 * cap[t]);
     FORMGPU_CUDA(ctx, dev_alloc(&ctx->d_world[t], cap[t]));
-    FORMGPU_CUDA(ctx, dev_alloc(&ctx->d_world_tmp[t], cap[t]));
-    FORMGPU_CUDA(ctx, dev_alloc(&ctx->d_world_slot[t], cap[t]));
     FORMGPU_CUDA(ctx, dev_alloc(&ctx->d_world_src[t], cap[t]));
+    FORMGPU_CUDA(ctx, dev_alloc(&ctx->d_cell_tab[t], cap[t]));
+    FORMGPU_CUDA(ctx, dev_alloc(&ctx->d_scatter_src[t], cap[t]));
     FORMGPU_CUDA(ctx, dev_alloc(&ctx->d_voxel_list[t], cap[t]));
   }
   FORMGPU_CUDA(ctx, dev_alloc(&ctx->d_mapmem,
@@ -339,13 +337,13 @@ void formgpu_destroy(formgpu_ctx *ctx) {
   F(ctx->d_dbg_valid); F(ctx->d_dbg_pvalid); F(ctx->d_dbg_curv);
   F(ctx->d_store_planar); F(ctx->d_store_point);
   for (int t = 0; t < 2; ++t) {
-    F(ctx->d_world[t]); F(ctx->d_world_tmp[t]);
-    F(ctx->d_world_slot[t]); F(ctx->d_world_src[t]); F(ctx->d_voxel_list[t]); F(ctx->d_match[t]);
+    F(ctx->d_world[t]); F(ctx->d_world_src[t]);
+    F(ctx->d_cell_tab[t]); F(ctx->d_scatter_src[t]); F(ctx->d_voxel_list[t]); F(ctx->d_match[t]);
   }
   F(ctx->d_mapmem); F(ctx->d_map_req); F(ctx->d_export); H(ctx->h_map_req);
   if (ctx->ev_upload) cudaEventDestroy(ctx->ev_upload);
   F(ctx->d_seg_planar); F(ctx->d_seg_point); F(ctx->d_pair);
-  F(ctx->d_partials); F(ctx->d_request); F(ctx->d_counters);
+  F(ctx->d_request); F(ctx->d_counters);
   F(ctx->d_moments); F(ctx->d_mom_partials); F(ctx->d_mom_tickets);
   comm_release(ctx);
   F(ctx->d_stage_planar); F(ctx->d_stage_point);
@@ -660,22 +658,6 @@ int formgpu_profile_read(formgpu_ctx *ctx, double ms[FORMGPU_KG_COUNT],
     ctx->prof.group[g] = GroupProf();
   }
   return FORMGPU_OK;
-}
-
-/* not part of the public header: timing experiments (profiles/microbench_calls.py) */
-const unsigned long long *formgpu_debug_timestamps(const formgpu_ctx *ctx) {
-  return ctx ? const_cast<const unsigned long long *>(ctx->h_flags) + 8 : nullptr;
-}
-
-uint64_t formgpu_debug_host_times(formgpu_ctx *ctx, double out[8]) {
-  if (!ctx) return 0;
-  for (int i = 0; i < 8; ++i) {
-    out[i] = ctx->dbg_host_us[i];
-    ctx->dbg_host_us[i] = 0;
-  }
-  const uint64_t n = ctx->dbg_host_calls;
-  ctx->dbg_host_calls = 0;
-  return n;
 }
 
 uint64_t formgpu_launch_count(const formgpu_ctx *ctx) { return ctx ? ctx->prof.total_launches : 0; }

@@ -41,26 +41,15 @@ struct formgpu_batch {
   std::vector<std::vector<int>> lin_indices;
   std::vector<unsigned long long> lin_seqs;
   std::vector<LinTask> tasks_scratch;
-  // sliced linearisation scratch: partial sums (56 doubles per CTA) and per-task tickets
-  double *d_partials = nullptr;
-  unsigned *d_tickets = nullptr;
-  size_t partial_cap = 0, ticket_cap = 0;
-  size_t partials_used = 0, tickets_used = 0; // within the current submit
   // extraction launches with at least this many rows use the many-row kernel variants
   // (kernels.hpp: kManyRowsMin; FORMGPU_MANY_ROWS_MIN overrides it, for tests and tuning)
   int many_rows_min = kManyRowsMin;
-  int assoc_lanes = kAssocLanes; // lanes per query of the batched association kernel (FORMGPU_ASSOC_LANES)
-  // stage 3 from the pair-moment cache (moments.cu); FORMGPU_STREAM_LINEARIZE=1 streams instead
-  bool moment_cache = true;
-  // host-scan extraction: keypoint structs go back by DMA from a device staging buffer (default)
-  // or, with FORMGPU_PACK_DMA=0, by the pack kernel's own stores into mapped host memory
-  bool pack_dma = true;
   // 13x13 blocks of a submission: the evaluation kernels write plain doubles into d_blocks and ONE
   // copy-engine transfer per submission takes them to h_blocks (page-locked).  SM stores of
-  // sequence-tagged words into mapped host memory (the single-sequence protocol, FORMGPU_BLOCK_DMA=0)
-  // move twice the bytes in 8-byte PCIe writes and kept the evaluation CTAs resident until the
-  // writes drained: 52 us per launch of ~1000 pairs, i.e. ~28 GB/s of PCIe stores.
-  bool block_dma = true;
+  // sequence-tagged words into mapped host memory (the single-sequence protocol) move twice the
+  // bytes in 8-byte PCIe writes and kept the evaluation CTAs resident until the writes drained:
+  // 52 us per launch of ~1000 pairs, i.e. ~28 GB/s of PCIe stores.  Errors still come back as
+  // tagged words.
   double *d_blocks = nullptr, *h_blocks = nullptr;
   size_t blocks_cap = 0, blocks_used = 0; // doubles
   std::vector<size_t> assoc_block_off, lin_block_off; // per sequence: offset into h_blocks, or kNoBlocks
@@ -223,94 +212,21 @@ template <typename T> const T *staged(const formgpu_batch *b, size_t offset) {
   return reinterpret_cast<const T *>(b->d_args + offset);
 }
 
-// Scratch of the batched linearisation launches: 56 doubles per slice, one ticket per task.
-int ensure_lin_scratch(formgpu_batch *b, size_t n_ctas, size_t n_tasks) {
-  if (n_ctas > b->partial_cap) {
-    BATCH_CUDA(b, cudaStreamSynchronize(b->stream));
-    if (b->d_partials) cudaFree(b->d_partials);
-    b->d_partials = nullptr;
-    size_t cap = std::max<size_t>(b->partial_cap * 2, 4096);
-    while (cap < n_ctas) cap *= 2;
-    BATCH_CUDA(b, cudaMalloc(reinterpret_cast<void **>(&b->d_partials), cap * 56 * sizeof(double)));
-    b->partial_cap = cap;
-  }
-  if (n_tasks > b->ticket_cap) {
-    BATCH_CUDA(b, cudaStreamSynchronize(b->stream));
-    if (b->d_tickets) cudaFree(b->d_tickets);
-    b->d_tickets = nullptr;
-    size_t cap = std::max<size_t>(b->ticket_cap * 2, 4096);
-    while (cap < n_tasks) cap *= 2;
-    BATCH_CUDA(b, cudaMalloc(reinterpret_cast<void **>(&b->d_tickets), cap * sizeof(unsigned)));
-    BATCH_CUDA(b, cudaMemsetAsync(b->d_tickets, 0, cap * sizeof(unsigned), b->stream));
-    b->ticket_cap = cap;
-  }
-  return FORMGPU_OK;
-}
-
-// Linearisation tasks of several contexts in ONE launch: every pair is cut into
-// ceil(size / kLinWarpSlice) warp-sized slices.  `size` is the host's estimate; the kernel
-// divides the TRUE range by the slice count, so a wrong estimate costs balance, not
-// correctness.  Slices of large pairs come first (they are the long pole).
+// Blocks / errors of the listed tasks of several contexts in ONE launch, evaluated from the
+// contexts' pair-moment caches (moments.cu): one CTA per task, ctx_args[task.ctx_index] is the
+// task's context.
 int stage_lin_groups(formgpu_batch *b, const std::vector<LinArgs> &ctx_args, const std::vector<LinTask> &tasks,
-                     const std::vector<uint32_t> &size_hint, bool error_only,
-                     std::vector<std::function<int()>> &launchers) {
+                     bool error_only, std::vector<std::function<int()>> &launchers) {
   if (tasks.empty()) return FORMGPU_OK;
-  if (b->moment_cache) {
-    // evaluation from the pair-moment cache: one warp per task, nothing is streamed
-    size_t off_ctx = 0, off_tasks = 0;
-    int rc = stage_args(b, ctx_args.data(), ctx_args.size(), &off_ctx);
-    if (rc) return rc;
-    rc = stage_args(b, tasks.data(), tasks.size(), &off_tasks);
-    if (rc) return rc;
-    const int n_tasks = (int)tasks.size();
-    launchers.push_back([=]() -> int {
-      BATCH_CUDA(b, eval_batch_launch(staged<LinArgs>(b, off_ctx), staged<LinTask>(b, off_tasks), n_tasks,
-                                      error_only, b->stream, b->prof));
-      return FORMGPU_OK;
-    });
-    return FORMGPU_OK;
-  }
-  std::vector<size_t> order(tasks.size());
-  for (size_t t = 0; t < order.size(); ++t) order[t] = t;
-  std::stable_sort(order.begin(), order.end(), [&](size_t x, size_t y) { return size_hint[x] > size_hint[y]; });
-  // Slice length: the per-slice cost (two butterfly reductions, partial sums, ticket) is
-  // worth ~250 correspondences, so slices grow with the launch - about kLinWarpTarget warps
-  // (two waves of resident warps) - between kLinWarpSlice and kLinWarpSliceMax.
-  unsigned long long total = 0;
-  for (uint32_t h : size_hint) total += h;
-  const uint32_t slice_len = (uint32_t)std::min<unsigned long long>(
-      std::max<unsigned long long>((total / kLinWarpTarget + 127) / 128 * 128, kLinWarpSlice), kLinWarpSliceMax);
-  std::vector<LinCta> slices;
-  slices.reserve(tasks.size() * 4);
-  for (size_t t : order) {
-    const LinArgs &ca = ctx_args[tasks[t].ctx_index];
-    const uint32_t n =
-        std::min<uint32_t>(std::max<uint32_t>((size_hint[t] + slice_len - 1) / slice_len, 1u), 4096u);
-    const uint32_t first = (uint32_t)slices.size();
-    for (uint32_t r = 0; r < n; ++r)
-      slices.push_back(LinCta{(uint32_t)t, first, (uint16_t)r, (uint16_t)n, tasks[t].ctx_index, ca.pair_row,
-                              tasks[t].dyn_slot_i_plus1, (uint32_t)ca.W + 1u});
-  }
-  // every launch of a submit gets its own scratch range: launches of one submit run back
-  // to back and could otherwise overlap on the partial sums (tickets are indexed by task)
-  const size_t part_base = b->partials_used, ticket_base = b->tickets_used;
-  b->partials_used += slices.size();
-  b->tickets_used += tasks.size();
-  int rc = ensure_lin_scratch(b, b->partials_used, b->tickets_used);
-  if (rc) return rc;
-  size_t off_ctx = 0, off_tasks = 0, off_slices = 0;
-  rc = stage_args(b, ctx_args.data(), ctx_args.size(), &off_ctx);
+  size_t off_ctx = 0, off_tasks = 0;
+  int rc = stage_args(b, ctx_args.data(), ctx_args.size(), &off_ctx);
   if (rc) return rc;
   rc = stage_args(b, tasks.data(), tasks.size(), &off_tasks);
   if (rc) return rc;
-  rc = stage_args(b, slices.data(), slices.size(), &off_slices);
-  if (rc) return rc;
-  const int n_slices = (int)slices.size();
+  const int n_tasks = (int)tasks.size();
   launchers.push_back([=]() -> int {
-    BATCH_CUDA(b, linearize_warp_launch(staged<LinArgs>(b, off_ctx), staged<LinTask>(b, off_tasks),
-                                        staged<LinCta>(b, off_slices), n_slices,
-                                        b->d_partials + part_base * 56, b->d_tickets + ticket_base,
-                                        error_only, b->stream, b->prof));
+    BATCH_CUDA(b, eval_batch_launch(staged<LinArgs>(b, off_ctx), staged<LinTask>(b, off_tasks), n_tasks, error_only,
+                                    b->stream, b->prof));
     return FORMGPU_OK;
   });
   return FORMGPU_OK;
@@ -355,9 +271,6 @@ int formgpu_batch_create_mixed(const formgpu_params *params, int device, void *s
   b->device = device;
   b->stream = static_cast<cudaStream_t>(stream);
   if (const char *env = std::getenv("FORMGPU_MANY_ROWS_MIN")) b->many_rows_min = std::atoi(env);
-  if (const char *env = std::getenv("FORMGPU_ASSOC_LANES")) b->assoc_lanes = std::atoi(env);
-  if (const char *env = std::getenv("FORMGPU_PACK_DMA")) b->pack_dma = env[0] != '0';
-  if (const char *env = std::getenv("FORMGPU_BLOCK_DMA")) b->block_dma = env[0] != '0';
   if (const char *env = std::getenv("FORMGPU_BATCH_TRACE")) b->trace.on = env[0] == '1';
   auto bail = [&](int rc, const std::string &msg) {
     g_batch_error = msg;
@@ -389,12 +302,9 @@ int formgpu_batch_create_mixed(const formgpu_params *params, int device, void *s
     if (rc != FORMGPU_OK)
       return bail(rc, "formgpu_create (sequence " + std::to_string(i) + "): " + formgpu_last_error(nullptr));
     c->moment_unit = kMomentUnit; // throughput-sized units (kernels.hpp)
+    c->moment_cache = true;       // the batched stage 3 evaluates from the cache only
     b->ctx.push_back(c);
   }
-  // switches read from the environment when a context is created are the same for every context
-  // of the batch; the batch takes them from its first
-  b->moment_cache = b->ctx[0]->moment_cache;
-  b->block_dma = b->block_dma && b->moment_cache; // the evaluation kernels write plain blocks
   b->assoc_block_off.assign(n_sequences, kNoBlocks);
   b->lin_block_off.assign(n_sequences, kNoBlocks);
   b->assoc_plans.resize(n_sequences);
@@ -423,8 +333,6 @@ void formgpu_batch_destroy(formgpu_batch *b) {
   for (formgpu_ctx *c : b->ctx) formgpu_destroy(c);
   if (b->h_args) cudaFreeHost(b->h_args);
   if (b->d_args) cudaFree(b->d_args);
-  if (b->d_partials) cudaFree(b->d_partials);
-  if (b->d_tickets) cudaFree(b->d_tickets);
   if (b->h_done) cudaFreeHost(const_cast<uint32_t *>(b->h_done));
   if (b->d_blocks) cudaFree(b->d_blocks);
   if (b->h_blocks) cudaFreeHost(b->h_blocks);
@@ -507,7 +415,7 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
     if (rc) return rc;
   }
   b->blocks_used = 0;
-  if (b->block_dma) {
+  {
     // upper bound of the block words this submission can produce (sized before anything is staged:
     // the argument blocks carry pointers into d_blocks)
     size_t doubles = 0;
@@ -517,8 +425,6 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
     if (rc) return rc;
   }
   b->args_used = 0;
-  b->partials_used = 0;
-  b->tickets_used = 0;
   auto set_status = [&](formgpu_request &q, int rc) {
     q.status = rc;
     if (rc != FORMGPU_OK && first_error == FORMGPU_OK) {
@@ -603,7 +509,7 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
         }
         ctx->prefetched_host = nullptr;
         scan_dev = ctx->d_scan;
-        if (b->pack_dma && q.planar_out && q.point_out) {
+        if (q.planar_out && q.point_out) {
           // f64 structs into device staging; a copy engine takes them to the caller (collect phase)
           if (!ctx->d_stage_planar) {
             BATCH_CUDA(b, cudaMalloc(reinterpret_cast<void **>(&ctx->d_stage_planar), ctx->kp_cap * sizeof(formgpu_planar_feat)));
@@ -702,10 +608,9 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
       rc = stage_args(b, regions.data(), regions.size(), &off_regions);
       if (rc) return rc;
       const int n_items = (int)regions.size();
-      const bool cells = items[0].cells != 0; // one switch per process (FORMGPU_CELL_BUCKETS)
       launchers.push_back([=]() -> int {
         map_build_batch_launch(staged<MapArgs>(b, off_items), staged<MapClearRegion>(b, off_regions), b->d_args, n_items,
-                               max_points, max_hash, max_clear, cells, b->stream, b->prof);
+                               max_points, max_hash, max_clear, b->stream, b->prof);
         BATCH_CUDA(b, cudaGetLastError());
         return FORMGPU_OK;
       });
@@ -720,7 +625,6 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
     int max_units = 0;
     std::vector<LinArgs> lin_ctx;
     std::vector<LinTask> &lin_tasks = b->tasks_scratch;
-    std::vector<uint32_t> hints;
     lin_tasks.clear();
     int max_query = 0;
     for (int pass = 0; pass < 2; ++pass) {
@@ -760,30 +664,14 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
           LinArgs la;
           lin_make_args(ctx, (int)plan.lin_tasks.size(), la);
           plan.lin_seq = la.seq;
-          if (b->block_dma) {
-            la.out_plain = b->d_blocks + b->blocks_used;
-            b->assoc_block_off[q.sequence] = b->blocks_used;
-            b->blocks_used += 91 * plan.lin_tasks.size();
-          }
+          la.out_plain = b->d_blocks + b->blocks_used;
+          b->assoc_block_off[q.sequence] = b->blocks_used;
+          b->blocks_used += 91 * plan.lin_tasks.size();
           const uint32_t ci = (uint32_t)lin_ctx.size();
           lin_ctx.push_back(la);
-          for (size_t k = 0; k < plan.lin_tasks.size(); ++k) {
-            LinTask t = plan.lin_tasks[k];
+          for (LinTask t : plan.lin_tasks) {
             t.ctx_index = ci;
             lin_tasks.push_back(t);
-            // size estimate: the pair's count after the previous association of this scan
-            // size estimate: the pair's count after the previous association of this scan, else
-            // the count of the same map scan's pair with the previous scan
-            const PairEntry &e = ctx->h_pair_table[(size_t)plan.slot_k * ctx->W + plan.lin_slots[k]];
-            uint32_t prev = e.n_planar + e.n_point;
-            if (!prev && ctx->cur_scan > 0) {
-              const int sp = find_slot(ctx, ctx->cur_scan - 1);
-              if (sp >= 0) {
-                const PairEntry &e2 = ctx->h_pair_table[(size_t)sp * ctx->W + plan.lin_slots[k]];
-                prev = e2.n_planar + e2.n_point;
-              }
-            }
-            hints.push_back(prev ? prev : (uint32_t)(plan.nq[0] + plan.nq[1]) / 4u);
           }
         } else if (plan.fused) {
           LinArgs la;
@@ -801,17 +689,14 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
       rc = stage_args(b, mitems.data(), mitems.size(), &off_m);
       if (rc) return rc;
       const int n_items = (int)aitems.size() / 2;
-      const bool moments = b->moment_cache;
-      const bool cells = aitems[0].cell_tab != nullptr; // one switch per process (FORMGPU_CELL_BUCKETS)
       launchers.push_back([=]() -> int {
-        assoc_batch_launch(staged<AssocArgs>(b, off_a), n_items, max_query, cells ? 1 : b->assoc_lanes, b->stream,
-                           b->prof);
+        assoc_batch_launch(staged<AssocArgs>(b, off_a), n_items, max_query, b->stream, b->prof);
         segment_build_batch_launch(staged<SegmentArgs>(b, off_s), n_items, max_query, b->stream, b->prof);
-        if (moments) moments_batch_launch(staged<MomentArgs>(b, off_m), n_items, max_units, b->stream, b->prof);
+        moments_batch_launch(staged<MomentArgs>(b, off_m), n_items, max_units, b->stream, b->prof);
         BATCH_CUDA(b, cudaGetLastError());
         return FORMGPU_OK;
       });
-      rc = stage_lin_groups(b, lin_ctx, lin_tasks, hints, false, launchers);
+      rc = stage_lin_groups(b, lin_ctx, lin_tasks, false, launchers);
       if (rc) return rc;
     }
   }
@@ -822,7 +707,6 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
     const size_t per_pair = eo ? 1 : 91;
     std::vector<LinArgs> lin_ctx;
     std::vector<LinTask> &lin_tasks = b->tasks_scratch;
-    std::vector<uint32_t> hints;
     std::vector<LinTask> tasks;
     lin_tasks.clear();
     for (size_t r : by_op[op]) {
@@ -850,7 +734,7 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
       live_lin[eo].push_back(r);
       if (!eo) b->lin_block_off[q.sequence] = kNoBlocks;
       if (tasks.empty()) continue;
-      if (!eo && b->block_dma) {
+      if (!eo) {
         la.out_plain = b->d_blocks + b->blocks_used; // task.out_index = position in q.pairs
         b->lin_block_off[q.sequence] = b->blocks_used;
         b->blocks_used += 91 * q.n_pairs;
@@ -860,10 +744,9 @@ int submit_build(formgpu_batch *b, formgpu_request *reqs, size_t n) {
       for (LinTask &t : tasks) {
         t.ctx_index = ci;
         lin_tasks.push_back(t);
-        hints.push_back(t.n_planar + t.n_point);
       }
     }
-    const int rc = stage_lin_groups(b, lin_ctx, lin_tasks, hints, eo != 0, launchers);
+    const int rc = stage_lin_groups(b, lin_ctx, lin_tasks, eo != 0, launchers);
     if (rc) return rc;
   }
   // ---- commit ----

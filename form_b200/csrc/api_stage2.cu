@@ -160,14 +160,12 @@ int map_rebuild_prepare(formgpu_ctx *ctx, const formgpu_scan_pose *poses, size_t
     a[t].n_total = (int)ctx->map_n[t];
     a[t].voxel_width = ctx->P.max_dist_matching; // form.cpp:61-65
     a[t].inv_voxel_width = 1.0 / ctx->P.max_dist_matching;
-    a[t].cells = ctx->cell_buckets ? 1 : 0;
-    a[t].pad_cells = 0;
     a[t].hash = ctx->d_hash[t];
     a[t].hash_mask = ctx->hash_mask[t];
-    a[t].world_tmp = ctx->d_world_tmp[t];
-    a[t].world_slot = ctx->d_world_slot[t];
-    a[t].world_src = ctx->d_world_src[t];
     a[t].world = ctx->d_world[t];
+    a[t].world_src = ctx->d_world_src[t];
+    a[t].cell_tab = ctx->d_cell_tab[t];
+    a[t].scatter_src = ctx->d_scatter_src[t];
     a[t].cursor = reinterpret_cast<uint32_t *>(ctx->d_mapmem) + 16 * t;
     a[t].voxel_list = ctx->d_voxel_list[t];
   }
@@ -249,11 +247,9 @@ int assoc_prepare(formgpu_ctx *ctx, const formgpu_pose *pose_k, const formgpu_sc
     aa[t].inv_voxel_width = 1.0 / ctx->P.max_dist_matching;
     aa[t].hash = ctx->d_hash[t];
     aa[t].hash_mask = ctx->hash_mask[t];
-    // with cell-ordered buckets pass 4 of the rebuild leaves the final points / ids in the
-    // scatter pass's scratch arrays and the per-voxel cell tables in d_world
-    aa[t].cell_tab = ctx->cell_buckets ? ctx->d_world[t] : nullptr;
-    aa[t].world = ctx->cell_buckets ? ctx->d_world_tmp[t] : ctx->d_world[t];
-    aa[t].world_src = ctx->cell_buckets ? ctx->d_world_slot[t] : ctx->d_world_src[t];
+    aa[t].cell_tab = ctx->d_cell_tab[t];
+    aa[t].world = ctx->d_world[t];
+    aa[t].world_src = ctx->d_world_src[t];
     aa[t].match = ctx->d_match[t];
     aa[t].W = W;
     aa[t].max_dist2 = ctx->P.max_dist_matching * ctx->P.max_dist_matching; // matcher.hpp:82

@@ -1,10 +1,6 @@
 // C-ABI (include/formgpu.h): stage 3 - linearisation and error evaluation.
 #include "api_common.hpp"
 
-#include <algorithm>
-#include <chrono>
-#include <cstdlib>
-
 using namespace formgpu;
 
 namespace formgpu {
@@ -30,10 +26,6 @@ void lin_make_args(formgpu_ctx *ctx, int n_tasks, LinArgs &a) {
   // CTAs per pair: as many as keep the launch within about one wave (2 CTAs per SM)
   a.cluster = kLinCluster;
   while (a.cluster > 1 && (size_t)a.cluster * (size_t)n_tasks > 2 * 148) a.cluster >>= 1;
-  if (const char *dbg = std::getenv("FORMGPU_DEBUG_CLUSTER")) a.cluster = std::max(1, std::atoi(dbg));
-  a.debug_flags = 0;
-  if (const char *dbg = std::getenv("FORMGPU_DEBUG_FLAGS")) a.debug_flags = std::atoi(dbg);
-  a.debug_ts = const_cast<unsigned long long *>(ctx->h_flags) + 8; // [16] behind the flags
   a.inv_sigma2 = 1.0 / (ctx->P.sigma * ctx->P.sigma);
   a.out = ctx->h_out;
   a.seq = ++ctx->seq;
@@ -186,15 +178,12 @@ namespace {
 // into mapped host memory.
 int run(formgpu_ctx *ctx, const formgpu_pair *pairs, size_t n_pairs, const formgpu_scan_pose *poses,
         size_t n_poses, bool error_only, double *out) {
-  using clk = std::chrono::steady_clock;
-  const auto t0 = clk::now();
   const size_t per_pair = error_only ? 1 : 91;
   static thread_local std::vector<LinTask> tasks;
   static thread_local std::vector<int> indices;
   int rc = lin_build_tasks(ctx, pairs, n_pairs, poses, n_poses, per_pair, out, tasks, indices);
   if (rc) return rc;
   unsigned long long seq = 0;
-  const auto t1 = clk::now();
   if (sharded_comm(ctx)) {
     // every rank evaluates the pairs from its partial moments into d_red (zeros for pairs without
     // a task), one all-reduce sums the blocks, the result is copied out
@@ -207,15 +196,7 @@ int run(formgpu_ctx *ctx, const formgpu_pair *pairs, size_t n_pairs, const formg
   }
   rc = lin_launch(ctx, tasks, error_only, &seq);
   if (rc) return rc;
-  const auto t2 = clk::now();
-  rc = lin_collect(ctx, indices, seq, per_pair, out);
-  if (rc) return rc;
-  const auto t3 = clk::now();
-  ctx->dbg_host_us[0] += std::chrono::duration<double, std::micro>(t1 - t0).count(); // build
-  ctx->dbg_host_us[1] += std::chrono::duration<double, std::micro>(t2 - t1).count(); // launch API
-  ctx->dbg_host_us[2] += std::chrono::duration<double, std::micro>(t3 - t2).count(); // wait
-  ctx->dbg_host_calls += 1;
-  return FORMGPU_OK;
+  return lin_collect(ctx, indices, seq, per_pair, out);
 }
 
 // device-output variants: blocks stay in device memory (zero-filled for empty pairs) and

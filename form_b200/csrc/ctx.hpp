@@ -13,7 +13,8 @@
 //   keypoint store d_store_planar  [W][kp_cap] PlanarRec       scan-local, lossless f32
 //                  d_store_point   [W][kq_cap] PointRec
 //   world map      d_hash_*        open-addressing voxel hash (per type)
-//                  d_world_*       voxel-sorted world points (32 B each)
+//                  d_world         voxel- and cell-ordered world points (32 B each)
+//                  d_world_src     their (slot, k), d_cell_tab: cell tables
 //   matches        d_match_*       per current keypoint: map id + dist^2
 //   correspondences d_seg_planar   [W][9][kp_cap] float        SoA p_i,n_i,p_j
 //                  d_seg_point     [W][6][kq_cap] float        SoA p_i,p_j
@@ -46,7 +47,7 @@ static_assert(sizeof(PlanarRec) == 32 && sizeof(PointRec) == 16, "record sizes")
 
 struct WorldPoint { // 32 B: world coordinates (f64) + tie-break key
   double x, y, z;
-  uint64_t tie; // (scan_id << 24) | k  -> rule R4/R5 ordering
+  uint64_t tie; // (rank of the scan id << 24) | k  -> rule R4/R5 ordering
 };
 static_assert(sizeof(WorldPoint) == 32, "WorldPoint size");
 
@@ -218,10 +219,11 @@ struct formgpu_ctx {
   unsigned char *d_mapmem = nullptr;
   formgpu::HashSlot *d_hash[2] = {nullptr, nullptr}; // views into d_mapmem (per rebuild)
   uint32_t hash_mask[2] = {0, 0};
-  formgpu::WorldPoint *d_world[2] = {nullptr, nullptr}; // voxel-sorted
-  formgpu::WorldPoint *d_world_tmp[2] = {nullptr, nullptr}; // unsorted, store order
-  uint32_t *d_world_slot[2] = {nullptr, nullptr}; // hash slot of each store point
-  uint32_t *d_world_src[2] = {nullptr, nullptr};  // voxel-sorted -> (slot<<20 | k)... see map.cu
+  // as the association reads them; the rebuild's first passes use them as scratch (MapArgs)
+  formgpu::WorldPoint *d_world[2] = {nullptr, nullptr};    // voxel- and cell-ordered map points
+  uint32_t *d_world_src[2] = {nullptr, nullptr};           // (window slot << 24 | k) of every map point
+  formgpu::WorldPoint *d_cell_tab[2] = {nullptr, nullptr}; // cell tables of the cell-ordered voxels
+  uint32_t *d_scatter_src[2] = {nullptr, nullptr};         // rebuild scratch
   uint32_t *d_voxel_list[2] = {nullptr, nullptr}; // hash slots of the occupied voxels
   size_t map_n[2] = {0, 0};                       // points in the built map
   size_t map_cap[2] = {0, 0};
@@ -231,9 +233,6 @@ struct formgpu_ctx {
   size_t map_req_bytes = 0;
   cudaEvent_t ev_upload = nullptr;    // guards reuse of the pinned request buffers
   bool map_built = false;
-  // voxel buckets ordered by 4x4x4 sub-cells, association searches cell by cell (default);
-  // FORMGPU_CELL_BUCKETS=0 at formgpu_create keeps the whole-bucket scans
-  bool cell_buckets = true;
   // single-sequence associations: warp-per-query whole-bucket search (lowest latency, default) or,
   // with FORMGPU_SINGLE_CELL_SEARCH=1, the cell search of the batched submits (tests)
   bool cell_search_single = false;
@@ -282,19 +281,15 @@ struct formgpu_ctx {
   unsigned *d_mom_tickets = nullptr; // [W], self-cleaning
   int mom_max_units = 0;
   uint32_t moment_unit = 128; // kMomentUnitSingle; contexts of a batch use kMomentUnit (api_batch.cu)
-  // linearize / error are evaluated from the cache (default) or, with
+  // linearize / error are evaluated from the cache (default, and always in a batch) or, with
   // FORMGPU_STREAM_LINEARIZE=1 and always in point-sharded mode, by streaming the correspondences
   bool moment_cache = true;
 
-  // ---- linearisation scratch ----
-  double *d_partials = nullptr;
-  size_t partial_cap = 0; // chunks
+  // ---- linearisation request ----
   void *d_request = nullptr;
   size_t request_bytes = 0;
   size_t out_cap = 0; // pairs
 
   // ---- instrumentation ----
   formgpu::Profiler prof;
-  double dbg_host_us[8] = {0, 0, 0, 0, 0, 0, 0, 0}; // host-side phase timers (experiments)
-  uint64_t dbg_host_calls = 0;
 };

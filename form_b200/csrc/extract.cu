@@ -1240,14 +1240,7 @@ void extract_batch_launch(const ExtractLaunchShape &sh, const ExtractArgs *items
     return v >= 32 && v <= 512 && v % 32 == 0 ? v : 192;
   }();
   const int select_threads = many_rows ? select_many : 512;
-  // development probe (the kernel is idempotent): how much does the step time move when this
-  // kernel's work doubles?
-  static const int repeat = [] {
-    const char *e = std::getenv("FORMGPU_DEBUG_SELECT_REPEAT");
-    return e ? std::atoi(e) : 0;
-  }();
-  for (int r = 0; r <= repeat; ++r)
-    extract_select_batch_kernel<<<grid, select_threads, sh.select_smem, stream>>>(items_dev);
+  extract_select_batch_kernel<<<grid, select_threads, sh.select_smem, stream>>>(items_dev);
   prof.end(FORMGPU_KG_EXTRACT_SELECT, 1);
   prof.begin(FORMGPU_KG_EXTRACT_NORMALS);
   // many rows: one thread per pick (one CTA per row); few rows: one warp per pick, four CTAs

@@ -116,20 +116,19 @@ struct MapArgs {
   int n_total;
   double voxel_width;
   double inv_voxel_width; // 1 / voxel_width (host, IEEE): fast path of voxel_coord
-  int cells;              // != 0: pass 4 orders the buckets of >= kCellMin points by cell code
-  int pad_cells;
   HashSlot *hash;
   uint32_t hash_mask;
-  WorldPoint *world_tmp; // store order; with cells: the FINAL voxel- and cell-sorted points
-  uint32_t *world_slot;  // hash slot per store-order point; with cells: the final world_src
-  uint32_t *world_src;   // voxel-sorted -> (window slot << 24 | k)
-  WorldPoint *world;     // voxel-sorted; with cells: the per-voxel cell tables (pass 4)
+  // what the association reads, written by pass 4; passes 1-3 use the arrays as scratch
+  WorldPoint *world;     // map points, voxel- and cell-ordered (pass 1: store order)
+  uint32_t *world_src;   // (window slot << 24 | k) of every map point (pass 1: hash slot per point)
+  WorldPoint *cell_tab;  // per-voxel cell tables (pass 3: the voxel-sorted points)
+  uint32_t *scatter_src; // pass 3: (window slot << 24 | k) of the voxel-sorted points
   uint32_t *cursor;      // [0] allocation cursor, [1] occupied voxels (zeroed before the build)
   uint32_t *voxel_list;  // hash slots of the occupied voxels, in creation order (insert pass)
 };
 /// Cell-ordered buckets (map_assoc.cu, pass 4): a voxel holding kCellMin..kCellMax points gets
-/// kCellFlag in its slot's count; its bucket is ordered by a kCellSub^3 cell code and carries a
-/// table of 64 u16 end offsets.
+/// kCellFlag in its slot's count; its bucket is ordered by a kCellSub^3 cell code and has a
+/// table of 64 u16 end offsets in cell_tab.
 constexpr uint32_t kCellFlag = 0x80000000u;
 constexpr uint32_t kCellMin = 16, kCellMax = 65535;
 constexpr int kCellSub = 4;
@@ -148,7 +147,7 @@ struct MapClearRegion {
 /// regions_dev[item] = the cursor + hash tables to clear first.
 /// `ring_dev`: base of the argument ring the regions' copy_src_off refer to.
 void map_build_batch_launch(const MapArgs *items_dev, const MapClearRegion *regions_dev, const unsigned char *ring_dev,
-                            int n_items, int max_points, uint32_t max_hash, size_t max_clear_bytes, bool cells,
+                            int n_items, int max_points, uint32_t max_hash, size_t max_clear_bytes,
                             cudaStream_t stream, Profiler &prof);
 
 struct AssocArgs {
@@ -164,8 +163,8 @@ struct AssocArgs {
   double pose[12];     // pose of the current scan
   double voxel_width;
   double inv_voxel_width; // 1 / voxel_width (host, IEEE): fast path of voxel_coord
-  // cell-ordered buckets: the offset table of a flagged voxel whose bucket starts at `start` lives
-  // in cell_tab[start .. start+3] (64 x u16 end offsets); nullptr = buckets are not cell-ordered
+  // the offset table of a flagged (cell-ordered) voxel whose bucket starts at `start` lives in
+  // cell_tab[start .. start+3] (64 x u16 end offsets)
   const WorldPoint *cell_tab;
   const HashSlot *hash;
   uint32_t hash_mask;
@@ -189,16 +188,13 @@ struct CombineArgs {
   int stride;                 // records per rank (planar + point candidates of the scan)
 };
 void assoc_combine_launch(const CombineArgs &planar, const CombineArgs &point, cudaStream_t stream, Profiler &prof);
-/// One sequence: `cell_search` = the one-thread-per-query search over the cell-ordered buckets (what
-/// batched submits always use); otherwise one WARP per query scans whole buckets - the lower
-/// latency for a single scan's ~30 k queries, which cannot fill the GPU either way.
+/// One sequence: `cell_search` = the one-thread-per-query search cell by cell (what batched submits
+/// always use); otherwise one WARP per query scans whole buckets - the lower latency for a single
+/// scan's ~30 k queries, which cannot fill the GPU either way.
 void assoc_launch(const AssocArgs &planar, const AssocArgs &point, bool cell_search, cudaStream_t stream,
                   Profiler &prof);
-/// `lanes` = lanes that share one query in the batched kernel (2, 4 or 8; kAssocLanes by default,
-/// FORMGPU_ASSOC_LANES overrides it per batch for tuning).
-constexpr int kAssocLanes = 4;
-void assoc_batch_launch(const AssocArgs *items_dev, int n_items, int max_query, int lanes, cudaStream_t stream,
-                        Profiler &prof);
+/// Batched submits: the cell search, one thread per query.
+void assoc_batch_launch(const AssocArgs *items_dev, int n_items, int max_query, cudaStream_t stream, Profiler &prof);
 
 struct SegmentArgs {
   int type;
@@ -288,9 +284,6 @@ struct LinArgs {
   int W;
   int n_tasks;
   int cluster;             // CTAs per pair for this launch: 1, 2, 4 or 8
-  int debug_flags;         // timing experiments only: 1 = skip system fence, 2 = skip expansion,
-                           // 4 = record %globaltimer checkpoints of pair 0 into debug_ts
-  unsigned long long *debug_ts; // [16] mapped pinned
   double inv_sigma2;
   // mapped pinned host memory (zero-copy), sequence-tagged words: [n_pairs][182] for
   // blocks, [n_pairs][2] for errors; word = 32 bits of payload | (seq & 0xffffffff) << 32
@@ -307,32 +300,9 @@ struct LinArgs {
   // pair-moment cache of the context (moments.cu): [W(j)][W(i)][kMomentStride] doubles
   const double *moments;
 };
-static_assert(sizeof(LinArgs) <= 128 && sizeof(LinArgs) % 8 == 0, "LinArgs: lin_warp_kernel copies it with lanes 16..31");
-/// Per-device attributes of the stage-3 kernels (formgpu_create, with the device current).
-cudaError_t linearize_configure();
+static_assert(sizeof(LinArgs) % 8 == 0, "LinArgs: the evaluation kernels copy it in 8-byte words");
 cudaError_t linearize_launch(const LinArgs &a, const LinInline *inline_req, bool error_only,
                              cudaStream_t stream, Profiler &prof);
-/// Batched launches: correspondences per warp slice the host aims for, and the slice table.
-constexpr uint32_t kLinWarpSlice = 384;     // shortest slice
-constexpr uint32_t kLinWarpSliceMax = 1536; // longest slice
-constexpr uint32_t kLinWarpTarget = 3552;   // warps aimed for: 2 x 148 SMs x 12 resident warps
-struct LinCta { // one warp-sized slice of a pair in a batched linearisation launch (32 B)
-  uint32_t task;  // index into the task array
-  uint32_t first; // index of the task's first slice (= base of its partial sums)
-  uint16_t rank;  // this slice's share of the pair: rank of n_cta
-  uint16_t n_cta; // slices of the pair
-  uint32_t ctx_index;      // = tasks[task].ctx_index, so task and context load together
-  const uint32_t *pair_row; // device [type][off|cnt][W+1] of the task's context (dynamic ranges)
-  uint32_t dyn_slot_i_plus1; // = tasks[task].dyn_slot_i_plus1
-  uint32_t row_stride;     // W + 1
-};
-static_assert(sizeof(LinCta) == 32, "LinCta size");
-/// Tasks of several contexts in one launch, one warp per slice (eight per CTA):
-/// ctx_args_dev[task.ctx_index] is the task's context; `partials` holds 56 doubles per
-/// slice, `tickets` one zeroed counter per task.
-cudaError_t linearize_warp_launch(const LinArgs *ctx_args_dev, const LinTask *tasks_dev,
-                                  const LinCta *entries_dev, int n_entries, double *partials,
-                                  unsigned *tickets, bool error_only, cudaStream_t stream, Profiler &prof);
 
 // ---- stage 3, cached form (moments.cu, FMA allowed: tolerance class) ----
 // Every association leaves, per pair (i, current scan), the POSE-INDEPENDENT second moments of

@@ -9,17 +9,6 @@ namespace formgpu {
 
 namespace {
 
-__device__ __forceinline__ unsigned long long globaltimer() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-#define LIN_TS(k)                                                                          \
-  do {                                                                                     \
-    if ((a.debug_flags & 4) && task.out_index == 0 && rank == 0 && tid == 0)               \
-      a.debug_ts[k] = globaltimer();                                                       \
-  } while (0)
-
 constexpr int kThreads = kLinThreads;
 constexpr int kWarps = kThreads / 32;
 
@@ -80,16 +69,6 @@ struct ExpandSmem {
   double Tq[3][7][13]; // per residual row r: W_q B_q[.][r]
 };
 
-// The basis only depends on the relative pose, so CTA 0 builds it at kernel start:
-// three threads fill it while the rest of the CTA is already streaming correspondences
-// (the first __syncthreads of the reduction publishes it).
-// kWarpScope: the cooperating group is one warp (small pairs of a batched launch) instead of
-// the CTA; `tid` / `nthreads` are then the lane and 32, and barriers are __syncwarp.
-template <bool kWarpScope> __device__ __forceinline__ void scope_sync() {
-  if (kWarpScope) __syncwarp();
-  else __syncthreads();
-}
-
 // entry (r, c) of the skew matrix [t]x
 __device__ __forceinline__ double skew_entry(const double *t, int r, int c) {
   if (r == c) return 0.0;
@@ -97,9 +76,8 @@ __device__ __forceinline__ double skew_entry(const double *t, int r, int c) {
   return ((c - r + 3) % 3 == 1) ? -v : v;
 }
 
-template <bool kWarpScope = false> __device__ __forceinline__ void zero_basis(ExpandSmem &S) {
-  const int tid = kWarpScope ? (int)(threadIdx.x & 31) : (int)threadIdx.x;
-  const int nthreads = kWarpScope ? 32 : (int)blockDim.x;
+__device__ __forceinline__ void zero_basis(ExpandSmem &S) {
+  const int tid = (int)threadIdx.x, nthreads = (int)blockDim.x;
   for (int i = tid; i < 7 * 13; i += nthreads) (&S.Bp[0][0])[i] = 0.0;
   for (int i = tid; i < 7 * 3 * 13; i += nthreads) (&S.Bq[0][0][0])[i] = 0.0;
 }
@@ -109,10 +87,8 @@ template <bool kWarpScope = false> __device__ __forceinline__ void zero_basis(Ex
 // kernel's stall samples: three serial chains while 125 threads waited at the barrier).
 //   plane-point: row = [ u1, -u2, -R^T u1 - R^T [t]x u2, R^T u2, -r ]
 //   point-point: rows = [ [P]x, -I, -[c]x R, R, -e ],  c = P + e - t
-template <bool kWarpScope = false>
 __device__ __forceinline__ void fill_basis(ExpandSmem &S, const double *rel, int first_thread = 0) {
-  const int tid = (kWarpScope ? (int)(threadIdx.x & 31) : (int)threadIdx.x) - first_thread;
-  const int nthreads = kWarpScope ? 32 : (int)blockDim.x;
+  const int tid = (int)threadIdx.x - first_thread, nthreads = (int)blockDim.x;
   const double *R = rel, *t = rel + 9;
   for (int item = tid; item >= 0 && item < 39; item += nthreads) {
     if (item < 9) { // (k, c)
@@ -152,11 +128,10 @@ __device__ __forceinline__ void fill_basis(ExpandSmem &S, const double *rel, int
 // The basis only depends on the relative pose, so CTA 0 builds it at kernel start while the
 // rest of the CTA is already streaming correspondences (the first __syncthreads of the
 // reduction publishes it).
-template <bool kWarpScope = false>
 __device__ __forceinline__ void build_basis(ExpandSmem &S, const double *rel) {
-  zero_basis<kWarpScope>(S);
-  scope_sync<kWarpScope>();
-  fill_basis<kWarpScope>(S, rel);
+  zero_basis(S);
+  __syncthreads();
+  fill_basis(S, rel);
 }
 
 // out = B^T W B in two short unrolled passes: T = W B (7 MACs per entry, all threads),
@@ -169,13 +144,11 @@ __device__ __forceinline__ void publish_tagged(volatile unsigned long long *dst,
   dst[1] = (bits >> 32) | (tag << 32);
 }
 
-template <bool kWarpScope = false>
 __device__ __forceinline__ void expand_and_publish(ExpandSmem &S, const double *Wp28, const double *Wq28,
                                                    bool has_planar, bool has_point, double inv_sigma2,
                                                    volatile unsigned long long *out182,
                                                    unsigned long long tag, double *plain91 = nullptr) {
-  const int tid = kWarpScope ? (int)(threadIdx.x & 31) : (int)threadIdx.x;
-  const int nthreads = kWarpScope ? 32 : (int)blockDim.x;
+  const int tid = (int)threadIdx.x, nthreads = (int)blockDim.x;
   if (tid < 28) {
     int p = 0, e = tid; // upper-triangular index -> (p, q)
     while (e >= 7 - p) {
@@ -186,7 +159,7 @@ __device__ __forceinline__ void expand_and_publish(ExpandSmem &S, const double *
     S.Wp[p][q] = S.Wp[q][p] = Wp28[tid];
     S.Wq[p][q] = S.Wq[q][p] = Wq28[tid];
   }
-  scope_sync<kWarpScope>();
+  __syncthreads();
   for (int idx = tid; idx < 91 + 273; idx += nthreads) {
     double v = 0.0;
     if (idx < 91) {
@@ -201,7 +174,7 @@ __device__ __forceinline__ void expand_and_publish(ExpandSmem &S, const double *
       S.Tq[r][k][y] = v;
     }
   }
-  scope_sync<kWarpScope>();
+  __syncthreads();
   for (int o = tid; o < 91; o += nthreads) {
     int x = 0, e = o;
     while (e >= 13 - x) {
@@ -233,56 +206,6 @@ __device__ __forceinline__ void shard_range(uint32_t n, int shard_rank, int shar
   const uint32_t hi = (uint32_t)(((unsigned long long)n * (unsigned)(shard_rank + 1)) / (unsigned)shard_world);
   begin = lo;
   count = hi - lo;
-}
-
-// Streaming 128-bit loads of the correspondence planes: read once, so they bypass L1
-// allocation; the data were written by an earlier kernel (segment scatter), hence .nc.
-__device__ __forceinline__ float4 ld_stream4(const float *p) {
-  float4 v;
-  asm("ld.global.nc.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];"
-      : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w)
-      : "l"(p));
-  return v;
-}
-
-#define LIN_COMP(v, k) ((k) == 0 ? (v).x : (k) == 1 ? (v).y : (k) == 2 ? (v).z : (v).w)
-
-// A warp streams the elements [lo, hi) of kPlanes SoA planes (`stride` floats apart, every
-// plane 16-byte aligned: the capacities are multiples of 4) as aligned float4 quads: lane l
-// owns the quads at a0 + 4 l + 128 c, a0 = lo rounded down to a quad.  The quad of the next
-// step is requested before the current one is reduced, so each lane keeps two 16-byte loads
-// per plane in flight (9 + 9 LDG.128 for plane-point rows) without staging through shared
-// memory; the first and last quad of a range are masked element by element.
-template <int kPlanes, typename Term>
-__device__ __forceinline__ void stream_quads(const float *base, size_t stride, uint32_t lo, uint32_t hi,
-                                             int lane, Term &&term) {
-  if (hi <= lo) return;
-  float4 cur[kPlanes], nxt[kPlanes];
-  uint32_t idx = (lo & ~3u) + 4u * (uint32_t)lane;
-  if (idx < hi) {
-#pragma unroll
-    for (int pl = 0; pl < kPlanes; ++pl) cur[pl] = ld_stream4(base + pl * stride + idx);
-  }
-#pragma unroll 1
-  for (; idx < hi; idx += 128u) {
-    const uint32_t nidx = idx + 128u;
-    if (nidx < hi) {
-#pragma unroll
-      for (int pl = 0; pl < kPlanes; ++pl) nxt[pl] = ld_stream4(base + pl * stride + nidx);
-    }
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const uint32_t e = idx + (uint32_t)k;
-      if (e >= lo && e < hi) {
-        float c[kPlanes];
-#pragma unroll
-        for (int pl = 0; pl < kPlanes; ++pl) c[pl] = LIN_COMP(cur[pl], k);
-        term(c);
-      }
-    }
-#pragma unroll
-    for (int pl = 0; pl < kPlanes; ++pl) cur[pl] = nxt[pl];
-  }
 }
 
 } // namespace

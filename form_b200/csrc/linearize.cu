@@ -88,7 +88,6 @@ __device__ __forceinline__ void lin_cluster_body(const LinArgs &a, const LinTask
 #pragma unroll
   for (int k = 0; k < 32; ++k) acc[k] = 0.0;
   double err_acc = 0.0;
-  LIN_TS(0);
   if (!kErrorOnly && rank == 0) build_basis(s_exp, task.rel);
 
   // ---- plane-point correspondences of this CTA's slice ----
@@ -117,13 +116,11 @@ __device__ __forceinline__ void lin_cluster_body(const LinArgs &a, const LinTask
       }
     }
   }
-  LIN_TS(1);
   if (!kErrorOnly) {
     block_reduce28(acc, s_warp, s_sum[0], tid);
 #pragma unroll
     for (int k = 0; k < 32; ++k) acc[k] = 0.0;
   }
-  LIN_TS(2);
   // ---- point-point correspondences ----
   {
     const uint32_t lo = (uint32_t)(((unsigned long long)task.n_point * rank) / kCluster);
@@ -164,9 +161,7 @@ __device__ __forceinline__ void lin_cluster_body(const LinArgs &a, const LinTask
   }
 
   // ---- gather the CTA sums through distributed shared memory ----
-  LIN_TS(3);
   cluster.sync();
-  LIN_TS(4);
   if (rank == 0) {
     if (kErrorOnly) {
       if (tid == 0) {
@@ -181,9 +176,7 @@ __device__ __forceinline__ void lin_cluster_body(const LinArgs &a, const LinTask
       s_total[which][e] = v;
     }
   }
-  LIN_TS(5);
   cluster.sync(); // the other CTAs' shared memory must outlive CTA 0's remote reads
-  LIN_TS(6);
   if (rank != 0) return;
   __syncthreads();
   // Publish straight into mapped pinned host memory.  Every 8-byte word carries the
@@ -196,12 +189,11 @@ __device__ __forceinline__ void lin_cluster_body(const LinArgs &a, const LinTask
       if (a.out_plain) a.out_plain[task.out_index] = s_total[0][0];
       else publish_tagged(a.out + 2 * (size_t)task.out_index, s_total[0][0], tag);
     }
-  } else if (!(a.debug_flags & 2)) {
+  } else {
     expand_and_publish(s_exp, s_total[0], s_total[1], has_planar, has_point, a.inv_sigma2,
                        a.out + 182 * (size_t)task.out_index, tag,
                        a.out_plain ? a.out_plain + 91 * (size_t)task.out_index : nullptr);
   }
-  LIN_TS(7);
 }
 
 } // namespace
@@ -219,205 +211,6 @@ __global__ void __launch_bounds__(kLinThreads) lin_global_kernel(LinArgs a) {
         reinterpret_cast<const unsigned long long *>(a.tasks + blockIdx.x / a.cluster)[threadIdx.x];
   __syncthreads();
   lin_cluster_body<kErrorOnly>(a, s_task);
-}
-
-// ---------------------------------------------------------------------------
-// batched launches: the tasks of several contexts in ONE grid, one WARP per slice
-// ---------------------------------------------------------------------------
-// A batched request holds hundreds of pairs of very different sizes (the pair with the
-// oldest key scan has ~15 k correspondences, most others a few hundred).  One cluster - or
-// one CTA - per pair leaves the launch latency-bound: ncu showed the CTAs waiting at the
-// barriers of their two block reductions (30 % of the stall samples) and on the partial-sum
-// fence, at 16 resident warps per SM.  Here the unit of work is a WARP: the host cuts every
-// pair into slices of about kLinWarpSlice correspondences (estimate; the kernel divides the
-// TRUE range by the slice count), a warp streams its slice as aligned 128-bit loads straight
-// into registers, two quads per plane in flight, reduces its 2 x 28 moments with the butterfly transpose alone - no
-// barrier anywhere in the kernel - and, if the pair has several slices, leaves them in
-// global memory and takes a ticket; the LAST warp of the pair adds the partial sums in slice
-// order (a fixed order, so the result does not depend on which warp came last), expands the
-// block in its own slice of shared memory and publishes it.  task.ctx_index selects the
-// context's argument block (segments, pair row, result buffer, sequence tag).
-constexpr int kLinWarpThreads = 128;              // 4 warps per CTA
-constexpr int kLinWarpTasks = kLinWarpThreads / 32;
-
-// Shared memory of one warp: its task / context blocks, the two moment vectors and the
-// expansion scratch of the pair's last warp.
-struct LinWarpSmem {
-  ExpandSmem exp;
-  LinTask task;
-  LinArgs args;
-  double sum[2][28];
-  uint32_t dyn[4];
-};
-
-template <bool kErrorOnly>
-__global__ void __launch_bounds__(kLinWarpThreads, 3)
-lin_warp_kernel(const LinArgs *ctx_args, const LinTask *tasks, const LinCta *entries, int n_entries,
-                double *partials, unsigned *tickets) {
-  extern __shared__ __align__(16) unsigned char lin_warp_smem[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int ei = blockIdx.x * kLinWarpTasks + warp;
-  if (ei >= n_entries) return;
-  LinWarpSmem &S = reinterpret_cast<LinWarpSmem *>(lin_warp_smem)[warp];
-  const LinCta me = entries[ei];
-  // task, context block and (for dynamic ranges) the pair row are independent loads
-  if (lane < (int)(sizeof(LinTask) / sizeof(unsigned long long)))
-    reinterpret_cast<unsigned long long *>(&S.task)[lane] =
-        reinterpret_cast<const unsigned long long *>(tasks + me.task)[lane];
-  if (lane >= 16 && lane < 16 + (int)(sizeof(LinArgs) / sizeof(unsigned long long)))
-    reinterpret_cast<unsigned long long *>(&S.args)[lane - 16] =
-        reinterpret_cast<const unsigned long long *>(ctx_args + me.ctx_index)[lane - 16];
-  if (lane < 4 && me.dyn_slot_i_plus1) // ranges written by the association queued just before
-    S.dyn[lane] = __ldcg(&me.pair_row[(size_t)lane * me.row_stride + (me.dyn_slot_i_plus1 - 1u)]);
-  __syncwarp();
-  const LinArgs &a = S.args;
-  uint32_t off_planar = S.task.off_planar, n_planar = S.task.n_planar;
-  uint32_t off_point = S.task.off_point, n_point = S.task.n_point;
-  if (me.dyn_slot_i_plus1) {
-    off_planar = S.dyn[0];
-    n_planar = S.dyn[1];
-    off_point = S.dyn[2];
-    n_point = S.dyn[3];
-    if (n_planar + n_point == 0) return; // empty pair: all its warps leave, nothing is published
-  }
-  const double *rel = S.task.rel; // relative pose of the pair (shared memory)
-  const int rank = me.rank, n_slices = me.n_cta;
-  // this warp's slice of the planar and of the point range
-  const uint32_t p_lo = (uint32_t)(((unsigned long long)n_planar * rank) / n_slices);
-  const uint32_t p_hi = (uint32_t)(((unsigned long long)n_planar * (rank + 1)) / n_slices);
-  const uint32_t q_lo = (uint32_t)(((unsigned long long)n_point * rank) / n_slices);
-  const uint32_t q_hi = (uint32_t)(((unsigned long long)n_point * (rank + 1)) / n_slices);
-  // plane 0 of the segment of slot_j; element indices below are relative to it
-  const float *gp = a.seg_planar + (size_t)S.task.slot_j * 9 * a.kp_cap;
-  const float *gq = a.seg_point + (size_t)S.task.slot_j * 6 * a.kq_cap;
-  const size_t stp = a.kp_cap, stq = a.kq_cap;
-  const double inv_sigma2 = a.inv_sigma2;
-  const unsigned long long tag = a.seq & 0xffffffffull;
-  volatile unsigned long long *out = a.out;
-  const int out_index = S.task.out_index;
-
-  double acc[32];
-  double err_acc = 0.0;
-#pragma unroll
-  for (int k = 0; k < 32; ++k) acc[k] = 0.0;
-  stream_quads<9>(gp, stp, off_planar + p_lo, off_planar + p_hi, lane, [&](const float(&c)[9]) {
-    const double pix = c[0], piy = c[1], piz = c[2];
-    const double nx = c[3], ny = c[4], nz = c[5];
-    double qx, qy, qz;
-    apply_rel(rel, (double)c[6], (double)c[7], (double)c[8], qx, qy, qz);
-    const double r = nx * (qx - pix) + ny * (qy - piy) + nz * (qz - piz);
-    if (kErrorOnly) {
-      err_acc += r * r;
-    } else {
-      const double v[7] = {ny * qz - nz * qy, nz * qx - nx * qz, nx * qy - ny * qx, nx, ny, nz, r};
-      int e = 0;
-#pragma unroll
-      for (int p = 0; p < 7; ++p)
-#pragma unroll
-        for (int q = p; q < 7; ++q) acc[e++] += v[p] * v[q];
-    }
-  });
-  if (!kErrorOnly) {
-    transpose_reduce<16>(acc, lane);
-    if (lane < 28) S.sum[0][lane] = acc[0];
-#pragma unroll
-    for (int k = 0; k < 32; ++k) acc[k] = 0.0;
-  }
-  stream_quads<6>(gq, stq, off_point + q_lo, off_point + q_hi, lane, [&](const float(&c)[6]) {
-    const double pix = c[0], piy = c[1], piz = c[2];
-    double qx, qy, qz;
-    apply_rel(rel, (double)c[3], (double)c[4], (double)c[5], qx, qy, qz);
-    const double ex = qx - pix, ey = qy - piy, ez = qz - piz;
-    if (kErrorOnly) {
-      err_acc += ex * ex + ey * ey + ez * ez;
-    } else {
-      const double v[7] = {pix, piy, piz, ex, ey, ez, 1.0};
-      int e = 0;
-#pragma unroll
-      for (int p = 0; p < 7; ++p)
-#pragma unroll
-        for (int q = p; q < 7; ++q) acc[e++] += v[p] * v[q];
-    }
-  });
-  if (kErrorOnly) {
-    double w = warp_sum(err_acc);
-    if (n_slices > 1) {
-      double *mine = partials + (size_t)(me.first + rank) * 56;
-      unsigned ticket = 0;
-      if (lane == 0) {
-        mine[0] = w;
-        __threadfence();
-        ticket = atomicAdd(&tickets[me.task], 1u);
-      }
-      ticket = __shfl_sync(0xffffffffu, ticket, 0);
-      if (ticket != (unsigned)(n_slices - 1)) return;
-      if (lane == 0) {
-        tickets[me.task] = 0u; // self-cleaning for the next launch
-        __threadfence();
-        const double *all = partials + (size_t)me.first * 56;
-        w = 0.0;
-        for (int r = 0; r < n_slices; ++r) w += __ldcg(&all[(size_t)r * 56]); // slice order
-      }
-    }
-    if (lane == 0) publish_tagged(out + 2 * (size_t)out_index, 0.5 * w * inv_sigma2, tag);
-    return;
-  }
-  if (q_hi > q_lo) transpose_reduce<16>(acc, lane); // warp-uniform; acc is all zero otherwise
-  if (lane < 28) S.sum[1][lane] = acc[0];
-  if (n_slices > 1) {
-    // leave the partial sums, take a ticket; the last warp of the pair finishes it
-    __syncwarp();
-    double *mine = partials + (size_t)(me.first + rank) * 56;
-    for (int e = lane; e < 56; e += 32) mine[e] = S.sum[e / 28][e % 28];
-    __threadfence();
-    __syncwarp();
-    unsigned ticket = 0;
-    if (lane == 0) ticket = atomicAdd(&tickets[me.task], 1u);
-    ticket = __shfl_sync(0xffffffffu, ticket, 0);
-    if (ticket != (unsigned)(n_slices - 1)) return;
-    if (lane == 0) tickets[me.task] = 0u; // self-cleaning for the next launch
-    __threadfence();
-    const double *all = partials + (size_t)me.first * 56;
-    // slice order (deterministic); eight loads in flight per step - a pair of 40 slices is 5
-    // L2 round trips on the launch's critical path instead of 40
-    double v0 = 0.0, v1 = 0.0; // elements lane and lane + 32
-    int r = 0;
-    for (; r + 8 <= n_slices; r += 8) {
-      double t0[8], t1[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        t0[u] = __ldcg(&all[(size_t)(r + u) * 56 + lane]);
-        t1[u] = lane < 24 ? __ldcg(&all[(size_t)(r + u) * 56 + 32 + lane]) : 0.0;
-      }
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        v0 += t0[u];
-        v1 += t1[u];
-      }
-    }
-    for (; r < n_slices; ++r) {
-      v0 += __ldcg(&all[(size_t)r * 56 + lane]);
-      if (lane < 24) v1 += __ldcg(&all[(size_t)r * 56 + 32 + lane]);
-    }
-    S.sum[lane / 28][lane % 28] = v0;
-    if (lane < 24) S.sum[(32 + lane) / 28][(32 + lane) % 28] = v1;
-  }
-  __syncwarp();
-  build_basis<true>(S.exp, rel); // starts with a __syncwarp
-  __syncwarp();
-  expand_and_publish<true>(S.exp, S.sum[0], S.sum[1], n_planar > 0, n_point > 0, inv_sigma2,
-                           out + 182 * (size_t)out_index, tag);
-}
-
-size_t lin_warp_smem_bytes() { return sizeof(LinWarpSmem) * kLinWarpTasks; }
-
-// Per-device kernel attributes: called by formgpu_create with the context's device current, so
-// every device a process drives is configured (no process-wide "done" flag).
-cudaError_t linearize_configure() {
-  const int smem = (int)lin_warp_smem_bytes();
-  cudaError_t e = cudaFuncSetAttribute(lin_warp_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e != cudaSuccess) return e;
-  return cudaFuncSetAttribute(lin_warp_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
 }
 
 namespace {
@@ -455,24 +248,6 @@ cudaError_t linearize_launch(const LinArgs &a, const LinInline *inline_req, bool
   }
   prof.end(group, 1);
   return e;
-}
-
-cudaError_t linearize_warp_launch(const LinArgs *ctx_args_dev, const LinTask *tasks_dev,
-                                  const LinCta *entries_dev, int n_entries, double *partials,
-                                  unsigned *tickets, bool error_only, cudaStream_t stream, Profiler &prof) {
-  if (n_entries <= 0) return cudaSuccess;
-  const size_t smem = lin_warp_smem_bytes();
-  const int group = error_only ? FORMGPU_KG_ERR_CHUNK : FORMGPU_KG_LIN_CHUNK;
-  const int grid = (n_entries + kLinWarpTasks - 1) / kLinWarpTasks;
-  prof.begin(group);
-  if (error_only)
-    lin_warp_kernel<true><<<grid, kLinWarpThreads, smem, stream>>>(ctx_args_dev, tasks_dev, entries_dev, n_entries,
-                                                                   partials, tickets);
-  else
-    lin_warp_kernel<false><<<grid, kLinWarpThreads, smem, stream>>>(ctx_args_dev, tasks_dev, entries_dev,
-                                                                    n_entries, partials, tickets);
-  prof.end(group, 1);
-  return cudaGetLastError();
 }
 
 } // namespace formgpu

@@ -12,19 +12,18 @@
 //   * an open-addressing table of 16-byte slots {packed voxel key, start, count}
 //     (linear probing, 64-bit CAS insert, load factor <= 0.5), and
 //   * the world points (32 B: x, y, z f64 + tie-break id) stored contiguously
-//     per voxel (CSR), so a bucket scan is a run of whole 32-byte sectors.
-// Search is cooperative: a group of lanes (32 for a single sequence, 4 by default in batched
-// submits) shares one query - it scans the centre voxel's bucket together, bounds the distance to
-// the 26 neighbour voxels of the reference's shift table (map.tpp:54-68) from the six faces of
-// the centre voxel, probes only the voxels that can still hold a closer point and scans their
-// buckets; a shuffle arg-min with the key (dist^2, shift rank, scan, k) implements rule R5
-// (identical to the reference's strict-< visiting order).
+//     per voxel (CSR), so a bucket scan is a run of whole 32-byte sectors; buckets of
+//     kCellMin..kCellMax points are ordered by 4x4x4 sub-cells and carry a cell table.
+// Two searches: a single sequence's association shares one query between the 32 lanes of a warp
+// (assoc_nn_body: whole buckets of the centre voxel and of the neighbour voxels of the reference's
+// shift table, map.tpp:54-68, that the face bounds cannot rule out); batched submits give a query
+// to one thread, which searches cell by cell (assoc_cells_body).  Both take the arg-min of the key
+// (dist^2, shift rank, scan, k): rule R5, identical to the reference's strict-< visiting order.
 #include "ctx.hpp"
 #include "kernels.hpp"
 
 #include <algorithm>
 #include <cfloat>
-#include <cstdlib>
 
 namespace formgpu {
 
@@ -178,11 +177,11 @@ __device__ __forceinline__ void map_insert_body(const MapArgs &a) {
     h = (h + 1) & a.hash_mask;
   }
   atomicAdd(&a.hash[h].count, 1u);
-  a.world_slot[g] = h;
+  a.world_src[g] = h;
   WorldPoint wp;
   wp.x = wx; wp.y = wy; wp.z = wz;
   wp.tie = ((unsigned long long)a.slot_rank[slot] << 24) | (unsigned long long)k; // rule R4 id
-  a.world_tmp[g] = wp;
+  a.world[g] = wp;
 }
 } // namespace
 __global__ void __launch_bounds__(256) map_insert_kernel(MapArgs pa, MapArgs qa) {
@@ -207,7 +206,7 @@ __device__ __forceinline__ void map_alloc_body(const MapArgs &a) {
   // cell-ordered bucket (map_cells_body): the flag travels in the count's top bit, and the voxel
   // enters the list of cell-ordered voxels, which grows downwards from the end of voxel_list
   // (occupied + cell-ordered voxels <= points, so the two lists cannot meet)
-  if (a.cells && cnt >= kCellMin && cnt <= kCellMax) {
+  if (cnt >= kCellMin && cnt <= kCellMax) {
     a.hash[h].count = cnt | kCellFlag;
     a.voxel_list[(uint32_t)a.n_total - 1u - atomicAdd(a.cursor + 2, 1u)] = h;
   }
@@ -222,7 +221,7 @@ __global__ void __launch_bounds__(256) map_alloc_batch_kernel(const MapArgs *ite
   map_alloc_body(s_a);
 }
 
-// pass 3: scatter into voxel-contiguous order
+// pass 3: scatter into voxel-contiguous order (`cell_tab`, `scatter_src`)
 namespace {
 __device__ __forceinline__ void map_scatter_body(const MapArgs &a) {
   __shared__ int s_off[kMaxWindow + 1];
@@ -230,11 +229,11 @@ __device__ __forceinline__ void map_scatter_body(const MapArgs &a) {
   __syncthreads();
   const int g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= a.n_total) return;
-  const uint32_t h = a.world_slot[g];
+  const uint32_t h = a.world_src[g];
   const uint32_t pos = atomicSub(&a.hash[h].start, 1u) - 1u;
-  a.world[pos] = a.world_tmp[g];
+  a.cell_tab[pos] = a.world[g];
   const int slot = find_slot_of(s_off, a.W, g);
-  a.world_src[pos] = ((uint32_t)slot << 24) | (uint32_t)(g - s_off[slot]);
+  a.scatter_src[pos] = ((uint32_t)slot << 24) | (uint32_t)(g - s_off[slot]);
 }
 } // namespace
 __global__ void __launch_bounds__(256) map_scatter_kernel(MapArgs pa, MapArgs qa) {
@@ -246,11 +245,11 @@ __global__ void __launch_bounds__(256) map_scatter_batch_kernel(const MapArgs *i
   map_scatter_body(s_a);
 }
 
-// pass 4 (cell-ordered buckets): copy every bucket from the scatter pass's output (`world`,
-// `world_src`) into the final arrays (`world_tmp`, `world_slot` - both dead once the scatter pass
+// pass 4 (cell-ordered buckets): copy every bucket from the scatter pass's output (`cell_tab`,
+// `scatter_src`) into the final arrays (`world`, `world_src` - both dead once the scatter pass
 // has run), ordering the buckets of kCellMin..kCellMax points by the kCellSub^3 cell code of
 // their points, and leave the table of the cells' END offsets (64 x u16 = 128 B) in the first
-// four records of `world` at the bucket's position - the source copy is dead by then, and a
+// four records of `cell_tab` at the bucket's position - the source copy is dead by then, and a
 // flagged bucket has at least kCellMin >= 4 records, so every voxel owns its table slot without
 // any allocation.  One warp per voxel, any bucket size: histogram over the 64 cells (integer
 // shared-memory atomics), exclusive prefix, scatter.  The order inside a cell is arbitrary, like
@@ -276,7 +275,7 @@ __device__ __forceinline__ int unpack_coord(unsigned long long key, int shift) {
 
 __device__ __forceinline__ void map_cells_body(const MapArgs &a) {
   __shared__ CellSmem s_cells[kCellWarps];
-  if (!a.cells || a.n_total <= 0) return;
+  if (a.n_total <= 0) return;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   CellSmem &S = s_cells[warp];
   const double w = a.voxel_width, inv_cw = (double)kCellSub * a.inv_voxel_width;
@@ -286,8 +285,8 @@ __device__ __forceinline__ void map_cells_body(const MapArgs &a) {
     const HashSlot s = a.hash[a.voxel_list[i]];
     if (s.count & kCellFlag) continue;
     for (uint32_t k = 0; k < s.count; ++k) {
-      a.world_tmp[s.start + k] = a.world[s.start + k];
-      a.world_slot[s.start + k] = a.world_src[s.start + k];
+      a.world[s.start + k] = a.cell_tab[s.start + k];
+      a.world_src[s.start + k] = a.scatter_src[s.start + k];
     }
   }
   // ---- cell-ordered buckets: one WARP per voxel ----
@@ -313,19 +312,19 @@ __device__ __forceinline__ void map_cells_body(const MapArgs &a) {
     int c0 = -1, c1 = -1;
     if (in_regs) {
       if ((uint32_t)lane < cnt) {
-        p0 = a.world[start + lane];
-        src0 = a.world_src[start + lane];
+        p0 = a.cell_tab[start + lane];
+        src0 = a.scatter_src[start + lane];
         c0 = code_of(p0);
         atomicAdd(&S.hist[c0], 1u);
       }
       if ((uint32_t)lane + 32u < cnt) {
-        p1 = a.world[start + lane + 32];
-        src1 = a.world_src[start + lane + 32];
+        p1 = a.cell_tab[start + lane + 32];
+        src1 = a.scatter_src[start + lane + 32];
         c1 = code_of(p1);
         atomicAdd(&S.hist[c1], 1u);
       }
     } else {
-      for (uint32_t i = lane; i < cnt; i += 32) atomicAdd(&S.hist[code_of(a.world[start + i])], 1u);
+      for (uint32_t i = lane; i < cnt; i += 32) atomicAdd(&S.hist[code_of(a.cell_tab[start + i])], 1u);
     }
     __syncwarp();
     // exclusive prefix over the 64 bins, two per lane
@@ -343,25 +342,25 @@ __device__ __forceinline__ void map_cells_body(const MapArgs &a) {
     if (in_regs) {
       if (c0 >= 0) {
         const uint32_t pos = atomicAdd(&S.cur[c0], 1u);
-        a.world_tmp[start + pos] = p0;
-        a.world_slot[start + pos] = src0;
+        a.world[start + pos] = p0;
+        a.world_src[start + pos] = src0;
       }
       if (c1 >= 0) {
         const uint32_t pos = atomicAdd(&S.cur[c1], 1u);
-        a.world_tmp[start + pos] = p1;
-        a.world_slot[start + pos] = src1;
+        a.world[start + pos] = p1;
+        a.world_src[start + pos] = src1;
       }
     } else {
       for (uint32_t i = lane; i < cnt; i += 32) {
-        const WorldPoint p = a.world[start + i];
+        const WorldPoint p = a.cell_tab[start + i];
         const uint32_t pos = atomicAdd(&S.cur[code_of(p)], 1u);
-        a.world_tmp[start + pos] = p;
-        a.world_slot[start + pos] = a.world_src[start + i];
+        a.world[start + pos] = p;
+        a.world_src[start + pos] = a.scatter_src[start + i];
       }
     }
     __syncwarp(); // every read of the source bucket is done: its head becomes the table
     // END offsets of cells 2 lane and 2 lane + 1 as one 32-bit word
-    reinterpret_cast<uint32_t *>(a.world + start)[lane] = (excl + h0) | ((excl + h0 + h1) << 16);
+    reinterpret_cast<uint32_t *>(a.cell_tab + start)[lane] = (excl + h0) | ((excl + h0 + h1) << 16);
     __syncwarp();
   }
 }
@@ -401,18 +400,14 @@ void map_build_launch(const MapArgs &pa, const MapArgs &qa, cudaStream_t stream,
   const int nt = max(pa.n_total, qa.n_total); // voxels <= points
   map_alloc_kernel<<<dim3((nt + 255) / 256, 2), 256, 0, stream>>>(pa, qa);
   map_scatter_kernel<<<gp, 256, 0, stream>>>(pa, qa);
-  int launches = 3;
-  if (pa.cells || qa.cells) {
-    // grid-stride: a thread per small voxel, a warp per cell-ordered voxel (<= points / 16)
-    const unsigned blocks = std::max(1u, std::min<unsigned>((unsigned)nt / (16u * kCellWarps) + 1u, 8 * 148));
-    map_cells_kernel<<<dim3(blocks, 2), kCellWarps * 32, 0, stream>>>(pa, qa);
-    ++launches;
-  }
-  prof.end(FORMGPU_KG_MAP_BUILD, launches);
+  // grid-stride: a thread per small voxel, a warp per cell-ordered voxel (<= points / 16)
+  const unsigned blocks = std::max(1u, std::min<unsigned>((unsigned)nt / (16u * kCellWarps) + 1u, 8 * 148));
+  map_cells_kernel<<<dim3(blocks, 2), kCellWarps * 32, 0, stream>>>(pa, qa);
+  prof.end(FORMGPU_KG_MAP_BUILD, 4);
 }
 
 void map_build_batch_launch(const MapArgs *items_dev, const MapClearRegion *regions_dev, const unsigned char *ring_dev,
-                            int n_items, int max_points, uint32_t max_hash, size_t max_clear_bytes, bool cells,
+                            int n_items, int max_points, uint32_t max_hash, size_t max_clear_bytes,
                             cudaStream_t stream, Profiler &prof) {
   if (n_items <= 0) return;
   prof.begin(FORMGPU_KG_MAP_BUILD);
@@ -424,13 +419,9 @@ void map_build_batch_launch(const MapArgs *items_dev, const MapClearRegion *regi
     map_insert_batch_kernel<<<gp, 256, 0, stream>>>(items_dev);
     map_alloc_batch_kernel<<<dim3((max_points + 255) / 256, 2, n_items), 256, 0, stream>>>(items_dev);
     map_scatter_batch_kernel<<<gp, 256, 0, stream>>>(items_dev);
-    launches += 3;
-    if (cells) {
-      const unsigned blocks =
-          std::max(1u, std::min<unsigned>((unsigned)max_points / (16u * kCellWarps) + 1u, 512u));
-      map_cells_batch_kernel<<<dim3(blocks, 2, n_items), kCellWarps * 32, 0, stream>>>(items_dev);
-      ++launches;
-    }
+    const unsigned blocks = std::max(1u, std::min<unsigned>((unsigned)max_points / (16u * kCellWarps) + 1u, 512u));
+    map_cells_batch_kernel<<<dim3(blocks, 2, n_items), kCellWarps * 32, 0, stream>>>(items_dev);
+    launches += 4;
   }
   prof.end(FORMGPU_KG_MAP_BUILD, launches);
 }
@@ -444,23 +435,6 @@ __device__ __forceinline__ int match_bin(const MatchRec &m, double max_d2) {
   return (m.slot != kNoSlot && m.dist_sqrd < max_d2) ? (int)m.slot : -1;
 }
 
-
-// A few lanes per query (kQueryLanes: 4 by default in batched submits, i.e. eight queries per
-// warp).  Every instruction of the per-query setup (f64 transform, voxel key, hashing, face
-// distances, arg-min) then serves several queries instead of one - the one-warp-per-query
-// version was issue-bound on exactly that redundant work (ncu: 67 % issue-active, 420 warp
-// instructions per query; 121 with four lanes).  Fewer lanes also mean longer per-lane bucket
-// scans whose lengths diverge across the warp: two lanes measured 2 % slower than four.
-//
-// Order of the search: (1) the group probes the CENTRE voxel and scans its bucket together;
-// (2) every lane bounds the squared distance from the query to the boxes of its share of the 26
-// neighbour voxels (pure arithmetic on the distances to the six faces of the centre voxel) and
-// keeps those that can still hold a point at least as close as the centre's best - exact
-// pruning: a skipped voxel cannot change the arg-min; (3) the surviving voxel ranks (typically
-// one to four of 26) are compacted through shared memory so that lane s of the group probes the
-// s-th survivor - one hash probe per lane instead of four; (4) the group scans the survivors'
-// buckets one after the other.  The arg-min key (dist^2, shift rank, scan, k) is rule R5, so
-// neither the scan order nor the split over lanes matters.
 // Read-only loads of the map go through the non-coherent path (the argument block lives in
 // shared memory in the batched kernel, which hides from the compiler that these are global).
 __device__ __forceinline__ HashSlot load_slot(const HashSlot *p) {
@@ -499,23 +473,29 @@ __device__ __forceinline__ void probe_voxel(const HashSlot *hash, uint32_t mask,
   }
 }
 
-// A single sequence's call (20 k queries) cannot fill the GPU either way and is latency-
-// bound, so it keeps 32 lanes per query (shortest bucket scans); batched launches use kAssocLanes.
-constexpr int kLanesSingle = 32;
-__host__ __device__ constexpr int queries_per_cta(int lanes) { return 8 * (32 / lanes); } // 256 threads
+// One WARP per query: a single sequence's call (20 k queries) cannot fill the GPU either way and
+// is latency-bound, so the 32 lanes of a warp share a query (shortest bucket scans).
+//
+// Order of the search: (1) the warp probes the CENTRE voxel and scans its bucket together;
+// (2) lane v bounds the squared distance from the query to the box of the neighbour voxel with
+// shift rank v (1..26; pure arithmetic on the distances to the six faces of the centre voxel) and
+// keeps it if it can still hold a point at least as close as the centre's best - exact pruning:
+// a skipped voxel cannot change the arg-min; (3) the surviving voxel ranks (typically one to four
+// of 26) are compacted through shared memory so that lane s probes the s-th survivor; (4) the
+// warp scans the survivors' buckets one after the other.  The arg-min key (dist^2, shift rank,
+// scan, k) is rule R5, so neither the scan order nor the split over lanes matters.
+constexpr int kNnWarps = 8; // queries per CTA (256 threads)
 
 namespace {
-template <int kQueryLanes> __device__ __forceinline__ void assoc_nn_body(const AssocArgs &a) {
-  constexpr int kGroups = 32 / kQueryLanes;                  // queries per warp
-  constexpr int kVox = (27 + kQueryLanes - 1) / kQueryLanes; // voxel ranks owned by a lane
-  constexpr int kDepth = kQueryLanes >= 32 ? 2 : 3;          // bucket points a lane keeps in flight
-  __shared__ unsigned char s_list[8][kGroups][28];           // compacted surviving voxel ranks
-  __shared__ uint2 s_bucket[8][kGroups][27];                 // their buckets {start, count}
-  const int lane = threadIdx.x & 31, sub = lane & (kQueryLanes - 1), grp = lane / kQueryLanes;
+__device__ __forceinline__ void assoc_nn_body(const AssocArgs &a) {
+  constexpr int kDepth = 2;                  // bucket points a lane keeps in flight
+  __shared__ unsigned char s_list[kNnWarps][28]; // compacted surviving voxel ranks
+  __shared__ uint2 s_bucket[kNnWarps][27];       // their buckets {start, count}
+  const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
-  const int q = (blockIdx.x * (blockDim.x >> 5) + warp) * kGroups + grp;
+  const int q = blockIdx.x * (blockDim.x >> 5) + warp;
   const int nb = a.W + 1;
-  const bool active = q >= a.q_begin && q < a.q_end; // whole groups are active or not; shuffles need every lane
+  const bool active = q >= a.q_begin && q < a.q_end; // the whole warp is active or not; shuffles need every lane
   const bool searchable = active && a.n_map > 0;
   double x = 0.0, y = 0.0, z = 0.0;
   if (active) {
@@ -543,21 +523,21 @@ template <int kQueryLanes> __device__ __forceinline__ void assoc_nn_body(const A
       best_pos = pos;
     }
   };
-  // the group scans a bucket together, kQueryLanes consecutive 32-byte points per step; a lane
-  // requests its next kDepth points before it looks at the first
+  // the warp scans a bucket together, 32 consecutive 32-byte points per step; a lane requests its
+  // next kDepth points before it looks at the first
   auto scan_bucket = [&](int b, uint32_t sb, uint32_t cb) {
-    uint32_t i = sub;
-    for (; i + (kDepth - 1) * kQueryLanes < cb; i += kDepth * kQueryLanes) {
+    uint32_t i = lane;
+    for (; i + (kDepth - 1) * 32 < cb; i += kDepth * 32) {
       WorldPoint p[kDepth];
 #pragma unroll
-      for (int u = 0; u < kDepth; ++u) p[u] = load_world(a.world + sb + i + u * kQueryLanes);
+      for (int u = 0; u < kDepth; ++u) p[u] = load_world(a.world + sb + i + u * 32);
 #pragma unroll
-      for (int u = 0; u < kDepth; ++u) consider(p[u], sb + i + u * kQueryLanes, b);
+      for (int u = 0; u < kDepth; ++u) consider(p[u], sb + i + u * 32, b);
     }
-    for (; i < cb; i += kQueryLanes) consider(load_world(a.world + sb + i), sb + i, b);
+    for (; i < cb; i += 32) consider(load_world(a.world + sb + i), sb + i, b);
   };
 
-  // (1) centre voxel: every lane of the group probes the same slot (one broadcast load)
+  // (1) centre voxel: every lane probes the same slot (one broadcast load)
   {
     uint32_t s0 = 0u, c0 = 0u;
     if (searchable) probe_voxel(a.hash, a.hash_mask, pack_key(cx, cy, cz), s0, c0);
@@ -566,14 +546,12 @@ template <int kQueryLanes> __device__ __forceinline__ void assoc_nn_body(const A
   }
   double bound = best;
 #pragma unroll
-  for (int off = kQueryLanes / 2; off > 0; off >>= 1)
-    bound = fmin(bound, __shfl_xor_sync(0xffffffffu, bound, off));
+  for (int off = 16; off > 0; off >>= 1) bound = fmin(bound, __shfl_xor_sync(0xffffffffu, bound, off));
 
-  // (2) squared distance from the query to the box of each of this lane's voxels, shrunk by a
-  // safety margin that covers the rounding of floor(x / w) at the voxel faces.  All shifts
-  // are -1 / 0 / +1 per axis, so the per-axis terms are the distances to the two faces of
-  // the centre voxel - computed once per query, then three selects per voxel.
-  constexpr unsigned kGroupMask = kQueryLanes == 32 ? 0xffffffffu : ((1u << (kQueryLanes & 31)) - 1u);
+  // (2) squared distance from the query to the box of this lane's voxel, shrunk by a safety
+  // margin that covers the rounding of floor(x / w) at the voxel faces.  All shifts are -1 / 0 /
+  // +1 per axis, so the per-axis terms are the distances to the two faces of the centre voxel -
+  // computed once per query, then three selects.
   double face2[3][2]; // [axis][0: towards -1, 1: towards +1], squared, margin applied
   {
     const double qq[3] = {wx, wy, wz};
@@ -588,52 +566,40 @@ template <int kQueryLanes> __device__ __forceinline__ void assoc_nn_body(const A
       face2[k][1] = dp * dp;
     }
   }
-  unsigned survivors = 0; // bit v: the voxel with shift rank v of this group's query must be searched
-  bool keep[kVox];
+  bool keep = false;
+  if (searchable && lane > 0 && lane < 27) {
+    double lb = 0.0;
 #pragma unroll
-  for (int r = 0; r < kVox; ++r) {
-    const int v = sub | (kQueryLanes * r);
-    keep[r] = false;
-    if (searchable && v > 0 && v < 27) {
-      double lb = 0.0;
-#pragma unroll
-      for (int k = 0; k < 3; ++k) {
-        const int sh = lane_shift(v, k);
-        lb += sh == 0 ? 0.0 : sh < 0 ? face2[k][0] : face2[k][1];
-      }
-      keep[r] = lb <= bound;
+    for (int k = 0; k < 3; ++k) {
+      const int sh = lane_shift(lane, k);
+      lb += sh == 0 ? 0.0 : sh < 0 ? face2[k][0] : face2[k][1];
     }
-    const unsigned bal = __ballot_sync(0xffffffffu, keep[r]);
-    survivors |= ((bal >> (grp * kQueryLanes)) & kGroupMask) << ((kQueryLanes * r) & 31);
+    keep = lb <= bound;
   }
+  const unsigned survivors = __ballot_sync(0xffffffffu, keep); // bit v: voxel v must be searched
 
-  // (3) compaction: the i-th surviving rank is probed by lane i % kQueryLanes, which leaves the
-  // bucket's {start, count} in shared memory for the whole group
+  // (3) compaction: the i-th surviving rank is probed by lane i, which leaves the bucket's
+  // {start, count} in shared memory for the whole warp
   const int n_surv = __popc(survivors);
-#pragma unroll
-  for (int r = 0; r < kVox; ++r) {
-    const int v = sub | (kQueryLanes * r);
-    if (keep[r]) s_list[warp][grp][__popc(survivors & ((1u << v) - 1u))] = (unsigned char)v;
-  }
+  if (keep) s_list[warp][__popc(survivors & ((1u << lane) - 1u))] = (unsigned char)lane;
   __syncwarp();
-  for (int i = sub; i < n_surv; i += kQueryLanes) {
-    const int v = s_list[warp][grp][i];
+  if (lane < n_surv) {
+    const int v = s_list[warp][lane];
     uint32_t st = 0u, ct = 0u;
     probe_voxel(a.hash, a.hash_mask,
                 pack_key(cx + lane_shift(v, 0), cy + lane_shift(v, 1), cz + lane_shift(v, 2)), st, ct);
-    s_bucket[warp][grp][i] = make_uint2(st, ct & ~kCellFlag);
+    s_bucket[warp][lane] = make_uint2(st, ct & ~kCellFlag);
   }
   __syncwarp();
 
-  // (4) the survivors' non-empty buckets, one after the other (no warp-wide operation inside:
-  // every group runs its own trip count)
+  // (4) the survivors' non-empty buckets, one after the other
   for (int i = 0; i < n_surv; ++i) {
-    const uint2 bk = s_bucket[warp][grp][i];
-    if (bk.y) scan_bucket(s_list[warp][grp][i], bk.x, bk.y);
+    const uint2 bk = s_bucket[warp][i];
+    if (bk.y) scan_bucket(s_list[warp][i], bk.x, bk.y);
   }
-  // arg-min over the group's lanes with the same key
+  // arg-min over the lanes with the same key
 #pragma unroll
-  for (int off = kQueryLanes / 2; off > 0; off >>= 1) {
+  for (int off = 16; off > 0; off >>= 1) {
     const double od = __shfl_xor_sync(0xffffffffu, best, off);
     const unsigned long long ot = __shfl_xor_sync(0xffffffffu, best_tie, off);
     const uint32_t op = __shfl_xor_sync(0xffffffffu, best_pos, off);
@@ -648,7 +614,7 @@ template <int kQueryLanes> __device__ __forceinline__ void assoc_nn_body(const A
       best_rank = orank;
     }
   }
-  if (active && sub == 0) {
+  if (active && lane == 0) {
     MatchRec m;
     if (best_pos == kNoSlot) {
       m.dist_sqrd = DBL_MAX;
@@ -762,7 +728,7 @@ constexpr unsigned shift_mask(int axis, int dir) {
 }
 constexpr unsigned kShiftNeg[3] = {shift_mask(0, -1), shift_mask(1, -1), shift_mask(2, -1)};
 constexpr unsigned kShiftPos[3] = {shift_mask(0, 1), shift_mask(1, 1), shift_mask(2, 1)};
-template <bool kDry = false> __device__ __forceinline__ void assoc_cells_body(const AssocArgs &a) {
+__device__ __forceinline__ void assoc_cells_body(const AssocArgs &a) {
   const int q = blockIdx.x * blockDim.x + threadIdx.x;
   const int lane = threadIdx.x & 31;
   const bool active = q >= a.q_begin && q < a.q_end;
@@ -1000,10 +966,6 @@ template <bool kDry = false> __device__ __forceinline__ void assoc_cells_body(co
     if (a.pack_rank) m.slot |= (uint32_t)best.rank << 8;
     m.k = src & 0xFFFFFFu;
   }
-  if (kDry) { // sensitivity probe (FORMGPU_DEBUG_ASSOC_REPEAT): the whole search, no side effects
-    if (mine && m.dist_sqrd < -1.0) a.match[q] = m; // never true: keeps the search alive
-    return;
-  }
   if (mine) a.match[q] = m;
   if (a.hist_cnt) hist_add(a, q, lane, mine, m);
 }
@@ -1057,23 +1019,15 @@ constexpr int kCellQueryThreads = 128;
 __global__ void __launch_bounds__(kCellQueryThreads) assoc_cells_kernel(AssocArgs pa, AssocArgs qa) {
   assoc_cells_body(blockIdx.y == 0 ? pa : qa);
 }
-template <bool kDry>
 __global__ void __launch_bounds__(kCellQueryThreads) assoc_cells_batch_kernel(const AssocArgs *items) {
   __shared__ AssocArgs s_a;
   load_item_args(s_a, items + 2 * blockIdx.z + blockIdx.y);
   if ((int)(blockIdx.x * kCellQueryThreads) >= s_a.n_query) return;
-  assoc_cells_body<kDry>(s_a);
+  assoc_cells_body(s_a);
 }
 
-__global__ void __launch_bounds__(256) assoc_nn_kernel(AssocArgs pa, AssocArgs qa) {
-  assoc_nn_body<kLanesSingle>(blockIdx.y == 0 ? pa : qa);
-}
-template <int kQueryLanes>
-__global__ void __launch_bounds__(256, 4) assoc_nn_batch_kernel(const AssocArgs *items) {
-  __shared__ AssocArgs s_a;
-  load_item_args(s_a, items + 2 * blockIdx.z + blockIdx.y);
-  if ((int)(blockIdx.x * queries_per_cta(kQueryLanes)) >= s_a.n_query) return;
-  assoc_nn_body<kQueryLanes>(s_a);
+__global__ void __launch_bounds__(kNnWarps * 32) assoc_nn_kernel(AssocArgs pa, AssocArgs qa) {
+  assoc_nn_body(blockIdx.y == 0 ? pa : qa);
 }
 
 void assoc_launch(const AssocArgs &pa, const AssocArgs &qa, bool cell_search, cudaStream_t stream,
@@ -1081,41 +1035,18 @@ void assoc_launch(const AssocArgs &pa, const AssocArgs &qa, bool cell_search, cu
   const int n = max(pa.n_query, qa.n_query);
   if (n <= 0) return;
   prof.begin(FORMGPU_KG_ASSOC_NN);
-  if (pa.cell_tab && cell_search) { // cell-ordered buckets: one thread per query
+  if (cell_search)
     assoc_cells_kernel<<<dim3((n + kCellQueryThreads - 1) / kCellQueryThreads, 2), kCellQueryThreads, 0, stream>>>(pa, qa);
-    prof.end(FORMGPU_KG_ASSOC_NN, 1);
-    return;
-  } else {
-    constexpr int per_cta = queries_per_cta(kLanesSingle);
-    assoc_nn_kernel<<<dim3((n + per_cta - 1) / per_cta, 2), 256, 0, stream>>>(pa, qa);
-  }
+  else
+    assoc_nn_kernel<<<dim3((n + kNnWarps - 1) / kNnWarps, 2), kNnWarps * 32, 0, stream>>>(pa, qa);
   prof.end(FORMGPU_KG_ASSOC_NN, 1);
 }
 
-void assoc_batch_launch(const AssocArgs *items_dev, int n_items, int max_query, int lanes, cudaStream_t stream,
-                        Profiler &prof) {
+void assoc_batch_launch(const AssocArgs *items_dev, int n_items, int max_query, cudaStream_t stream, Profiler &prof) {
   if (n_items <= 0 || max_query <= 0) return;
   prof.begin(FORMGPU_KG_ASSOC_NN);
-  if (lanes == 1) { // cell-ordered buckets: one thread per query
-    // development probe: how much does the step time move when this kernel's work doubles?
-    static const int repeat = [] {
-      const char *e = std::getenv("FORMGPU_DEBUG_ASSOC_REPEAT");
-      return e ? std::atoi(e) : 0;
-    }();
-    for (int r = 0; r < repeat; ++r)
-      assoc_cells_batch_kernel<true><<<dim3((max_query + kCellQueryThreads - 1) / kCellQueryThreads, 2, n_items),
-                                       kCellQueryThreads, 0, stream>>>(items_dev);
-    assoc_cells_batch_kernel<false><<<dim3((max_query + kCellQueryThreads - 1) / kCellQueryThreads, 2, n_items),
-                                      kCellQueryThreads, 0, stream>>>(items_dev);
-    prof.end(FORMGPU_KG_ASSOC_NN, 1);
-    return;
-  }
-  const auto grid = [&](int per_cta) { return dim3((max_query + per_cta - 1) / per_cta, 2, n_items); };
-  switch (lanes) {
-  case 2: assoc_nn_batch_kernel<2><<<grid(queries_per_cta(2)), 256, 0, stream>>>(items_dev); break;
-  case 8: assoc_nn_batch_kernel<8><<<grid(queries_per_cta(8)), 256, 0, stream>>>(items_dev); break;
-  default: assoc_nn_batch_kernel<4><<<grid(queries_per_cta(4)), 256, 0, stream>>>(items_dev); break;
-  }
+  assoc_cells_batch_kernel<<<dim3((max_query + kCellQueryThreads - 1) / kCellQueryThreads, 2, n_items),
+                             kCellQueryThreads, 0, stream>>>(items_dev);
   prof.end(FORMGPU_KG_ASSOC_NN, 1);
 }
 

@@ -388,7 +388,7 @@ __device__ __forceinline__ void eval_body(const LinArgs &a, const LinTask &task,
   double ev = 0.0, r0v = 0.0;
   if (tid < kMomentPlanar + kMomentPoint) ev = __ldcg(entry + tid);
   if (tid < 12) r0v = __ldcg(entry + kMomentPlanar + kMomentPoint + tid);
-  if (!kErrorOnly) zero_basis<false>(S.exp);
+  if (!kErrorOnly) zero_basis(S.exp);
   for (int i = tid; i < 7 * 13; i += kEvalThreads) (&S.Sc[0][0])[i] = 0.0;
   for (int i = tid; i < 7 * 7; i += kEvalThreads) (&S.Zc[0][0])[i] = 0.0;
   if (tid < kMomentPlanar) {
@@ -422,7 +422,7 @@ __device__ __forceinline__ void eval_body(const LinArgs &a, const LinTask &task,
   }
   // ---- phase 1: basis (threads 72..110) and coefficient matrices (threads 0..26, 32..40, 64..66,
   // 96; tests/test_moment_model.py: coeff_S, coeff_Z), both from rel / rel0 alone ----
-  if (!kErrorOnly) fill_basis<false>(S.exp, S.rel, 72);
+  if (!kErrorOnly) fill_basis(S.exp, S.rel, 72);
   {
     const double *rel = S.rel, *rel0 = S.rel0;
     auto dR = [&](int r, int c) { // (R R0^T)[r][c]
@@ -516,9 +516,8 @@ __device__ __forceinline__ void eval_body(const LinArgs &a, const LinTask &task,
     return;
   }
   // ---- phases 4-5: the 13x13 block ----
-  expand_and_publish<false>(S.exp, S.Wp28, S.Wq28, true, true, a.inv_sigma2,
-                            a.out + 182 * (size_t)task.out_index, tag,
-                            a.out_plain ? a.out_plain + 91 * (size_t)task.out_index : nullptr);
+  expand_and_publish(S.exp, S.Wp28, S.Wq28, true, true, a.inv_sigma2, a.out + 182 * (size_t)task.out_index, tag,
+                     a.out_plain ? a.out_plain + 91 * (size_t)task.out_index : nullptr);
 }
 
 } // namespace

@@ -39,7 +39,6 @@ public:
     if (params.size() != traces.size()) throw HotPathError("BatchReplay: one params entry per trace");
     for (size_t s = 0; s < params.size(); ++s)
       m_seq[s].points = (size_t)params[s].num_rows * (size_t)params[s].num_columns;
-    if (const char *env = std::getenv("FORM_REPLAY_SKIP_KEYPOINTS")) m_skip_keypoints = env[0] == '1'; // probe only
     if (const char *env = std::getenv("FORM_REPLAY_PREFETCH")) m_prefetch = env[0] != '0';
     const int rc = formgpu_batch_create_mixed(params.data(), device, stream, traces.size(), &m_batch);
     if (rc != FORMGPU_OK)
@@ -233,7 +232,7 @@ private:
       r.scan = scans[op.scan];
       r.n_points = q.points;
       r.scan_idx = op.scan;
-      if (!on_device && !m_skip_keypoints) {
+      if (!on_device) {
         r.planar_out = reinterpret_cast<formgpu_planar_feat *>(q.planar);
         r.planar_cap = q.planar_cap;
         r.point_out = reinterpret_cast<formgpu_point_feat *>(q.point);
@@ -377,7 +376,6 @@ private:
   formgpu_batch *m_batch = nullptr;
   bool m_host_ready = false;
   bool m_on_device = false;
-  bool m_skip_keypoints = false; // development probe: host scans in, only the counts back
   bool m_prefetch = true;        // FORM_REPLAY_PREFETCH=0: every scan is uploaded by its EXTRACT request
   const formgpu_point4f *const *const *m_scans = nullptr;
   size_t m_rounds = 0;

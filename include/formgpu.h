@@ -450,9 +450,9 @@ int formgpu_batch_create(const formgpu_params *p, int device, void *stream, size
                          formgpu_batch **out);
 /* A batch whose sequence i is configured by params[i] (n_sequences entries): sensors of different
  * shapes and parameter variants share one launch per kernel.  Every field of formgpu_params may
- * differ from sequence to sequence.  Shared by the whole batch: `device`, `stream`, and the switches
- * read from the environment when a context is created (FORMGPU_CELL_BUCKETS,
- * FORMGPU_STREAM_LINEARIZE), which the batch takes from its first context.  Every entry goes
+ * differ from sequence to sequence.  Shared by the whole batch: `device` and `stream`.  The contexts
+ * of a batch always evaluate linearisations and errors from their pair-moment caches
+ * (FORMGPU_STREAM_LINEARIZE applies to single contexts only).  Every entry goes
  * through formgpu_create's parameter checks before any CUDA call; when one fails,
  * formgpu_batch_last_error(NULL) names the index of its sequence. */
 int formgpu_batch_create_mixed(const formgpu_params *params, int device, void *stream, size_t n_sequences,

@@ -46,45 +46,8 @@ def main():
             return (time.perf_counter() - t0) / n * 1e6
 
         print(f"pairs of current scan: {len(pairs)}, correspondences {ncorr}; window pairs {len(allpairs)}")
-        for cl in ("", "1", "2", "4", "8"):
-            for flags in ("0",):
-                if cl:
-                    os.environ["FORMGPU_DEBUG_CLUSTER"] = cl
-                else:
-                    os.environ.pop("FORMGPU_DEBUG_CLUSTER", None)
-                os.environ["FORMGPU_DEBUG_FLAGS"] = flags
-                t1 = timeit(lambda: ctx.linearize(pairs, poses))
-                t2 = timeit(lambda: ctx.linearize(allpairs, poses), 100)
-                print(f"cluster={cl or 'auto':>4s} flags={flags}: linearize(cur scan) {t1:7.2f} us   linearize(window) {t2:7.2f} us")
-        # in-kernel phase timeline of pair 0 (%globaltimer, ns)
-        import ctypes as C
-        lib = _capi.gpu_lib()
-        lib.formgpu_debug_timestamps.restype = C.POINTER(C.c_uint64)
-        lib.formgpu_debug_timestamps.argtypes = [C.c_void_p]
-        os.environ.pop("FORMGPU_DEBUG_CLUSTER", None)
-        os.environ["FORMGPU_DEBUG_FLAGS"] = "4"
-        names = ["start", "planar loop", "reduce planar", "point loop+reduce", "cluster.sync 1", "gather",
-                 "cluster.sync 2", "expand+publish"]
-        acc = np.zeros(8)
-        n_rep = 50
-        for _ in range(n_rep):
-            t_host0 = time.perf_counter()
-            ctx.linearize(pairs, poses)
-            t_host = (time.perf_counter() - t_host0) * 1e6
-            ts = np.array([lib.formgpu_debug_timestamps(ctx._h)[i] for i in range(8)], dtype=np.float64)
-            acc[1:] += np.diff(ts)
-            acc[0] += t_host
-        print("lin kernel phases (ns, mean):", ", ".join(f"{n}={v / n_rep:.0f}" for n, v in zip(names[1:], acc[1:])),
-              f"| kernel span {acc[1:].sum() / n_rep:.0f} ns | host call {acc[0] / n_rep:.1f} us")
-        os.environ["FORMGPU_DEBUG_FLAGS"] = "0"
-        lib.formgpu_debug_host_times.restype = C.c_uint64
-        lib.formgpu_debug_host_times.argtypes = [C.c_void_p, C.c_void_p]
-        hb = np.zeros(8)
-        lib.formgpu_debug_host_times(ctx._h, _capi.ptr(hb))
-        t_py = timeit(lambda: ctx.linearize(pairs, poses))
-        n = lib.formgpu_debug_host_times(ctx._h, _capi.ptr(hb))
-        print(f"linearize host phases per call: build {hb[0] / n:.2f} us, launch API {hb[1] / n:.2f} us, "
-              f"wait {hb[2] / n:.2f} us (python total {t_py:.2f} us)")
+        print(f"linearize(cur scan)  {timeit(lambda: ctx.linearize(pairs, poses)):7.2f} us")
+        print(f"linearize(window)    {timeit(lambda: ctx.linearize(allpairs, poses), 100):7.2f} us")
         print(f"error(cur scan)      {timeit(lambda: ctx.error(pairs, poses)):7.2f} us")
         print(f"associate            {timeit(lambda: ctx.associate(est[k]), 100):7.2f} us")
         print(f"map_rebuild          {timeit(lambda: ctx.map_rebuild(poses), 100):7.2f} us")

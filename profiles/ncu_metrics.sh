@@ -8,5 +8,5 @@ COUNT=${3:-400}
 # replay saves / restores device memory around every kernel and takes minutes
 M="gpu__time_duration.sum,launch__grid_size,smsp__inst_executed.sum,smsp__issue_active.avg.pct_of_peak_sustained_active,sm__warps_active.avg.pct_of_peak_sustained_active,smsp__thread_inst_executed_per_inst_executed.ratio"
 SEQS=${4:-16}
-ncu --metrics $M --clock-control none -k regex:'batch|lin_warp|normals_rows|eval_global' --launch-skip $SKIP -c $COUNT --csv --log-file $OUT \
+ncu --metrics $M --clock-control none -k regex:'batch|normals_rows|eval_global' --launch-skip $SKIP -c $COUNT --csv --log-file $OUT \
     python profiles/batch_probe.py $SEQS 10 3

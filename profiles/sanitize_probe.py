@@ -1,6 +1,5 @@
 """Workload for compute-sanitizer (profiles/sanitize.sh): a batched replay of three short VLP-16
-sequences (every batched kernel incl. the ticketed moment merge and the cached evaluation), then
-the same with FORMGPU_STREAM_LINEARIZE=1 (ticketed slice merge of lin_warp_kernel)."""
+sequences (every batched kernel incl. the ticketed moment merge and the cached evaluation)."""
 import os
 import sys
 
@@ -25,13 +24,11 @@ def main():
             est.register_scan(s)
         runs.append((est, scans))
     host_ptrs = [[s.ctypes.data for s in scans] for _, scans in runs]
-    for stream in ("0", "1"):
-        os.environ["FORMGPU_STREAM_LINEARIZE"] = stream
-        br = BatchReplay([est.trace() for est, _ in runs], p)
-        br.run(0, n, host_ptrs, on_device=False)
-        st = br.stats()
-        assert st["scans"] == 3 * n and st["lin_pairs"] > 0
-        br.close()
+    br = BatchReplay([est.trace() for est, _ in runs], p)
+    br.run(0, n, host_ptrs, on_device=False)
+    st = br.stats()
+    assert st["scans"] == 3 * n and st["lin_pairs"] > 0
+    br.close()
     print("probe ok")
 
 

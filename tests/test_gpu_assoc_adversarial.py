@@ -6,11 +6,9 @@ bytes) and with the independent brute-force rule R5 on the checked queries.
 
 | configuration | association kernel |
 |---|---|
-| warp        | assoc_nn_kernel over cell-ordered buckets (the single-context default) |
+| warp        | assoc_nn_kernel, one warp per query (the single-context default) |
 | cells       | assoc_cells_kernel (FORMGPU_SINGLE_CELL_SEARCH=1) |
-| whole       | assoc_nn_kernel over whole buckets (FORMGPU_CELL_BUCKETS=0) |
 | batch       | assoc_cells_batch_kernel (raw formgpu_batch_* requests) |
-| lanes2/4/8  | assoc_nn_batch_kernel<L> (FORMGPU_CELL_BUCKETS=0, FORMGPU_ASSOC_LANES=L) |
 | mixed       | one formgpu_batch_create_mixed submission per operation for scenes of widths 0.5, 0.8, 64 |
 
 Stage 3 on the same windows: linearisation and error against the oracle at the association poses,
@@ -33,13 +31,9 @@ SCENES = {s.name: s for s in A.all_scenes()}
 CONFIGS = {
     "warp": {},
     "cells": {"FORMGPU_SINGLE_CELL_SEARCH": "1"},
-    "whole": {"FORMGPU_CELL_BUCKETS": "0"},
     "batch": {},
-    "lanes2": {"FORMGPU_CELL_BUCKETS": "0", "FORMGPU_ASSOC_LANES": "2"},
-    "lanes4": {"FORMGPU_CELL_BUCKETS": "0", "FORMGPU_ASSOC_LANES": "4"},
-    "lanes8": {"FORMGPU_CELL_BUCKETS": "0", "FORMGPU_ASSOC_LANES": "8"},
 }
-ENV = ("FORMGPU_SINGLE_CELL_SEARCH", "FORMGPU_CELL_BUCKETS", "FORMGPU_ASSOC_LANES", "FORMGPU_STREAM_LINEARIZE")
+ENV = ("FORMGPU_SINGLE_CELL_SEARCH", "FORMGPU_STREAM_LINEARIZE")
 
 
 def _env(monkeypatch, cfg):
@@ -161,7 +155,7 @@ def _check(scene, recs, label):
 def test_association_matches_oracle_and_brute_force(name, config, monkeypatch):
     _env(monkeypatch, CONFIGS[config])
     scene = SCENES[name]
-    if config in ("warp", "cells", "whole"):
+    if config in ("warp", "cells"):
         with Context(scene.make_params()) as ctx:
             recs = A.run(scene, ctx)
     else:
@@ -175,7 +169,7 @@ def test_association_matches_oracle_and_brute_force(name, config, monkeypatch):
 
 @pytest.mark.parametrize("group", [("lattice_w0.5", "face_aligned", "huge_bucket", "large_ids"),
                                    ("gates", "synthetic_far", "sparse", "buckets_19", "far_w1.0")])
-@pytest.mark.parametrize("config", ["batch", "lanes4"])
+@pytest.mark.parametrize("config", ["batch"])
 def test_one_mixed_launch(group, config, monkeypatch):
     """Scenes of different widths (0.5, 0.8, 64; 1.0, 0.8, 0.5) and sensor shapes in one
     formgpu_batch_create_mixed batch: every submission carries one operation of each, so one

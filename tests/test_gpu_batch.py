@@ -83,6 +83,37 @@ def test_batched_replay_is_bit_identical_to_single_contexts():
         assert b2.stats(s) == br.stats(s)
 
 
+def test_batches_ignore_the_streaming_switch(monkeypatch):
+    """FORMGPU_STREAM_LINEARIZE=1 applies to single contexts only: a batch created with it in the
+    environment evaluates from the pair-moment cache like any other batch, so its blocks (checksum)
+    and every counter are bit-identical to those of a batch created without it."""
+    import torch
+
+    from form_b200.pipeline import BatchReplay
+
+    n = 10
+    runs = [_record("vlp-16", seq, n) for seq in (1, 6)]
+    p = runs[0][2]
+    dev = [[torch.from_numpy(s.view(np.uint8)).cuda() for s in scans] for _, scans, _ in runs]
+    torch.cuda.synchronize()
+    ptrs = [[d.data_ptr() for d in seq] for seq in dev]
+
+    def replay():
+        br = BatchReplay([est.trace() for est, _, _ in runs], p)
+        try:
+            br.run(0, n, ptrs, on_device=True)
+            return [br.stats(s) for s in range(len(runs))]
+        finally:
+            br.close()
+
+    monkeypatch.delenv("FORMGPU_STREAM_LINEARIZE", raising=False)
+    want = replay()
+    monkeypatch.setenv("FORMGPU_STREAM_LINEARIZE", "1")
+    got = replay()
+    assert all(w["lin_pairs"] > 0 for w in want)
+    assert got == want
+
+
 def test_captured_last_scan_is_what_its_calls_returned():
     """capture_last_scan (bench.py --dump-outputs): over a run of several scans, the records kept are
     those of its LAST scan only - keypoints as the live estimator got them, counts and blocks that

@@ -1,40 +1,16 @@
-"""Cell-ordered voxel buckets (map_assoc.cu pass 4 + the cell-by-cell search of assoc_nn) are the
-default; every other GPU test therefore runs with them.  Here the same stage-2 parity checks run
-with FORMGPU_CELL_BUCKETS=0 (whole-bucket scans, the round-1 search) so that both paths stay
-bit-identical to the oracle: neighbour ids, squared-distance bits, pair counts, novel sets."""
+"""The cell search of the batched submits (assoc_cells_body: one thread per query, cell by cell over
+the cell-ordered voxel buckets of map_assoc.cu pass 4) on single contexts, through
+FORMGPU_SINGLE_CELL_SEARCH=1, so that it goes through every stage-2 oracle check of the
+single-context sequences: neighbour ids, squared-distance bits, pair counts, novel sets."""
 import pytest
 
-import test_gpu_batch
 import test_gpu_stages
 
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(autouse=True)
-def whole_bucket_scans(monkeypatch):
-    monkeypatch.setenv("FORMGPU_CELL_BUCKETS", "0")
-
-
-def test_plain_os1_64_sequence():
-    test_gpu_stages._run_sequence("os1-64", 8, remove_at={4: [1], 6: [0, 3]})
-
-
-def test_plain_vlp16_sparse():
-    test_gpu_stages._run_sequence("vlp-16", 10, seq=2, remove_at={5: [2]})
-
-
-def test_plain_small_matching_distance():
-    test_gpu_stages._run_sequence("vlp-16", 5, overrides=dict(max_dist_matching=0.3, min_dist_map=0.05))
-
-
-def test_plain_batched_replay_is_bit_identical_to_single_contexts():
-    test_gpu_batch.test_batched_replay_is_bit_identical_to_single_contexts()
-
-
-# ---- the cell search of the batched submits, on single contexts (every stage-2 oracle check) ----
 @pytest.fixture
 def cell_search(monkeypatch):
-    monkeypatch.setenv("FORMGPU_CELL_BUCKETS", "1")
     monkeypatch.setenv("FORMGPU_SINGLE_CELL_SEARCH", "1")
 
 

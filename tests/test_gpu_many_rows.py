@@ -1,9 +1,8 @@
-"""Kernel variants that only batched submits use.  Many-row extraction kernels (192-thread select
-CTAs, thread-per-pick normals; kernels.hpp: kManyRowsMin, FORMGPU_MANY_ROWS_MIN) and the lanes
-per query of the batched association kernel (kAssocLanes, FORMGPU_ASSOC_LANES): keypoints -
-normals included - are compared bit for bit with the CPU oracle on the synthetic sensor shapes,
-parameter variants and the edge-case scans of test_gpu_extract; association counters with the
-single-sequence path."""
+"""Kernel variants that only batched submits use: the many-row extraction kernels (192-thread
+select CTAs, thread-per-pick normals; kernels.hpp: kManyRowsMin, FORMGPU_MANY_ROWS_MIN) and, above
+that threshold, the latency-shaped ones.  Keypoints - normals included - are compared bit for bit
+with the CPU oracle on the synthetic sensor shapes, parameter variants and the edge-case scans of
+test_gpu_extract."""
 import ctypes as C
 import zlib
 
@@ -95,36 +94,6 @@ def test_large_and_single_scan_batches_match_oracle():
     scans = [synth.scan("os1-64", s, 9) for s in range(5)]
     _batch_extract_vs_oracle(params, scans, rows, cols)
     _batch_extract_vs_oracle(params, scans[:1], rows, cols)
-
-
-@pytest.mark.parametrize("lanes", [2, 8])
-def test_association_lane_variants_match_single_contexts(monkeypatch, lanes):
-    """FORMGPU_ASSOC_LANES selects how many lanes share a query in the batched association
-    kernel (default kAssocLanes = 4): every variant must reproduce the single-sequence path's
-    match / pair / novel counters exactly and its blocks to 1e-12."""
-    import torch
-
-    from form_b200.pipeline import BatchReplay, Replay
-    from test_gpu_batch import _record
-
-    monkeypatch.setenv("FORMGPU_ASSOC_LANES", str(lanes))
-    n = 10
-    runs = [_record("vlp-16", seq, n) for seq in (1, 6)]
-    p = runs[0][2]
-    dev = [[torch.from_numpy(s.view(np.uint8)).cuda() for s in scans] for _, scans, _ in runs]
-    torch.cuda.synchronize()
-    ptrs = [[d.data_ptr() for d in seq] for seq in dev]
-    br = BatchReplay([est.trace() for est, _, _ in runs], p)
-    br.run(0, n, ptrs, on_device=True)
-    for s, ((est, _, _), pp) in enumerate(zip(runs, ptrs)):
-        r = Replay(est.trace(), p)
-        r.run_device(0, n, pp)
-        ref, got = r.stats(), br.stats(s)
-        for k in ref:
-            if k == "checksum":
-                assert abs(got[k] - ref[k]) <= 1e-12 * abs(ref[k]), (lanes, s, k, got[k], ref[k])
-            else:
-                assert got[k] == ref[k], (lanes, s, k, got[k], ref[k])
 
 
 def test_few_row_variants_still_match_oracle(monkeypatch):
