@@ -190,6 +190,7 @@ __global__ void __launch_bounds__(256) map_insert_kernel(MapArgs pa, MapArgs qa)
 __global__ void __launch_bounds__(256) map_insert_batch_kernel(const MapArgs *items) {
   __shared__ MapArgs s_a;
   load_item_args(s_a, items + 2 * blockIdx.z + blockIdx.y);
+  pdl_wait();
   map_insert_body(s_a);
 }
 
@@ -218,6 +219,7 @@ __global__ void __launch_bounds__(256) map_alloc_kernel(MapArgs pa, MapArgs qa) 
 __global__ void __launch_bounds__(256) map_alloc_batch_kernel(const MapArgs *items) {
   __shared__ MapArgs s_a;
   load_item_args(s_a, items + 2 * blockIdx.z + blockIdx.y);
+  pdl_wait();
   map_alloc_body(s_a);
 }
 
@@ -242,6 +244,7 @@ __global__ void __launch_bounds__(256) map_scatter_kernel(MapArgs pa, MapArgs qa
 __global__ void __launch_bounds__(256) map_scatter_batch_kernel(const MapArgs *items) {
   __shared__ MapArgs s_a;
   load_item_args(s_a, items + 2 * blockIdx.z + blockIdx.y);
+  pdl_wait();
   map_scatter_body(s_a);
 }
 
@@ -371,6 +374,7 @@ __global__ void __launch_bounds__(kCellWarps * 32) map_cells_kernel(MapArgs pa, 
 __global__ void __launch_bounds__(kCellWarps * 32) map_cells_batch_kernel(const MapArgs *items) {
   __shared__ MapArgs s_a;
   load_item_args(s_a, items + 2 * blockIdx.z + blockIdx.y);
+  pdl_wait();
   map_cells_body(s_a);
 }
 
@@ -416,11 +420,11 @@ void map_build_batch_launch(const MapArgs *items_dev, const MapClearRegion *regi
   int launches = 1;
   if (max_points > 0) {
     const dim3 gp((max_points + 255) / 256, 2, n_items);
-    map_insert_batch_kernel<<<gp, 256, 0, stream>>>(items_dev);
-    map_alloc_batch_kernel<<<dim3((max_points + 255) / 256, 2, n_items), 256, 0, stream>>>(items_dev);
-    map_scatter_batch_kernel<<<gp, 256, 0, stream>>>(items_dev);
+    launch_pdl(map_insert_batch_kernel, gp, 256, 0, stream, items_dev);
+    launch_pdl(map_alloc_batch_kernel, dim3((max_points + 255) / 256, 2, n_items), 256, 0, stream, items_dev);
+    launch_pdl(map_scatter_batch_kernel, gp, 256, 0, stream, items_dev);
     const unsigned blocks = std::max(1u, std::min<unsigned>((unsigned)max_points / (16u * kCellWarps) + 1u, 512u));
-    map_cells_batch_kernel<<<dim3(blocks, 2, n_items), kCellWarps * 32, 0, stream>>>(items_dev);
+    launch_pdl(map_cells_batch_kernel, dim3(blocks, 2, n_items), kCellWarps * 32, 0, stream, items_dev);
     launches += 4;
   }
   prof.end(FORMGPU_KG_MAP_BUILD, launches);
@@ -1022,6 +1026,7 @@ __global__ void __launch_bounds__(kCellQueryThreads) assoc_cells_kernel(AssocArg
 __global__ void __launch_bounds__(kCellQueryThreads) assoc_cells_batch_kernel(const AssocArgs *items) {
   __shared__ AssocArgs s_a;
   load_item_args(s_a, items + 2 * blockIdx.z + blockIdx.y);
+  pdl_wait();
   if ((int)(blockIdx.x * kCellQueryThreads) >= s_a.n_query) return;
   assoc_cells_body(s_a);
 }
@@ -1045,8 +1050,8 @@ void assoc_launch(const AssocArgs &pa, const AssocArgs &qa, bool cell_search, cu
 void assoc_batch_launch(const AssocArgs *items_dev, int n_items, int max_query, cudaStream_t stream, Profiler &prof) {
   if (n_items <= 0 || max_query <= 0) return;
   prof.begin(FORMGPU_KG_ASSOC_NN);
-  assoc_cells_batch_kernel<<<dim3((max_query + kCellQueryThreads - 1) / kCellQueryThreads, 2, n_items),
-                             kCellQueryThreads, 0, stream>>>(items_dev);
+  launch_pdl(assoc_cells_batch_kernel, dim3((max_query + kCellQueryThreads - 1) / kCellQueryThreads, 2, n_items),
+             kCellQueryThreads, 0, stream, items_dev);
   prof.end(FORMGPU_KG_ASSOC_NN, 1);
 }
 
@@ -1183,6 +1188,7 @@ __global__ void __launch_bounds__(256) segment_scatter_kernel(SegmentArgs pa, Se
 __global__ void __launch_bounds__(256) segment_scatter_batch_kernel(const SegmentArgs *items) {
   __shared__ SegmentArgs s_a;
   load_item_args(s_a, items + 2 * blockIdx.z + blockIdx.y);
+  pdl_wait();
   segment_scatter_body(s_a);
 }
 
@@ -1200,7 +1206,7 @@ void segment_build_batch_launch(const SegmentArgs *items_dev, int n_items, int m
                                 cudaStream_t stream, Profiler &prof) {
   if (n_items <= 0 || max_query <= 0) return;
   prof.begin(FORMGPU_KG_SEGMENT);
-  segment_scatter_batch_kernel<<<dim3((max_query + 255) / 256, 2, n_items), 256, 0, stream>>>(items_dev);
+  launch_pdl(segment_scatter_batch_kernel, dim3((max_query + 255) / 256, 2, n_items), 256, 0, stream, items_dev);
   prof.end(FORMGPU_KG_SEGMENT, 1);
 }
 
@@ -1242,6 +1248,7 @@ __global__ void __launch_bounds__(256) commit_kernel(CommitArgs pa, CommitArgs q
 __global__ void __launch_bounds__(256) commit_batch_kernel(const CommitArgs *items) {
   __shared__ CommitArgs s_a;
   load_item_args(s_a, items + 2 * blockIdx.z + blockIdx.y);
+  pdl_wait();
   commit_body(s_a);
 }
 
@@ -1257,7 +1264,7 @@ void commit_batch_launch(const CommitArgs *items_dev, int n_items, int max_query
                          Profiler &prof) {
   if (n_items <= 0 || max_query <= 0) return;
   prof.begin(FORMGPU_KG_COMMIT);
-  commit_batch_kernel<<<dim3((max_query + 255) / 256, 2, n_items), 256, 0, stream>>>(items_dev);
+  launch_pdl(commit_batch_kernel, dim3((max_query + 255) / 256, 2, n_items), 256, 0, stream, items_dev);
   prof.end(FORMGPU_KG_COMMIT, 1);
 }
 

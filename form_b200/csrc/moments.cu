@@ -340,6 +340,7 @@ __global__ void __launch_bounds__(kMomentThreads, 2) moment_batch_kernel(const M
     reinterpret_cast<unsigned long long *>(&s_a)[i] =
         reinterpret_cast<const unsigned long long *>(items + blockIdx.z)[i];
   __syncthreads();
+  pdl_wait();
   moment_body(s_a, s_w[threadIdx.x >> 5]);
 }
 
@@ -542,6 +543,7 @@ eval_global_kernel(const LinArgs *ctx_args, const LinTask *tasks, int n_tasks) {
     reinterpret_cast<unsigned long long *>(&s.args)[tid - 32] =
         reinterpret_cast<const unsigned long long *>(ctx_args + tasks[blockIdx.x].ctx_index)[tid - 32];
   __syncthreads();
+  pdl_wait(); // the cache entries come from the moment kernel queued before (batched submits)
   eval_body<kErrorOnly>(s.args, s.task, s);
 }
 
@@ -556,8 +558,8 @@ void moments_batch_launch(const MomentArgs *items_dev, int n_items, int max_unit
                           Profiler &prof) {
   if (n_items <= 0 || max_units <= 0) return;
   prof.begin(FORMGPU_KG_LIN_CHUNK);
-  moment_batch_kernel<<<dim3((max_units + kMomentWarps - 1) / kMomentWarps, 1, n_items), kMomentThreads, 0,
-                        stream>>>(items_dev);
+  launch_pdl(moment_batch_kernel, dim3((max_units + kMomentWarps - 1) / kMomentWarps, 1, n_items), kMomentThreads, 0,
+             stream, items_dev);
   prof.end(FORMGPU_KG_LIN_CHUNK, 1);
 }
 
@@ -586,10 +588,11 @@ cudaError_t eval_batch_launch(const LinArgs *ctx_args_dev, const LinTask *tasks_
   const int group = error_only ? FORMGPU_KG_ERR_FINALIZE : FORMGPU_KG_LIN_FINALIZE;
   const int grid = n_tasks;
   prof.begin(group);
-  if (error_only) eval_global_kernel<true><<<grid, kEvalThreads, 0, stream>>>(ctx_args_dev, tasks_dev, n_tasks);
-  else eval_global_kernel<false><<<grid, kEvalThreads, 0, stream>>>(ctx_args_dev, tasks_dev, n_tasks);
+  const cudaError_t e =
+      error_only ? launch_pdl(eval_global_kernel<true>, grid, kEvalThreads, 0, stream, ctx_args_dev, tasks_dev, n_tasks)
+                 : launch_pdl(eval_global_kernel<false>, grid, kEvalThreads, 0, stream, ctx_args_dev, tasks_dev, n_tasks);
   prof.end(group, 1);
-  return cudaGetLastError();
+  return e != cudaSuccess ? e : cudaGetLastError();
 }
 
 } // namespace formgpu
